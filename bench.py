@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- SW GCUPS of the B200 path on BASELINE.json's configurations.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config 2] [--mode M] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config 2] [--mode M] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic input.  The headline workload is BASELINE.json
 configs[1]: ONE fixed set of 1M x 150-nt reads (seed 3) vs 8 influenza-A-length segments, score only (2.04e12 cells per
@@ -45,6 +45,37 @@ DPX_INSTR_PER_CELL = 2.25  # 4.5 DPX/ALU instructions per packed cell pair (DESI
 EXPECTED_CHECKSUM = {("cfg2", "score", 1_000_000): 268486591, ("cfg3", "align", 1_000_000): 4405153473,
                      ("cfg5", "score", 1_000_000): 767435248, ("cfg1", "score", 10_000): 1466752,
                      ("cfg4", "score", 20_000): 23653328}
+DUMP_BYTES = 64_000_000  # --dump-outputs writes at most this much
+
+
+def dump_outputs(out_dir: str, outs: dict, n: int, n_prof: int, mode: str):
+    """Writes the result arrays of the last timed step as float64 ``out_dir/<name>.npy``: one value per pair (pair =
+    read * n_prof + profiled sequence), and in the CIGAR modes ``cigar_len`` (words per pair) and the pairs' ``cigar``
+    words back to back.  When that exceeds DUMP_BYTES a seeded sample of reads is written; ``read_index`` lists the
+    reads kept.  The sample depends only on n and n_prof, so two builds of the project dump the same pairs.  CIGAR words
+    past the size limit are cut off."""
+    per_pair = ["score", "status", "tier"]
+    if mode != "score":
+        per_pair += ["ref_start", "ref_end", "query_start", "query_end"]
+    if mode == "align":
+        per_pair.append("hazard")
+    has_cigar = "cigar" in outs
+    limit = DUMP_BYTES - 4096  # room for the .npy headers
+    row_bytes = 8 * (1 + n_prof * (len(per_pair) + has_cigar))
+    k = min(n, (limit // 2 if has_cigar else limit) // row_bytes)
+    rows = np.arange(n) if k == n else np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+    pairs = (rows[:, None] * n_prof + np.arange(n_prof)[None, :]).reshape(-1)
+    arrays = {"read_index": rows}
+    arrays.update({name: outs[name][pairs] for name in per_pair})
+    if has_cigar:
+        lo = outs["cigar_off"][pairs].astype(np.int64)
+        lens = outs["cigar_off"][pairs + 1].astype(np.int64) - lo
+        arrays["cigar_len"] = lens
+        words = np.repeat(lo - (np.cumsum(lens) - lens), lens) + np.arange(int(lens.sum()))
+        arrays["cigar"] = outs["cigar"][words[: (limit - 8 * sum(a.size for a in arrays.values())) // 8]]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.astype(np.float64))
 
 
 def env_int(name, default):
@@ -302,8 +333,9 @@ def pinned(torch, arr: np.ndarray):
 
 
 def run_leg(ctx: Ctx, config: int, mode_override, n_override, steps: int, warmup: int, cpu: bool, cpu_seconds: float,
-            align_opts=None, sample_clocks: bool = False, full_parity: bool = True, scoring=None):
-    """Times one configuration on this rank's shard; returns the record rank 0 prints (None on the other ranks)."""
+            align_opts=None, sample_clocks: bool = False, full_parity: bool = True, scoring=None, dump_dir=None):
+    """Times one configuration on this rank's shard; returns the record rank 0 prints (None on the other ranks).
+    ``dump_dir``: rank 0 writes its shard's results of the last timed step there (dump_outputs)."""
     from zoe_b200 import CudaProfiles
 
     torch = ctx.torch
@@ -417,6 +449,8 @@ def run_leg(ctx: Ctx, config: int, mode_override, n_override, steps: int, warmup
     wall_ms = (time.perf_counter() - t0) * 1e3
     e2e_ms = ctx.max_over_ranks(max(ev2.elapsed_time(ev3), wall_ms))
     e2e_stats = prof.last_stats()
+    if dump_dir and ctx.rank == 0:
+        dump_outputs(dump_dir, outs, n, n_prof, mode)
     n_words = int(outs["cigar_off"][pairs]) if mode in ("align", "3pass") else 0
     d2h = {"score": pairs * 6, "ranges": pairs * 22}.get(mode, pairs * (5 * 4 + 3 + 8) + 8 + n_words * 4)
     # additive checksum: the per-rank values sum to the N = 1 value
@@ -675,7 +709,14 @@ def main():
                     help="full: cfg 1 / 3 / 5 are checked on the whole set (SURVEY 8(d)); sample: a bounded prefix")
     ap.add_argument("--scoring", default=None, help="match,mismatch,gap_open,gap_extend for the DNA configurations "
                                                     "(e.g. 4,-2,-3,-1: many E == H == F ties -> literal striped kernels)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the headline workload's results of the last timed step to DIR/<name>.npy (float64, "
+                         "at most 64 MB: a seeded sample of reads when larger)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's results; the reference arm times a prefix of the workload")
     if args.scoring:
         global SCORING
         SCORING = tuple(int(v) for v in args.scoring.split(","))
@@ -692,7 +733,7 @@ def main():
     cpu = not args.no_cpu_baseline
     full = args.parity == "full"
     head = run_leg(ctx, args.config, args.mode, args.n, args.steps, args.warmup, cpu, 12.0, args.align_opts,
-                   sample_clocks=True, full_parity=full)
+                   sample_clocks=True, full_parity=full, dump_dir=args.dump_outputs)
 
     legs = {}
     want = []
