@@ -135,6 +135,23 @@ struct Ops<false> {
     static __device__ __forceinline__ uint32_t splat(int v) { return (uint32_t)v; }
 };
 
+// Where the packed score kernel takes the gap penalties from.  A DPX instruction accepts a 32-bit immediate but no
+// constant-bank or uniform-register operand, so a penalty known only at run time occupies a vector register in three of
+// the four DPX instructions of every row (max3 with go, the two addmax with -ge).
+//   GapRt         the penalties of ScoreParams, kept opaque in registers (any scoring)
+//   GapImm<O, E>  go = O, ge = E compiled in: the DPX instructions take them as immediates
+// With immediates ptxas emits the "- go" of a row as VIADD rather than IMAD.IADD.  Pinning it to IMAD (a mad.lo.u32
+// with a multiplier of 1 ptxas cannot see) measured slower on B200, config 2: 281.1 against 279.9 ms per step.
+struct GapRt {
+    static constexpr bool kImm = false;
+    static constexpr int GO = 0, GE = 0;
+};
+template <int GO_, int GE_>
+struct GapImm {
+    static constexpr bool kImm = true;
+    static constexpr int GO = GO_, GE = GE_;
+};
+
 __device__ __forceinline__ uint32_t half2_max_bits(uint32_t a, uint32_t b) {
     uint32_t r;
     asm("max.f16x2 %0, %1, %2;" : "=r"(r) : "r"(a), "r"(b));
@@ -304,7 +321,7 @@ __device__ __forceinline__ void build_task_table(const TaskSmem &m, const ScoreP
 #ifndef ZOE_SCORE2_THREADS
 #define ZOE_SCORE2_THREADS 384
 #endif
-template <int G, int K, bool PACKED, int NS, bool PP = (ZOE_SCORE_PP && NS == 2 && K <= 19)>
+template <int G, int K, bool PACKED, int NS, class Gap = GapRt, bool PP = (ZOE_SCORE_PP && NS == 2 && K <= 19)>
 __global__ void __launch_bounds__((NS == 2 && (PP || K > 20)) ? ZOE_SCORE2_THREADS : 512) sw_score_kernel(const ScoreParams p) {
     using O = Ops<PACKED>;
     constexpr int K4 = (K + 3) / 4;
@@ -322,7 +339,8 @@ __global__ void __launch_bounds__((NS == 2 && (PP || K > 20)) ? ZOE_SCORE2_THREA
     const int tab_bytes = sm.tab_bytes;
     const uint8_t *cc = p.cols_in_smem ? s_cc : p.ccodes;
 
-    uint32_t go_s = O::splat(p.go), neg_ge = O::splat(-p.ge);
+    static_assert(!Gap::kImm || PACKED, "compiled-in gap penalties exist for the packed kernels only");
+    uint32_t go_s = O::splat(Gap::kImm ? Gap::GO : p.go), neg_ge = O::splat(Gap::kImm ? -Gap::GE : -p.ge);
     const uint4 *tab_lane = tab + lig;
     // Loop invariants kept opaque so the compiler does not rematerialise them inside the hot loops (S2R + address
     // arithmetic); the table offset stays a 32-bit offset into the shared array so the loads remain LDS.128.
@@ -330,7 +348,10 @@ __global__ void __launch_bounds__((NS == 2 && (PP || K > 20)) ? ZOE_SCORE2_THREA
     // lane 0 receives zeros from "above": multiplying by an opaque 0/1 keeps that on the FMA pipe (a SEL would
     // take an ALU slot, and the ALU pipe is what bounds this kernel)
     uint32_t nz = lig != 0 ? 1u : 0u;
-    asm volatile("" : "+r"(go_s), "+r"(neg_ge), "+r"(tab_lane_off), "+r"(nz));
+    if constexpr (Gap::kImm)
+        asm volatile("" : "+r"(tab_lane_off), "+r"(nz));
+    else
+        asm volatile("" : "+r"(go_s), "+r"(neg_ge), "+r"(tab_lane_off), "+r"(nz));
 
     // Static round-robin task assignment: every group of a warp makes the same number of trips,
     // so the warp never diverges on the task loop (invalid trips run on empty sequences).

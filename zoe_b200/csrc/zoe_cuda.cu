@@ -9,6 +9,8 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <array>
+#include <utility>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -116,6 +118,26 @@ struct Device {
     bool timed_kernel = false;
 };
 
+// Scorings (gap open, gap extend; positive penalties) whose packed score kernels are compiled with the penalties as
+// immediates (GapImm, sw_score.cuh); any other scoring runs the kernels that read them from ScoreParams.  Every pair adds
+// 28 kernels to the build.  (10, 1) is the scoring of all five benchmark configurations.
+struct GapPair {
+    int go, ge;
+};
+constexpr GapPair kGapImmPairs[] = {{10, 1}};
+constexpr int kNumGapImm = sizeof(kGapImmPairs) / sizeof(kGapImmPairs[0]);
+using ScoreFn = void (*)(const ScoreParams);
+using GapImmFns = std::array<ScoreFn, kNumGapImm>;
+template <int G, int K, int NS, size_t... I>
+constexpr GapImmFns gap_imm_fns(std::index_sequence<I...>) {
+    return {sw_score_kernel<G, K, true, NS, GapImm<kGapImmPairs[I].go, kGapImmPairs[I].ge>>...};
+}
+int gap_imm_index(int go, int ge) {
+    for (int i = 0; i < kNumGapImm; ++i)
+        if (kGapImmPairs[i].go == go && kGapImmPairs[i].ge == ge) return i;
+    return -1;
+}
+
 struct KernelEntry {
     int G, K;
     void (*packed)(const ScoreParams);
@@ -131,6 +153,7 @@ struct KernelEntry {
     void (*scan_rev)(const WinParams);   // ranges: reverse pass (score-rate scan + in-kernel pin)
     void (*scan2)(const WinParams);      // pass A, two tasks per group (K <= 20), codes in shared memory / ...
     void (*scan2_g)(const WinParams);    // ... codes from global memory
+    GapImmFns packed_imm, packed2_imm;   // packed / packed2 with the penalties of kGapImmPairs[i] compiled in
 };
 
 // the two-task pass A exists for K <= 20 (two H / F register sets per thread); a rejected experiment (see pick_scan2):
@@ -156,7 +179,9 @@ struct Scan2<G, K, false> {
             sw_ends_kernel<G, K, true>, sw_ends_kernel<G, K, false>, sw_align_scan_kernel<G, K, false>,     \
             sw_align_winfill_kernel<G, K, false>, sw_align_scan_kernel<G, K, true, true>,                   \
             Scan2<G, K, (ZOE_CUDA_WITH_SCAN2 != 0) && (K <= 20)>::smem(),                                  \
-            Scan2<G, K, (ZOE_CUDA_WITH_SCAN2 != 0) && (K <= 20)>::gmem()                                   \
+            Scan2<G, K, (ZOE_CUDA_WITH_SCAN2 != 0) && (K <= 20)>::gmem(),                                  \
+            gap_imm_fns<G, K, 1>(std::make_index_sequence<kNumGapImm>{}),                                   \
+            gap_imm_fns<G, K, 2>(std::make_index_sequence<kNumGapImm>{})                                    \
     }
 
 // Row capacity G*K of each instantiation; the host picks the tightest fit for the longest
@@ -206,6 +231,7 @@ struct zoe_cuda_ctx {
     std::vector<int8_t> weights;  // S*S, zoe's weights[ref_idx][query_idx]
     uint8_t lut[256];
     int go = 0, ge = 0;  // positive penalties
+    bool no_gap_imm = false;  // ZOE_CUDA_NO_GAP_IMM: always the run-time-penalty score kernels (A/B runs, tests)
     int profiled_is_query = 0;
     int max_weight = 0;
     int lanes[3] = {32, 16, 8};
@@ -784,6 +810,7 @@ int launch_score(zoe_cuda_ctx *ctx, Device &d, const KernelEntry &k, bool packed
     // sequences whose codes fit shared memory: the steady-state loops read the column codes from shared memory
     // (5.8 -> 6.9 TCUPS on a 131-kb panel); every launch re-reads the streamed batch, which is tiny next to the sweep
     const size_t n_launches = ctx->groups.empty() ? 1 : ctx->groups.size();
+    const int imm = ctx->no_gap_imm ? -1 : gap_imm_index(ctx->go, ctx->ge);
     for (size_t gi = 0; gi < n_launches; ++gi) {
         uint32_t n_cseq = ctx->n_prof;
         size_t cc_bytes = ctx->ccodes.size();
@@ -801,6 +828,7 @@ int launch_score(zoe_cuda_ctx *ctx, Device &d, const KernelEntry &k, bool packed
         }
         const bool two_streams = packed && n_cseq >= 2 && !getenv("ZOE_CUDA_ONE_STREAM");
         void (*fn)(const ScoreParams) = packed ? (two_streams ? k.packed2 : k.packed) : k.wide;
+        if (packed && imm >= 0) fn = two_streams ? k.packed2_imm[imm] : k.packed_imm[imm];
         LaunchPlan plan;
         int rc = plan_launch(ctx, k, fn, &plan, cc_bytes);
         if (rc) return rc;
@@ -2665,6 +2693,7 @@ int zoe_cuda_create(zoe_cuda_ctx **out, const int *device_ids, int n_devices) {
     if (n_devices > count) return ZOE_CUDA_E_BAD_ARG;
     zoe_cuda_ctx *ctx = new zoe_cuda_ctx();
     for (int i = 0; i < 256; ++i) ctx->lut[i] = 0;
+    ctx->no_gap_imm = getenv("ZOE_CUDA_NO_GAP_IMM") != nullptr;
     for (int k = 0; k < n_devices; ++k) {
         Device d;
         d.id = device_ids ? device_ids[k] : k;
