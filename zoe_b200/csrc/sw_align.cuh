@@ -496,7 +496,9 @@ __global__ void __launch_bounds__(128) sw_align_exact_kernel(const ExactParams x
         const int m = (int)(x.coff[cj + 1] - x.coff[cj]);
         const uint32_t want = x.score_in[gid];
         const uint8_t want_tier = tier_for(x.tp, want);
-        if (want_tier == 0) continue;  // Overflowed in every allowed type: nothing to align (warp-uniform)
+        // Overflowed in every allowed type: nothing to align (warp-uniform).  A packed overflow whose exact score then
+        // fell beyond the widest type is listed too, with score 0 (tier_for(0) is the first tier, not "Overflowed").
+        if (want == 0 || want_tier == 0) continue;
         const int N = want_tier == 8 ? x.lanes8 : (want_tier == 16 ? x.lanes16 : x.lanes32);
         const int nv = (m + N - 1) / N;
         // lane t owns SIMD lanes t and t+32 (N <= 64)

@@ -634,7 +634,8 @@ __global__ void exact_partition_kernel(const ExactPartitionParams q) {
     const uint32_t ent = q.hazard_list[i];
     const uint32_t gid = ent & ~kEndUnknown;
     const uint8_t tier = tier_for(q.tp, q.score[gid]);
-    if (tier == 0) return;
+    // score 0: a packed overflow whose exact score fell beyond the widest allowed type (Overflowed, like tier 0)
+    if (tier == 0 || q.score[gid] == 0) return;
     int which = 4;
     if (tier == 8 && q.fast8) which = (ent & kEndUnknown) ? 2 : 0;
     if (tier == 16 && q.fast16) which = (ent & kEndUnknown) ? 3 : 1;
