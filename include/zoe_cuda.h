@@ -142,6 +142,38 @@ int zoe_cuda_sw_align_3pass_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_con
                                   uint32_t *query_start, uint32_t *query_end, uint32_t *cigar, uint64_t *cigar_off,
                                   uint64_t cigar_cap);
 
+/* Both-strand search.  Each entry point takes exactly the arguments of its single-strand twin above plus a trailing
+ * `strand` (n * n_profiled entries, may be NULL): 0 = the streamed sequence as given, 1 = its reverse complement.
+ * For pair (i, j) let F be what the single-strand call returns for (seq_i, j) and R what it returns for
+ * (revcomp(seq_i), j), with the same scoring, lanes, width policy, orientation and align options.  The result is R with
+ * strand 1 when R ranks strictly above F, else F with strand 0; the rank is Overflowed > Some(score), ordered by score,
+ * > Unmapped, so every tie (equal scores, both Overflowed, both Unmapped, a palindromic read) goes to the forward strand.
+ * Every output of the winning strand is returned exactly as the single-strand call returns it (score, status, tier,
+ * ranges, CIGAR, hazard): coordinates and CIGAR of a reverse-strand result refer to revcomp(seq_i), as SAM reports a
+ * FLAG 16 record, for profiled_is_query 0 and 1 alike.  A 0-length sequence is Unmapped on strand 0.
+ *   revcomp  reverses the bytes and maps each through one table: A<->T, C<->G, U->A, R<->Y, K<->M, B<->V, D<->H; S, W, N
+ *            map to themselves; lowercase letters map the same way and keep their case; every other byte is unchanged.
+ *   cigar_cap  the capacity the selected strands' CIGARs need; ZOE_CUDA_E_CIGAR_CAP reports that need in cigar_off[0].
+ * The strands are aligned as one doubled batch, so a call takes at most 2^30 - 1 sequences and, for align / ranges /
+ * 3-pass, at most (2^31 - 1) / 2 pairs per device; larger batches fail with ZOE_CUDA_E_BAD_ARG.
+ * zoe_cuda_last_stats counts the work done: pairs and cells count both strands, and the tier / overflowed / unmapped
+ * counters cover all 2 * n * n_profiled strand-pairs. */
+int zoe_cuda_sw_score_both_strands_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_concat, const uint64_t *offsets,
+                                         uint64_t n, uint32_t *score, uint8_t *status, uint8_t *tier, uint8_t *strand);
+int zoe_cuda_sw_score_ranges_both_strands_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_concat, const uint64_t *offsets,
+                                                uint64_t n, uint32_t *score, uint8_t *status, uint8_t *tier,
+                                                uint32_t *ref_start, uint32_t *ref_end, uint32_t *query_start,
+                                                uint32_t *query_end, uint8_t *strand);
+int zoe_cuda_sw_align_both_strands_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_concat, const uint64_t *offsets,
+                                         uint64_t n, uint32_t *score, uint8_t *status, uint8_t *tier, uint32_t *ref_start,
+                                         uint32_t *ref_end, uint32_t *query_start, uint32_t *query_end, uint32_t *cigar,
+                                         uint64_t *cigar_off, uint64_t cigar_cap, uint8_t *hazard, uint8_t *strand);
+int zoe_cuda_sw_align_3pass_both_strands_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_concat, const uint64_t *offsets,
+                                               uint64_t n, uint32_t *score, uint8_t *status, uint8_t *tier,
+                                               uint32_t *ref_start, uint32_t *ref_end, uint32_t *query_start,
+                                               uint32_t *query_end, uint32_t *cigar, uint64_t *cigar_off, uint64_t cigar_cap,
+                                               uint8_t *strand);
+
 /* Batched sneaky_snake(reference, query, threshold) (src/alignment/sneaky_snake.rs:78-131): the SneakySnake
  * pre-alignment filter for pair i = (reference i, query i).  out[i]: 1 = Some(true) (edits within
  * floor(len(query) * threshold)), 0 = Some(false), 2 = None (threshold outside 0..=1, or the length difference exceeds

@@ -74,6 +74,9 @@ struct ScoreAndRanges {
 
 enum class SeqSrc { Query, Reference };
 
+// Which strand of a streamed sequence a both-strand result belongs to (zoe_cuda.h, both-strand search)
+enum class Strand : uint8_t { Forward = 0, Reverse = 1 };
+
 struct WeightMatrix {
     int S = 0;
     std::vector<int8_t> weights;  // S*S, weights[ref_idx][query_idx]
@@ -139,14 +142,81 @@ class CudaProfiles {
 
     // out[i * n_profiled + j] == profiles[j].sw_score_ranges_from_i8(SeqSrc::X(&seqs[i])) (profile_set.rs:313-322)
     std::vector<MaybeAligned<ScoreAndRanges>> sw_score_ranges_batch(const std::vector<std::string> &seqs) {
+        return ranges(seqs, nullptr);
+    }
+
+    std::vector<MaybeAligned<uint32_t>> sw_score_batch(const std::vector<std::string> &seqs) { return scores(seqs, nullptr); }
+
+    // out[i * n_profiled + j] == profiles[j].sw_align_from_i8(SeqSrc::X(&seqs[i])) with X as given at construction
+    std::vector<MaybeAligned<Alignment>> sw_align_batch(const std::vector<std::string> &seqs) { return align(seqs, false); }
+
+    // out[i * n_profiled + j] == profiles[j].sw_align_from_i8_3pass(SeqSrc::X(&seqs[i])) (profile_set.rs:213-231)
+    std::vector<MaybeAligned<Alignment>> sw_align_3pass_batch(const std::vector<std::string> &seqs) { return align(seqs, true); }
+
+    // Both-strand search (zoe_cuda.h): the better of seqs[i] and its reverse complement for every pair, with the strand;
+    // a reverse-strand result's coordinates and CIGAR refer to the reverse complement.
+    std::vector<std::pair<MaybeAligned<uint32_t>, Strand>> sw_score_both_strands(const std::vector<std::string> &seqs) {
+        std::vector<uint8_t> strand;
+        return with_strand(scores(seqs, &strand), strand);
+    }
+    std::vector<std::pair<MaybeAligned<ScoreAndRanges>, Strand>> sw_score_ranges_both_strands(const std::vector<std::string> &seqs) {
+        std::vector<uint8_t> strand;
+        return with_strand(ranges(seqs, &strand), strand);
+    }
+    std::vector<std::pair<MaybeAligned<Alignment>, Strand>> sw_align_both_strands(const std::vector<std::string> &seqs) {
+        std::vector<uint8_t> strand;
+        return with_strand(align(seqs, false, &strand), strand);
+    }
+    std::vector<std::pair<MaybeAligned<Alignment>, Strand>> sw_align_3pass_both_strands(const std::vector<std::string> &seqs) {
+        std::vector<uint8_t> strand;
+        return with_strand(align(seqs, true, &strand), strand);
+    }
+
+  private:
+    template <class T>
+    static std::vector<std::pair<T, Strand>> with_strand(std::vector<T> v, const std::vector<uint8_t> &strand) {
+        std::vector<std::pair<T, Strand>> out;
+        out.reserve(v.size());
+        for (size_t k = 0; k < v.size(); ++k) out.emplace_back(std::move(v[k]), static_cast<Strand>(strand[k]));
+        return out;
+    }
+
+    // strand != nullptr: the both-strand entry point, the strand of every pair into *strand
+    std::vector<MaybeAligned<uint32_t>> scores(const std::vector<std::string> &seqs, std::vector<uint8_t> *strand) {
+        std::vector<uint8_t> buf;
+        std::vector<uint64_t> off;
+        pack(seqs, buf, off);
+        size_t pairs = seqs.size() * targets_.size();
+        std::vector<uint32_t> score(pairs + 1);
+        std::vector<uint8_t> status(pairs + 1), tier(pairs + 1);
+        if (strand) {
+            strand->assign(pairs + 1, 0);
+            check(zoe_cuda_sw_score_both_strands_batch(ctx_, buf.data(), off.data(), seqs.size(), score.data(), status.data(),
+                                                       tier.data(), strand->data()));
+        } else {
+            check(zoe_cuda_sw_score_batch(ctx_, buf.data(), off.data(), seqs.size(), score.data(), status.data(), tier.data()));
+        }
+        std::vector<MaybeAligned<uint32_t>> out(pairs);
+        for (size_t k = 0; k < pairs; ++k) out[k] = {static_cast<Status>(status[k]), score[k]};
+        return out;
+    }
+
+    std::vector<MaybeAligned<ScoreAndRanges>> ranges(const std::vector<std::string> &seqs, std::vector<uint8_t> *strand) {
         std::vector<uint8_t> buf;
         std::vector<uint64_t> off;
         pack(seqs, buf, off);
         size_t pairs = seqs.size() * targets_.size();
         std::vector<uint32_t> score(pairs + 1), rs(pairs + 1), re(pairs + 1), qs(pairs + 1), qe(pairs + 1);
         std::vector<uint8_t> status(pairs + 1), tier(pairs + 1);
-        check(zoe_cuda_sw_score_ranges_batch(ctx_, buf.data(), off.data(), seqs.size(), score.data(), status.data(),
-                                             tier.data(), rs.data(), re.data(), qs.data(), qe.data()));
+        if (strand) {
+            strand->assign(pairs + 1, 0);
+            check(zoe_cuda_sw_score_ranges_both_strands_batch(ctx_, buf.data(), off.data(), seqs.size(), score.data(),
+                                                              status.data(), tier.data(), rs.data(), re.data(), qs.data(),
+                                                              qe.data(), strand->data()));
+        } else {
+            check(zoe_cuda_sw_score_ranges_batch(ctx_, buf.data(), off.data(), seqs.size(), score.data(), status.data(),
+                                                 tier.data(), rs.data(), re.data(), qs.data(), qe.data()));
+        }
         std::vector<MaybeAligned<ScoreAndRanges>> out(pairs);
         for (size_t k = 0; k < pairs; ++k) {
             out[k].status = static_cast<Status>(status[k]);
@@ -155,27 +225,8 @@ class CudaProfiles {
         return out;
     }
 
-    std::vector<MaybeAligned<uint32_t>> sw_score_batch(const std::vector<std::string> &seqs) {
-        std::vector<uint8_t> buf;
-        std::vector<uint64_t> off;
-        pack(seqs, buf, off);
-        size_t pairs = seqs.size() * targets_.size();
-        std::vector<uint32_t> score(pairs + 1);
-        std::vector<uint8_t> status(pairs + 1), tier(pairs + 1);
-        check(zoe_cuda_sw_score_batch(ctx_, buf.data(), off.data(), seqs.size(), score.data(), status.data(), tier.data()));
-        std::vector<MaybeAligned<uint32_t>> out(pairs);
-        for (size_t k = 0; k < pairs; ++k) out[k] = {static_cast<Status>(status[k]), score[k]};
-        return out;
-    }
-
-    // out[i * n_profiled + j] == profiles[j].sw_align_from_i8(SeqSrc::X(&seqs[i])) with X as given at construction
-    std::vector<MaybeAligned<Alignment>> sw_align_batch(const std::vector<std::string> &seqs) { return align(seqs, false); }
-
-    // out[i * n_profiled + j] == profiles[j].sw_align_from_i8_3pass(SeqSrc::X(&seqs[i])) (profile_set.rs:213-231)
-    std::vector<MaybeAligned<Alignment>> sw_align_3pass_batch(const std::vector<std::string> &seqs) { return align(seqs, true); }
-
-  private:
-    std::vector<MaybeAligned<Alignment>> align(const std::vector<std::string> &seqs, bool three_pass) {
+    std::vector<MaybeAligned<Alignment>> align(const std::vector<std::string> &seqs, bool three_pass,
+                                               std::vector<uint8_t> *strand = nullptr) {
         std::vector<uint8_t> buf;
         std::vector<uint64_t> off;
         pack(seqs, buf, off);
@@ -184,7 +235,18 @@ class CudaProfiles {
         std::vector<uint8_t> status(pairs + 1), tier(pairs + 1);
         std::vector<uint64_t> coff(pairs + 2);
         std::vector<uint32_t> cig(16 * pairs + 1024);
+        if (strand) strand->assign(pairs + 1, 0);
         auto call = [&]() {
+            if (strand)
+                return three_pass
+                           ? zoe_cuda_sw_align_3pass_both_strands_batch(ctx_, buf.data(), off.data(), seqs.size(), score.data(),
+                                                                        status.data(), tier.data(), rs.data(), re.data(),
+                                                                        qs.data(), qe.data(), cig.data(), coff.data(),
+                                                                        cig.size(), strand->data())
+                           : zoe_cuda_sw_align_both_strands_batch(ctx_, buf.data(), off.data(), seqs.size(), score.data(),
+                                                                  status.data(), tier.data(), rs.data(), re.data(), qs.data(),
+                                                                  qe.data(), cig.data(), coff.data(), cig.size(), nullptr,
+                                                                  strand->data());
             return three_pass
                        ? zoe_cuda_sw_align_3pass_batch(ctx_, buf.data(), off.data(), seqs.size(), score.data(), status.data(),
                                                        tier.data(), rs.data(), re.data(), qs.data(), qe.data(), cig.data(),
@@ -211,7 +273,7 @@ class CudaProfiles {
                 a.ref_range = {rs[k], re[k]};
                 a.query_range = {qs[k], qe[k]};
                 for (uint64_t w = coff[k]; w < coff[k + 1]; ++w) a.states.push_back({cig[w] >> 4, ops[cig[w] & 7]});
-                bool streamed_is_query = streamed_are_ == SeqSrc::Query;
+                bool streamed_is_query = streamed_are_ == SeqSrc::Query;  // (a sequence and its reverse complement: same length)
                 a.ref_len = (uint32_t)(streamed_is_query ? targets_[j].size() : seqs[i].size());
                 a.query_len = (uint32_t)(streamed_is_query ? seqs[i].size() : targets_[j].size());
             }

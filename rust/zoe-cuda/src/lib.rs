@@ -18,6 +18,13 @@ pub struct CudaProfiles {
 // One context per host thread (like LocalProfiles); it may be moved, not shared.
 unsafe impl Send for CudaProfiles {}
 
+/// Which strand of a streamed sequence a both-strand result belongs to.
+#[derive(Debug, Clone, Copy, PartialEq, Eq)]
+pub enum Strand {
+    Forward = 0,
+    Reverse = 1,
+}
+
 #[derive(Debug)]
 pub enum CudaError {
     Profile(ProfileError),
@@ -87,16 +94,51 @@ impl CudaProfiles {
     /// `out[i * n_profiled + j] == profiles[j].sw_align_from_i8(seq_src(seqs[i]))` where `seq_src` is
     /// `SeqSrc::Query` when the profiled sequences are references, `SeqSrc::Reference` otherwise.
     pub fn sw_align_batch(&self, seqs: &[&[u8]]) -> Result<Vec<MaybeAligned<Alignment<u32>>>, CudaError> {
-        self.align(seqs, false)
+        self.align(seqs, false, None)
     }
 
     /// `out[i * n_profiled + j] == profiles[j].sw_align_from_i8_3pass(seq_src(seqs[i]))` (profile_set.rs:213-231):
     /// ranges from two score passes, then a banded alignment of the bounding box (three_pass.rs:21-104).
     pub fn sw_align_3pass_batch(&self, seqs: &[&[u8]]) -> Result<Vec<MaybeAligned<Alignment<u32>>>, CudaError> {
-        self.align(seqs, true)
+        self.align(seqs, true, None)
     }
 
-    fn align(&self, seqs: &[&[u8]], three_pass: bool) -> Result<Vec<MaybeAligned<Alignment<u32>>>, CudaError> {
+    /// Both-strand search: for every pair, the better of `sw_score_batch` on `seqs[i]` and on its reverse complement
+    /// (Overflowed > Some by score > Unmapped; ties to `Strand::Forward`), with the strand.
+    pub fn sw_score_both_strands_batch(&self, seqs: &[&[u8]]) -> Result<Vec<(MaybeAligned<u32>, Strand)>, CudaError> {
+        let (concat, offsets) = pack(seqs);
+        let pairs = seqs.len() * self.profiled_lens.len();
+        let (mut score, mut status, mut tier, mut sd) = (vec![0u32; pairs], vec![0u8; pairs], vec![0u8; pairs], vec![0u8; pairs]);
+        self.check(unsafe {
+            sys::zoe_cuda_sw_score_both_strands_batch(self.ctx, concat.as_ptr(), offsets.as_ptr(), seqs.len() as u64,
+                                                      score.as_mut_ptr(), status.as_mut_ptr(), tier.as_mut_ptr(), sd.as_mut_ptr())
+        }, 0, 0)?;
+        Ok(score.iter().zip(&status).zip(&sd).map(|((&s, &st), &d)| (maybe(st, s), strand(d))).collect())
+    }
+
+    /// Both-strand `sw_score_ranges_batch`; a reverse-strand result's ranges refer to the reverse complement.
+    pub fn sw_score_ranges_both_strands_batch(&self, seqs: &[&[u8]]) -> Result<Vec<(MaybeAligned<ScoreAndRanges<u32>>, Strand)>, CudaError> {
+        let mut sd = vec![0u8; seqs.len() * self.profiled_lens.len()];
+        let out = self.ranges(seqs, Some(&mut sd))?;
+        Ok(out.into_iter().zip(sd).map(|(m, d)| (m, strand(d))).collect())
+    }
+
+    /// Both-strand `sw_align_batch`; a reverse-strand result's ranges and CIGAR refer to the reverse complement (SAM FLAG 16).
+    pub fn sw_align_both_strands_batch(&self, seqs: &[&[u8]]) -> Result<Vec<(MaybeAligned<Alignment<u32>>, Strand)>, CudaError> {
+        let mut sd = vec![0u8; seqs.len() * self.profiled_lens.len()];
+        let out = self.align(seqs, false, Some(&mut sd))?;
+        Ok(out.into_iter().zip(sd).map(|(m, d)| (m, strand(d))).collect())
+    }
+
+    /// Both-strand `sw_align_3pass_batch`.
+    pub fn sw_align_3pass_both_strands_batch(&self, seqs: &[&[u8]]) -> Result<Vec<(MaybeAligned<Alignment<u32>>, Strand)>, CudaError> {
+        let mut sd = vec![0u8; seqs.len() * self.profiled_lens.len()];
+        let out = self.align(seqs, true, Some(&mut sd))?;
+        Ok(out.into_iter().zip(sd).map(|(m, d)| (m, strand(d))).collect())
+    }
+
+    /// `strand`: the both-strand entry points, the strand of every pair written there.
+    fn align(&self, seqs: &[&[u8]], three_pass: bool, mut strand: Option<&mut Vec<u8>>) -> Result<Vec<MaybeAligned<Alignment<u32>>>, CudaError> {
         let (concat, offsets) = pack(seqs);
         let np = self.profiled_lens.len();
         let pairs = seqs.len() * np;
@@ -107,7 +149,19 @@ impl CudaProfiles {
         let mut cigar = vec![0u32; 16 * pairs + 1024];
         loop {
             let rc = unsafe {
-                if three_pass {
+                if let Some(sd) = strand.as_deref_mut() {
+                    if three_pass {
+                        sys::zoe_cuda_sw_align_3pass_both_strands_batch(self.ctx, concat.as_ptr(), offsets.as_ptr(), seqs.len() as u64,
+                            score.as_mut_ptr(), status.as_mut_ptr(), tier.as_mut_ptr(), rs.as_mut_ptr(), re.as_mut_ptr(),
+                            qs.as_mut_ptr(), qe.as_mut_ptr(), cigar.as_mut_ptr(), coff.as_mut_ptr(), cigar.len() as u64,
+                            sd.as_mut_ptr())
+                    } else {
+                        sys::zoe_cuda_sw_align_both_strands_batch(self.ctx, concat.as_ptr(), offsets.as_ptr(), seqs.len() as u64,
+                            score.as_mut_ptr(), status.as_mut_ptr(), tier.as_mut_ptr(), rs.as_mut_ptr(), re.as_mut_ptr(),
+                            qs.as_mut_ptr(), qe.as_mut_ptr(), cigar.as_mut_ptr(), coff.as_mut_ptr(), cigar.len() as u64,
+                            std::ptr::null_mut(), sd.as_mut_ptr())
+                    }
+                } else if three_pass {
                     sys::zoe_cuda_sw_align_3pass_batch(self.ctx, concat.as_ptr(), offsets.as_ptr(), seqs.len() as u64,
                         score.as_mut_ptr(), status.as_mut_ptr(), tier.as_mut_ptr(), rs.as_mut_ptr(), re.as_mut_ptr(),
                         qs.as_mut_ptr(), qe.as_mut_ptr(), cigar.as_mut_ptr(), coff.as_mut_ptr(), cigar.len() as u64)
@@ -155,15 +209,25 @@ impl CudaProfiles {
     /// `out[i * n_profiled + j] == profiles[j].sw_score_ranges_from_i8(seq_src(seqs[i]))`
     /// (profile_set.rs:313-322): score plus 0-based half-open ranges, no traceback matrix.
     pub fn sw_score_ranges_batch(&self, seqs: &[&[u8]]) -> Result<Vec<MaybeAligned<ScoreAndRanges<u32>>>, CudaError> {
+        self.ranges(seqs, None)
+    }
+
+    /// `strand`: the both-strand entry point, the strand of every pair written there.
+    fn ranges(&self, seqs: &[&[u8]], strand: Option<&mut Vec<u8>>) -> Result<Vec<MaybeAligned<ScoreAndRanges<u32>>>, CudaError> {
         let (concat, offsets) = pack(seqs);
         let pairs = seqs.len() * self.profiled_lens.len();
         let mut score = vec![0u32; pairs];
         let (mut status, mut tier) = (vec![0u8; pairs], vec![0u8; pairs]);
         let (mut rs, mut re, mut qs, mut qe) = (vec![0u32; pairs], vec![0u32; pairs], vec![0u32; pairs], vec![0u32; pairs]);
         self.check(unsafe {
-            sys::zoe_cuda_sw_score_ranges_batch(self.ctx, concat.as_ptr(), offsets.as_ptr(), seqs.len() as u64,
-                score.as_mut_ptr(), status.as_mut_ptr(), tier.as_mut_ptr(), rs.as_mut_ptr(), re.as_mut_ptr(),
-                qs.as_mut_ptr(), qe.as_mut_ptr())
+            match strand {
+                Some(sd) => sys::zoe_cuda_sw_score_ranges_both_strands_batch(self.ctx, concat.as_ptr(), offsets.as_ptr(),
+                    seqs.len() as u64, score.as_mut_ptr(), status.as_mut_ptr(), tier.as_mut_ptr(), rs.as_mut_ptr(),
+                    re.as_mut_ptr(), qs.as_mut_ptr(), qe.as_mut_ptr(), sd.as_mut_ptr()),
+                None => sys::zoe_cuda_sw_score_ranges_batch(self.ctx, concat.as_ptr(), offsets.as_ptr(), seqs.len() as u64,
+                    score.as_mut_ptr(), status.as_mut_ptr(), tier.as_mut_ptr(), rs.as_mut_ptr(), re.as_mut_ptr(),
+                    qs.as_mut_ptr(), qe.as_mut_ptr()),
+            }
         }, 0, 0)?;
         Ok((0..pairs).map(|k| match status[k] {
             sys::ZOE_CUDA_SOME => MaybeAligned::Some(ScoreAndRanges {
@@ -250,6 +314,10 @@ fn maybe(status: u8, score: u32) -> MaybeAligned<u32> {
         sys::ZOE_CUDA_OVERFLOWED => MaybeAligned::Overflowed,
         _ => MaybeAligned::Unmapped,
     }
+}
+
+fn strand(v: u8) -> Strand {
+    if v == 1 { Strand::Reverse } else { Strand::Forward }
 }
 
 fn pack(seqs: &[&[u8]]) -> (Vec<u8>, Vec<u64>) {

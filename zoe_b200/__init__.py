@@ -10,7 +10,9 @@ from .alignment import (  # noqa: F401
     ProfileError,
     ScoreAndRanges,
     SeqSrc,
+    Strand,
     ZoeCudaError,
+    reverse_complement,
 )
 from .sneaky_snake import SneakySnake  # noqa: F401
 from .matrices import (  # noqa: F401

@@ -20,6 +20,8 @@ SYMBOLS = [
     "zoe_cuda_last_stats", "zoe_cuda_dpx_peak", "zoe_cuda_stream", "zoe_cuda_set_align_options", "zoe_cuda_set_width_policy",
     "zoe_cuda_sw_score_ranges_batch", "zoe_cuda_run_ranges_staged", "zoe_cuda_sw_align_3pass_batch",
     "zoe_cuda_run_3pass_staged", "zoe_cuda_sneaky_snake_batch", "zoe_cuda_set_memory_budget",
+    "zoe_cuda_sw_score_both_strands_batch", "zoe_cuda_sw_score_ranges_both_strands_batch",
+    "zoe_cuda_sw_align_both_strands_batch", "zoe_cuda_sw_align_3pass_both_strands_batch",
 ]
 
 
@@ -66,6 +68,10 @@ def load() -> C.CDLL:
     lib.zoe_cuda_sw_align_3pass_batch.argtypes = [p, u8p, u64p, C.c_uint64, u32p, u8p, u8p, u32p, u32p, u32p, u32p, u32p,
                                                   u64p, C.c_uint64]
     lib.zoe_cuda_run_3pass_staged.argtypes = [p]
+    lib.zoe_cuda_sw_score_both_strands_batch.argtypes = lib.zoe_cuda_sw_score_batch.argtypes + [u8p]
+    lib.zoe_cuda_sw_score_ranges_both_strands_batch.argtypes = lib.zoe_cuda_sw_score_ranges_batch.argtypes + [u8p]
+    lib.zoe_cuda_sw_align_both_strands_batch.argtypes = lib.zoe_cuda_sw_align_batch.argtypes + [u8p]
+    lib.zoe_cuda_sw_align_3pass_both_strands_batch.argtypes = lib.zoe_cuda_sw_align_3pass_batch.argtypes + [u8p]
     lib.zoe_cuda_sneaky_snake_batch.argtypes = [p, u8p, u64p, u8p, u64p, C.c_uint64, C.c_float, u8p]
     lib.zoe_cuda_stage_streamed.argtypes = [p, u8p, u64p, C.c_uint64]
     lib.zoe_cuda_run_score_staged.argtypes = [p]

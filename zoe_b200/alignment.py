@@ -125,6 +125,31 @@ class ScoreAndRanges:
 _CIGAR_OPS = {0: "M", 1: "I", 2: "D", 4: "S"}
 
 
+class Strand(Enum):
+    """Which strand of a streamed sequence a both-strand result belongs to."""
+
+    Forward = 0
+    Reverse = 1
+
+
+def _complement_table() -> bytes:
+    # the Python copy of the device table (csrc/strands.cuh, complement_base)
+    t = bytearray(range(256))
+    for a, b in (b"AT", b"TA", b"UA", b"CG", b"GC", b"RY", b"YR", b"KM", b"MK", b"BV", b"VB", b"DH", b"HD"):
+        t[a] = b
+        t[a | 0x20] = b | 0x20
+    return bytes(t)
+
+
+_COMPLEMENT = _complement_table()
+
+
+def reverse_complement(seq: bytes) -> bytes:
+    """The reverse complement the both-strand search aligns: bytes reversed, each mapped through the complement table
+    (A<->T, C<->G, U->A, R<->Y, K<->M, B<->V, D<->H; S, W, N and every other byte unchanged; lowercase keeps its case)."""
+    return bytes(seq).translate(_COMPLEMENT)[::-1]
+
+
 def _pack(seqs: Sequence[bytes]):
     offs = np.zeros(len(seqs) + 1, dtype=np.uint64)
     if len(seqs):
@@ -248,6 +273,22 @@ class CudaProfiles:
         shape = (n, self.n_profiled)
         return score[:pairs].reshape(shape), status[:pairs].reshape(shape), tier[:pairs].reshape(shape)
 
+    def sw_score_both_strands_arrays(self, buf: np.ndarray, offs: np.ndarray):
+        """:meth:`sw_score_arrays` of the both-strand search: (score, status, tier, strand), each ``[n, n_profiled]``;
+        strand 0 = the sequence as given won, 1 = its reverse complement."""
+        n = len(offs) - 1
+        pairs = n * self.n_profiled
+        score = np.zeros(max(pairs, 1), dtype=np.uint32)
+        status = np.zeros(max(pairs, 1), dtype=np.uint8)
+        tier = np.zeros(max(pairs, 1), dtype=np.uint8)
+        strand = np.zeros(max(pairs, 1), dtype=np.uint8)
+        self._check(self._lib.zoe_cuda_sw_score_both_strands_batch(
+            self._h, _p(buf, C.c_uint8), _p(offs, C.c_uint64), n, _p(score, C.c_uint32), _p(status, C.c_uint8),
+            _p(tier, C.c_uint8), _p(strand, C.c_uint8)))
+        shape = (n, self.n_profiled)
+        return (score[:pairs].reshape(shape), status[:pairs].reshape(shape), tier[:pairs].reshape(shape),
+                strand[:pairs].reshape(shape))
+
     def sw_score_into(self, buf: np.ndarray, offs: np.ndarray, score: np.ndarray, status: np.ndarray, tier: np.ndarray):
         """Like :meth:`sw_score_arrays` but writes into caller-owned (ideally pinned) output arrays."""
         self._check(self._lib.zoe_cuda_sw_score_batch(self._h, _p(buf, C.c_uint8), _p(offs, C.c_uint64), len(offs) - 1,
@@ -294,6 +335,15 @@ class CudaProfiles:
     def align_arrays(self, buf: np.ndarray, offs: np.ndarray, cigar_cap: Optional[int] = None, three_pass: bool = False):
         """Alignments for a packed batch; returns a dict of flat arrays (pair index = i*n_profiled+j).
         ``three_pass``: ``sw_align_from_i8_3pass`` (ranges + banded box alignment) instead of ``sw_align_from_i8``."""
+        return self._align_arrays(buf, offs, cigar_cap, three_pass, both_strands=False)
+
+    def align_both_strands_arrays(self, buf: np.ndarray, offs: np.ndarray, cigar_cap: Optional[int] = None,
+                                  three_pass: bool = False):
+        """:meth:`align_arrays` of the both-strand search: every pair's better strand, plus a ``"strand"`` array
+        (0 forward, 1 reverse complement; a reverse result's ranges and CIGAR refer to the reverse complement)."""
+        return self._align_arrays(buf, offs, cigar_cap, three_pass, both_strands=True)
+
+    def _align_arrays(self, buf, offs, cigar_cap, three_pass: bool, both_strands: bool):
         n = len(offs) - 1
         pairs = max(n * self.n_profiled, 1)
         out = {
@@ -303,6 +353,8 @@ class CudaProfiles:
             "query_end": np.zeros(pairs, dtype=np.uint32), "cigar_off": np.zeros(pairs + 1, dtype=np.uint64),
             "hazard": np.zeros(pairs, dtype=np.uint8),
         }
+        if both_strands:
+            out["strand"] = np.zeros(pairs, dtype=np.uint8)
         cap = int(cigar_cap) if cigar_cap else max(16 * pairs, 1024)
         for _ in range(2):
             out["cigar"] = np.zeros(cap, dtype=np.uint32)
@@ -317,16 +369,23 @@ class CudaProfiles:
         return out
 
     def _align_call(self, buf: np.ndarray, offs: np.ndarray, out: dict, three_pass: bool) -> int:
+        """One align / 3-pass call into ``out``; the both-strand entry point when ``out`` has a ``"strand"`` array."""
         args = [self._h, _p(buf, C.c_uint8), _p(offs, C.c_uint64), len(offs) - 1, _p(out["score"], C.c_uint32),
                 _p(out["status"], C.c_uint8), _p(out["tier"], C.c_uint8), _p(out["ref_start"], C.c_uint32),
                 _p(out["ref_end"], C.c_uint32), _p(out["query_start"], C.c_uint32), _p(out["query_end"], C.c_uint32),
                 _p(out["cigar"], C.c_uint32), _p(out["cigar_off"], C.c_uint64), len(out["cigar"])]
+        if "strand" in out:
+            strand = _p(out["strand"], C.c_uint8)
+            if three_pass:
+                return self._lib.zoe_cuda_sw_align_3pass_both_strands_batch(*args, strand)
+            return self._lib.zoe_cuda_sw_align_both_strands_batch(*args, _p(out["hazard"], C.c_uint8), strand)
         if three_pass:
             return self._lib.zoe_cuda_sw_align_3pass_batch(*args)
         return self._lib.zoe_cuda_sw_align_batch(*args, _p(out["hazard"], C.c_uint8))
 
     def align_into(self, buf: np.ndarray, offs: np.ndarray, out: dict, three_pass: bool = False):
-        """Like :meth:`align_arrays` but into caller-owned (ideally pinned) arrays; ``out['cigar']`` is the capacity."""
+        """Like :meth:`align_arrays` but into caller-owned (ideally pinned) arrays; ``out['cigar']`` is the capacity.
+        With a ``"strand"`` array in ``out``, the both-strand search (:meth:`align_both_strands_arrays`)."""
         self._check(self._align_call(buf, offs, out, three_pass))
 
     def run_3pass_staged(self):
@@ -334,22 +393,32 @@ class CudaProfiles:
 
     def ranges_arrays(self, buf: np.ndarray, offs: np.ndarray):
         """``sw_score_ranges`` for a packed batch: dict of flat arrays (pair index = i*n_profiled+j)."""
+        return self._ranges_arrays(buf, offs, both_strands=False)
+
+    def ranges_both_strands_arrays(self, buf: np.ndarray, offs: np.ndarray):
+        """:meth:`ranges_arrays` of the both-strand search, plus a ``"strand"`` array (0 forward, 1 reverse complement)."""
+        return self._ranges_arrays(buf, offs, both_strands=True)
+
+    def _ranges_arrays(self, buf: np.ndarray, offs: np.ndarray, both_strands: bool):
         n = len(offs) - 1
         pairs = max(n * self.n_profiled, 1)
         out = {k: np.zeros(pairs, dtype=np.uint32) for k in ("score", "ref_start", "ref_end", "query_start", "query_end")}
         out.update({k: np.zeros(pairs, dtype=np.uint8) for k in ("status", "tier")})
-        self._check(self._lib.zoe_cuda_sw_score_ranges_batch(
-            self._h, _p(buf, C.c_uint8), _p(offs, C.c_uint64), n, _p(out["score"], C.c_uint32),
-            _p(out["status"], C.c_uint8), _p(out["tier"], C.c_uint8), _p(out["ref_start"], C.c_uint32),
-            _p(out["ref_end"], C.c_uint32), _p(out["query_start"], C.c_uint32), _p(out["query_end"], C.c_uint32)))
+        if both_strands:
+            out["strand"] = np.zeros(pairs, dtype=np.uint8)
+        self.ranges_into(buf, offs, out)
         return out
 
     def ranges_into(self, buf: np.ndarray, offs: np.ndarray, out: dict):
-        """Like :meth:`ranges_arrays` but into caller-owned (ideally pinned) arrays."""
-        self._check(self._lib.zoe_cuda_sw_score_ranges_batch(
-            self._h, _p(buf, C.c_uint8), _p(offs, C.c_uint64), len(offs) - 1, _p(out["score"], C.c_uint32),
-            _p(out["status"], C.c_uint8), _p(out["tier"], C.c_uint8), _p(out["ref_start"], C.c_uint32),
-            _p(out["ref_end"], C.c_uint32), _p(out["query_start"], C.c_uint32), _p(out["query_end"], C.c_uint32)))
+        """Like :meth:`ranges_arrays` but into caller-owned (ideally pinned) arrays.  With a ``"strand"`` array in
+        ``out``, the both-strand search (:meth:`ranges_both_strands_arrays`)."""
+        args = [self._h, _p(buf, C.c_uint8), _p(offs, C.c_uint64), len(offs) - 1, _p(out["score"], C.c_uint32),
+                _p(out["status"], C.c_uint8), _p(out["tier"], C.c_uint8), _p(out["ref_start"], C.c_uint32),
+                _p(out["ref_end"], C.c_uint32), _p(out["query_start"], C.c_uint32), _p(out["query_end"], C.c_uint32)]
+        if "strand" in out:
+            self._check(self._lib.zoe_cuda_sw_score_ranges_both_strands_batch(*args, _p(out["strand"], C.c_uint8)))
+        else:
+            self._check(self._lib.zoe_cuda_sw_score_ranges_batch(*args))
 
     def run_ranges_staged(self):
         self._check(self._lib.zoe_cuda_run_ranges_staged(self._h))
@@ -357,16 +426,21 @@ class CudaProfiles:
     def sw_score_ranges_batch(self, src: "SeqSrc"):
         """``out[i][j] == profiles[j].sw_score_ranges_from_i8(SeqSrc::X(seqs[i]))`` as
         ``MaybeAligned[ScoreAndRanges]`` (profile_set.rs:313-322)."""
-        want_pq = src.kind == "Reference"
+        self._check_src(src)
+        seqs = [bytes(s) for s in src.seq]
+        buf, offs = _pack(seqs)
+        return self._ranges_rows(len(seqs), self.ranges_arrays(buf, offs))
+
+    def _check_src(self, src: "SeqSrc"):
+        want_pq = src.kind == "Reference"  # streamed sequences are references <=> profiled are queries
         if want_pq != self.profiled_is_query:
             raise ValueError(
                 f"this CudaProfiles was built with profiled_is_query={self.profiled_is_query}; "
                 f"SeqSrc.{src.kind} needs the opposite orientation")
-        seqs = [bytes(s) for s in src.seq]
-        buf, offs = _pack(seqs)
-        a = self.ranges_arrays(buf, offs)
+
+    def _ranges_rows(self, n: int, a: dict):
         out = []
-        for i in range(len(seqs)):
+        for i in range(n):
             row = []
             for j in range(self.n_profiled):
                 k = i * self.n_profiled + j
@@ -406,14 +480,12 @@ class CudaProfiles:
 
     def sw_align_batch(self, src: SeqSrc, three_pass: bool = False):
         """``out[i][j] == profiles[j].sw_align_from_i8(SeqSrc::X(seqs[i]))`` for the SeqSrc given."""
-        want_pq = src.kind == "Reference"  # streamed sequences are references <=> profiled are queries
-        if want_pq != self.profiled_is_query:
-            raise ValueError(
-                f"this CudaProfiles was built with profiled_is_query={self.profiled_is_query}; "
-                f"SeqSrc.{src.kind} needs the opposite orientation")
+        self._check_src(src)
         seqs = [bytes(s) for s in src.seq]
         buf, offs = _pack(seqs)
-        a = self.align_arrays(buf, offs, three_pass=three_pass)
+        return self._alignment_rows(seqs, self.align_arrays(buf, offs, three_pass=three_pass))
+
+    def _alignment_rows(self, seqs: Sequence[bytes], a: dict):
         out = []
         for i in range(len(seqs)):
             row = []
@@ -435,3 +507,36 @@ class CudaProfiles:
                     (int(a["query_start"][k]), int(a["query_end"][k])), cig, ref_len, query_len)))
             out.append(row)
         return out
+
+    # ---- both-strand search: every streamed sequence and its reverse complement, the better strand per pair ----
+    def _with_strand(self, rows, strand: np.ndarray):
+        return [[(m, Strand(int(strand[i * self.n_profiled + j]))) for j, m in enumerate(row)] for i, row in enumerate(rows)]
+
+    def sw_score_both_strands_batch(self, seqs: Sequence[bytes]):
+        """``[[(MaybeAligned[int], Strand)]]``: the better of ``sw_score_batch([s])`` and
+        ``sw_score_batch([reverse_complement(s)])`` per pair; ties go to ``Strand.Forward``."""
+        buf, offs = _pack([bytes(s) for s in seqs])
+        score, status, _, strand = self.sw_score_both_strands_arrays(buf, offs)
+        return [[(self._maybe(int(status[i, j]), int(score[i, j])), Strand(int(strand[i, j])))
+                 for j in range(self.n_profiled)] for i in range(len(seqs))]
+
+    def sw_score_ranges_both_strands_batch(self, src: "SeqSrc"):
+        """``[[(MaybeAligned[ScoreAndRanges], Strand)]]``; a reverse result's ranges refer to the reverse complement."""
+        self._check_src(src)
+        seqs = [bytes(s) for s in src.seq]
+        buf, offs = _pack(seqs)
+        a = self.ranges_both_strands_arrays(buf, offs)
+        return self._with_strand(self._ranges_rows(len(seqs), a), a["strand"])
+
+    def sw_align_both_strands_batch(self, src: SeqSrc, three_pass: bool = False):
+        """``[[(MaybeAligned[Alignment], Strand)]]``: the better strand of every pair, aligned as the single-strand
+        call aligns it; a reverse result's ranges and CIGAR refer to the reverse complement (SAM FLAG 16)."""
+        self._check_src(src)
+        seqs = [bytes(s) for s in src.seq]
+        buf, offs = _pack(seqs)
+        a = self.align_both_strands_arrays(buf, offs, three_pass=three_pass)
+        return self._with_strand(self._alignment_rows(seqs, a), a["strand"])
+
+    def sw_align_3pass_both_strands_batch(self, src: SeqSrc):
+        """The 3-pass alignment (:meth:`sw_align_3pass_batch`) of the both-strand search."""
+        return self.sw_align_both_strands_batch(src, three_pass=True)

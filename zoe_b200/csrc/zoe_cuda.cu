@@ -33,6 +33,7 @@
 #include "sw_ranges.cuh"
 #include "sw_3pass.cuh"
 #include "sneaky_snake.cuh"
+#include "strands.cuh"
 
 using namespace zoe_cuda;
 
@@ -113,6 +114,9 @@ struct Device {
     uint64_t cig_total = 0;
     // long-row score path
     DevBuf long_ids, long_bnd, long_queue;
+    // both-strand search (strands.cuh): the doubled batch is built here and swapped into rseq / roff; the selected
+    // strand's per-pair outputs are gathered into the sel_* buffers and swapped into the ones the fetch paths read
+    DevBuf xs_seq, xs_off, strand, sel32[5], sel8[3], sel_cig_count, sel_cig_off, sel_cig_out, sel_ctr;
     uint64_t n_first = 0, n_count = 0;  // shard of the streamed batch owned by this device
     uint64_t rseq_bytes = 0;
     bool timed_kernel = false;
@@ -2676,6 +2680,435 @@ int fetch_alignments(zoe_cuda_ctx *ctx, uint32_t *score, uint8_t *status, uint8_
     return 0;
 }
 
+// Queues the D2H copies of a device's score outputs behind its kernels (score entry points).
+int queue_score_d2h(zoe_cuda_ctx *ctx, Device &d, uint32_t *score, uint8_t *status, uint8_t *tier) {
+    if (d.n_count == 0) return 0;
+    CU(ctx, cudaSetDevice(d.id));
+    size_t first = (size_t)d.n_first * ctx->n_prof, pairs = (size_t)d.n_count * ctx->n_prof;
+    if (score)
+        CU(ctx, cudaMemcpyAsync(score + first, d.score.p, pairs * sizeof(uint32_t), cudaMemcpyDeviceToHost, d.stream));
+    if (status) CU(ctx, cudaMemcpyAsync(status + first, d.status.p, pairs, cudaMemcpyDeviceToHost, d.stream));
+    if (tier) CU(ctx, cudaMemcpyAsync(tier + first, d.tier.p, pairs, cudaMemcpyDeviceToHost, d.stream));
+    return 0;
+}
+
+// Queues the D2H copies of every device's ranges outputs (ranges entry points).
+int queue_ranges_d2h(zoe_cuda_ctx *ctx, uint32_t *score, uint8_t *status, uint8_t *tier, uint32_t *ref_start,
+                     uint32_t *ref_end, uint32_t *query_start, uint32_t *query_end) {
+    for (Device &d : ctx->devs) {
+        if (d.n_count == 0) continue;
+        CU(ctx, cudaSetDevice(d.id));
+        size_t first = (size_t)d.n_first * ctx->n_prof, pairs = (size_t)d.n_count * ctx->n_prof;
+        auto d2h = [&](void *dst, const DevBuf &src, size_t elem) -> cudaError_t {
+            if (!dst) return cudaSuccess;
+            return cudaMemcpyAsync((uint8_t *)dst + first * elem, src.p, pairs * elem, cudaMemcpyDeviceToHost, d.stream);
+        };
+        CU(ctx, d2h(score, d.score, 4));
+        CU(ctx, d2h(status, d.status, 1));
+        CU(ctx, d2h(tier, d.tier, 1));
+        CU(ctx, d2h(ref_start, d.ref_start, 4));
+        CU(ctx, d2h(ref_end, d.ref_end, 4));
+        CU(ctx, d2h(query_start, d.query_start, 4));
+        CU(ctx, d2h(query_end, d.query_end, 4));
+    }
+    return 0;
+}
+
+// ---------------------------------------------------------------------------------------------
+// both-strand search (strands.cuh, DESIGN.md 4.8): stage -> strand expansion -> the unchanged pipelines on the doubled
+// batch -> strand selection -> the unchanged fetch paths on the real shard
+// ---------------------------------------------------------------------------------------------
+// While a both-strand call runs its pipelines, the host bookkeeping describes the doubled, interleaved batch the
+// expansion kernel built (count, cells, per-sequence lengths, every device's shard); the rest of the call sees the real
+// batch.  The destructor restores the real batch, leaves nothing "staged" (the device holds a doubled batch), and on
+// an error return drains every stream so that no copy from the caller's buffers is still in flight.
+struct DoubledView {
+    zoe_cuda_ctx *ctx;
+    bool doubled = false, ok = false;
+    std::vector<uint32_t> real_len;
+    explicit DoubledView(zoe_cuda_ctx *c) : ctx(c) {}
+    DoubledView(const DoubledView &) = delete;
+    DoubledView &operator=(const DoubledView &) = delete;
+    void enter() {
+        ctx->staged_n *= 2;
+        ctx->staged_cells *= 2;
+        real_len.swap(ctx->staged_len);
+        ctx->staged_len.resize(2 * real_len.size());
+        for (size_t i = 0; i < real_len.size(); ++i) ctx->staged_len[2 * i] = ctx->staged_len[2 * i + 1] = real_len[i];
+        for (Device &d : ctx->devs) {
+            d.n_first *= 2;
+            d.n_count *= 2;
+        }
+        doubled = true;
+    }
+    void leave() {
+        if (!doubled) return;
+        ctx->staged_n /= 2;
+        ctx->staged_cells /= 2;
+        ctx->staged_len.swap(real_len);
+        for (Device &d : ctx->devs) {
+            d.n_first /= 2;
+            d.n_count /= 2;
+        }
+        doubled = false;
+    }
+    ~DoubledView() {
+        leave();
+        ctx->staged = false;
+        if (ok) return;
+        for (Device &d : ctx->devs) {
+            cudaSetDevice(d.id);
+            if (d.copy_stream) cudaStreamSynchronize(d.copy_stream);
+            cudaStreamSynchronize(d.stream);
+            d.copy_pending = false;
+        }
+    }
+};
+
+// Checks the doubled batch against the single-strand limits (sequences per call; with pair_limit, pairs per device for
+// the align / ranges / 3-pass pipelines), before anything is queued.
+int check_both_strands_limits(zoe_cuda_ctx *ctx, uint64_t n, bool pair_limit) {
+    if (n >= 0x7fffffffULL / 2 + 1)
+        return fail(ctx, ZOE_CUDA_E_BAD_ARG, "batch too large: a both-strand search doubles the batch, so it takes at most "
+                    "%llu sequences (half the single-strand limit)", 0x7fffffffULL / 2);
+    if (pair_limit && ctx->have_profiled) {
+        shard(ctx, n);
+        for (Device &d : ctx->devs)
+            if (2 * d.n_count * ctx->n_prof >= 0x7fffffffULL)
+                return fail(ctx, ZOE_CUDA_E_BAD_ARG, "too many pairs: a both-strand search doubles the pairs of a device "
+                            "(%llu) past the %llu of one call; halve the batch",
+                            (unsigned long long)(2 * d.n_count * ctx->n_prof), 0x7fffffffULL - 1);
+    }
+    return 0;
+}
+
+// Queues the strand expansion of the device's staged shard and swaps the doubled batch into rseq / roff.  The pair
+// buffers staging sized for the real shard are grown for the doubled one.
+int expand_strands(zoe_cuda_ctx *ctx, Device &d) {
+    if (d.n_count == 0) return 0;
+    CU(ctx, cudaSetDevice(d.id));
+    CU(ctx, d.xs_seq.reserve(2 * d.rseq_bytes + 16));
+    CU(ctx, d.xs_off.reserve((2 * d.n_count + 1) * sizeof(uint64_t)));
+    const uint32_t blocks = (uint32_t)std::min<uint64_t>((d.n_count + 7) / 8, (uint64_t)d.sm_count * 16);
+    strand_expand_kernel<<<blocks, 256, 0, d.stream>>>(d.rseq.as<uint8_t>(), d.roff.as<uint64_t>(), d.n_count,
+                                                       d.xs_seq.as<uint8_t>(), d.xs_off.as<uint64_t>());
+    CU(ctx, cudaGetLastError());
+    ctx->last_launches++;
+    std::swap(d.rseq, d.xs_seq);
+    std::swap(d.roff, d.xs_off);
+    d.rseq_bytes *= 2;
+    const size_t pairs = (size_t)2 * d.n_count * ctx->n_prof;
+    CU(ctx, d.best.reserve(pairs * sizeof(int32_t)));
+    CU(ctx, d.score.reserve(pairs * sizeof(uint32_t)));
+    CU(ctx, d.status.reserve(pairs));
+    CU(ctx, d.tier.reserve(pairs));
+    CU(ctx, d.wide_ids.reserve((2 * d.n_count + 1) * sizeof(uint32_t)));
+    return 0;
+}
+
+// Stages a both-strand batch (one upload: the expansion needs the whole shard), expands it on every device and switches
+// the host bookkeeping to the doubled view.
+int stage_both_strands(zoe_cuda_ctx *ctx, DoubledView &view, const uint8_t *concat, const uint64_t *offsets, uint64_t n,
+                       bool pair_limit) {
+    int rc = check_both_strands_limits(ctx, n, pair_limit);
+    if (rc) return rc;
+    rc = stage_on_devices(ctx, concat, offsets, n, /*split=*/false);
+    if (rc) return rc;
+    for (Device &d : ctx->devs) {
+        rc = expand_strands(ctx, d);
+        if (rc) return rc;
+    }
+    view.enter();
+    return 0;
+}
+
+enum class StrandOutputs { Score, Ranges, Align, ThreePass };
+
+// Strand selection on one device (doubled view): gathers the selected strand's per-pair outputs into the buffers the
+// fetch paths read and writes d.strand.  For the alignments, also the selected CIGAR lengths and their offsets
+// (sel_cig_count -> sel_cig_off, the CIGAR offset scan of the align pipeline); *cig_need gets the selected total.
+int select_strands(zoe_cuda_ctx *ctx, Device &d, StrandOutputs kind, uint64_t *cig_need) {
+    *cig_need = 0;
+    const uint64_t n_out = d.n_count / 2 * ctx->n_prof;
+    if (n_out == 0) return 0;
+    CU(ctx, cudaSetDevice(d.id));
+    const bool cig = kind == StrandOutputs::Align || kind == StrandOutputs::ThreePass;
+    StrandSelectParams p{};
+    DevBuf *b32[5] = {&d.score, &d.ref_start, &d.ref_end, &d.query_start, &d.query_end};
+    DevBuf *b8[3] = {&d.status, &d.tier, &d.hazard};
+    p.n32 = kind == StrandOutputs::Score ? 1 : 5;
+    p.n8 = kind == StrandOutputs::Align ? 3 : 2;
+    for (int k = 0; k < p.n32; ++k) {
+        CU(ctx, d.sel32[k].reserve(n_out * sizeof(uint32_t)));
+        p.in32[k] = b32[k]->as<uint32_t>();
+        p.out32[k] = d.sel32[k].as<uint32_t>();
+    }
+    for (int k = 0; k < p.n8; ++k) {
+        CU(ctx, d.sel8[k].reserve(n_out));
+        p.in8[k] = b8[k]->as<uint8_t>();
+        p.out8[k] = d.sel8[k].as<uint8_t>();
+    }
+    CU(ctx, d.strand.reserve(n_out));
+    p.strand = d.strand.as<uint8_t>();
+    p.n_out = n_out;
+    p.n_prof = ctx->n_prof;
+    if (cig) {
+        CU(ctx, d.sel_cig_count.reserve(n_out * sizeof(uint32_t)));
+        p.cig_off = d.cig_off.as<uint64_t>();
+        p.cig_count = d.sel_cig_count.as<uint32_t>();
+    }
+    strand_select_kernel<<<(uint32_t)((n_out + 255) / 256), 256, 0, d.stream>>>(p);
+    CU(ctx, cudaGetLastError());
+    ctx->last_launches++;
+    for (int k = 0; k < p.n32; ++k) std::swap(*b32[k], d.sel32[k]);
+    for (int k = 0; k < p.n8; ++k) std::swap(*b8[k], d.sel8[k]);
+    if (!cig) return 0;
+    CU(ctx, d.sel_cig_off.reserve((n_out + 1) * sizeof(uint64_t)));
+    CU(ctx, d.sel_ctr.reserve(sizeof(unsigned long long)));
+    unsigned long long *base = d.sel_ctr.as<unsigned long long>();
+    CU(ctx, cudaMemsetAsync(base, 0, sizeof(unsigned long long), d.stream));
+    const uint32_t *cnt = d.sel_cig_count.as<uint32_t>();
+    uint64_t *off = d.sel_cig_off.as<uint64_t>();
+    if (n_out >= (1u << 16)) {
+        const uint32_t nbk = (uint32_t)((n_out + 1023) / 1024);
+        CU(ctx, d.cig_bsum.reserve((size_t)nbk * sizeof(unsigned long long)));
+        cigar_block_sum_kernel<<<nbk, 1024, 0, d.stream>>>(cnt, 0, n_out, d.cig_bsum.as<unsigned long long>());
+        CU(ctx, cudaGetLastError());
+        cigar_scan_sums_kernel<<<1, 1024, 0, d.stream>>>(d.cig_bsum.as<unsigned long long>(), nbk, base, off + n_out);
+        CU(ctx, cudaGetLastError());
+        cigar_block_scan_kernel<<<nbk, 1024, 0, d.stream>>>(cnt, 0, n_out, d.cig_bsum.as<unsigned long long>(), off);
+        CU(ctx, cudaGetLastError());
+        ctx->last_launches += 3;
+    } else {
+        cigar_scan_kernel<<<1, 1024, 0, d.stream>>>(cnt, 0, n_out, off, base);
+        CU(ctx, cudaGetLastError());
+        ctx->last_launches++;
+    }
+    unsigned long long need = 0;
+    CU(ctx, cudaMemcpyAsync(&need, base, sizeof(need), cudaMemcpyDeviceToHost, d.stream));
+    CU(ctx, cudaStreamSynchronize(d.stream));
+    *cig_need = need;
+    return 0;
+}
+
+// Copies the selected strands' CIGAR words (select_strands ran) into a compact stream and swaps it and its offsets into
+// the buffers fetch_alignments reads.  Needs every word of the doubled run in d.cig_out.
+int gather_strand_cigars(zoe_cuda_ctx *ctx, Device &d, uint64_t total) {
+    const uint64_t n_out = d.n_count / 2 * ctx->n_prof;
+    d.cig_total = total;
+    if (n_out == 0) return 0;
+    CU(ctx, cudaSetDevice(d.id));
+    CU(ctx, d.sel_cig_out.reserve(std::max<uint64_t>(total, 1) * sizeof(uint32_t)));
+    if (total) {
+        const uint32_t blocks = (uint32_t)std::min<uint64_t>((n_out + 7) / 8, (uint64_t)d.sm_count * 16);
+        strand_cigar_gather_kernel<<<blocks, 256, 0, d.stream>>>(d.cig_out.as<uint32_t>(), d.cig_off.as<uint64_t>(),
+                                                                 d.strand.as<uint8_t>(), n_out, ctx->n_prof,
+                                                                 d.sel_cig_off.as<uint64_t>(), d.sel_cig_out.as<uint32_t>());
+        CU(ctx, cudaGetLastError());
+        ctx->last_launches++;
+    }
+    std::swap(d.cig_off, d.sel_cig_off);
+    std::swap(d.cig_out, d.sel_cig_out);
+    return 0;
+}
+
+// Copies every device's strand choices into the caller's array (real view).
+int queue_strand_d2h(zoe_cuda_ctx *ctx, uint8_t *strand) {
+    if (!strand) return 0;
+    for (Device &d : ctx->devs) {
+        if (d.n_count == 0) continue;
+        CU(ctx, cudaSetDevice(d.id));
+        CU(ctx, cudaMemcpyAsync(strand + (size_t)d.n_first * ctx->n_prof, d.strand.p, (size_t)d.n_count * ctx->n_prof,
+                                cudaMemcpyDeviceToHost, d.stream));
+    }
+    return 0;
+}
+
+// The statistics of a both-strand call count the work done: gather_stats ran on the real view, its counters on the
+// doubled batch.
+int gather_both_strands_stats(zoe_cuda_ctx *ctx) {
+    int rc = gather_stats(ctx);
+    ctx->stats.pairs *= 2;
+    ctx->stats.cells *= 2;
+    return rc;
+}
+
+constexpr int kNotMixed = 1;
+int align_split_long_short(zoe_cuda_ctx *ctx, bool both_strands, const uint8_t *streamed_concat, const uint64_t *offsets,
+                           uint64_t n, uint32_t *score, uint8_t *status, uint8_t *tier, uint32_t *ref_start,
+                           uint32_t *ref_end, uint32_t *query_start, uint32_t *query_end, uint32_t *cigar,
+                           uint64_t *cigar_off, uint64_t cigar_cap, uint8_t *hazard, uint8_t *strand);
+
+// The align and 3-pass both-strand entry points.  The doubled run gets its own device CIGAR capacity (the caller's
+// capacity bounds the selected strands only); a run whose non-selected strands overflowed it is repeated once with the
+// exact need.
+int align_both_strands(zoe_cuda_ctx *ctx, bool three_pass, const uint8_t *streamed_concat, const uint64_t *offsets,
+                       uint64_t n, uint32_t *score, uint8_t *status, uint8_t *tier, uint32_t *ref_start, uint32_t *ref_end,
+                       uint32_t *query_start, uint32_t *query_end, uint32_t *cigar, uint64_t *cigar_off, uint64_t cigar_cap,
+                       uint8_t *hazard, uint8_t *strand) {
+    if (!cigar_off || (!cigar && cigar_cap)) return fail(ctx, ZOE_CUDA_E_BAD_ARG, "null CIGAR outputs");
+    begin_call(ctx);
+    DoubledView view(ctx);
+    int rc = check_both_strands_limits(ctx, n, true);
+    if (rc) return rc;
+    rc = stage_on_devices(ctx, streamed_concat, offsets, n, /*split=*/false);
+    if (rc) return rc;
+    if (!three_pass && n > 0 && ctx->staged_max_len > (uint32_t)kMaxRowsSinglePass &&
+        ctx->staged_min_len <= (uint32_t)kMaxRowsSinglePass) {
+        for (Device &d : ctx->devs) {
+            CU(ctx, cudaSetDevice(d.id));
+            CU(ctx, cudaStreamSynchronize(d.stream));
+        }
+        rc = align_split_long_short(ctx, true, streamed_concat, offsets, n, score, status, tier, ref_start, ref_end,
+                                    query_start, query_end, cigar, cigar_off, cigar_cap, hazard, strand);
+        if (rc != kNotMixed) {
+            view.ok = rc == 0;
+            return rc;
+        }
+    }
+    for (Device &d : ctx->devs) {
+        rc = expand_strands(ctx, d);
+        if (rc) return rc;
+    }
+    view.enter();
+    const StrandOutputs kind = three_pass ? StrandOutputs::ThreePass : StrandOutputs::Align;
+    uint64_t dev_cap = 2 * cigar_cap + 1024;
+    std::vector<uint64_t> need(ctx->devs.size());
+    for (int attempt = 0;; ++attempt) {
+        rc = for_each_device(ctx, [&](Device &d) {
+            return three_pass ? run_3pass_on_device(ctx, d, dev_cap) : run_align_on_device(ctx, d, dev_cap);
+        });
+        if (rc) return rc;
+        uint64_t total = 0, widest = 0;
+        for (size_t k = 0; k < ctx->devs.size(); ++k) {
+            rc = select_strands(ctx, ctx->devs[k], kind, &need[k]);
+            if (rc) return rc;
+            total += need[k];
+            widest = std::max<uint64_t>(widest, ctx->devs[k].cig_total);
+        }
+        if (total > cigar_cap) {
+            cigar_off[0] = total;
+            return fail(ctx, ZOE_CUDA_E_CIGAR_CAP, "CIGAR buffer too small: the selected strands need %llu words, have %llu",
+                        (unsigned long long)total, (unsigned long long)cigar_cap);
+        }
+        if (widest <= dev_cap) break;
+        if (attempt > 0) return fail(ctx, ZOE_CUDA_E_STATE, "internal error: both-strand CIGAR capacity not met on the re-run");
+        dev_cap = widest;
+    }
+    for (size_t k = 0; k < ctx->devs.size(); ++k) {
+        rc = gather_strand_cigars(ctx, ctx->devs[k], need[k]);
+        if (rc) return rc;
+    }
+    view.leave();
+    rc = queue_strand_d2h(ctx, strand);
+    if (rc) return rc;
+    rc = fetch_alignments(ctx, score, status, tier, ref_start, ref_end, query_start, query_end, cigar, cigar_off, cigar_cap,
+                          three_pass ? nullptr : hazard);
+    if (rc) return rc;
+    if (n == 0) cigar_off[0] = 0;
+    rc = sync_and_time(ctx);
+    if (rc) return rc;
+    view.ok = true;
+    return gather_both_strands_stats(ctx);
+}
+
+// A batch that mixes long (> 1024 residues) and short sequences is aligned in two parts: the short ones take the fast
+// pipelines, the long ones the long-row path (run_align_on_device, long_mode); results are merged in the caller's order.
+// Each part re-enters the entry point the caller used (single- or both-strand).  Returns kNotMixed, having done nothing,
+// when the batch has only one kind.
+int align_split_long_short(zoe_cuda_ctx *ctx, bool both_strands, const uint8_t *streamed_concat, const uint64_t *offsets,
+                           uint64_t n, uint32_t *score, uint8_t *status, uint8_t *tier, uint32_t *ref_start,
+                           uint32_t *ref_end, uint32_t *query_start, uint32_t *query_end, uint32_t *cigar,
+                           uint64_t *cigar_off, uint64_t cigar_cap, uint8_t *hazard, uint8_t *strand) {
+    std::vector<uint64_t> idx[2];  // [0] short, [1] long
+    for (uint64_t i = 0; i < n; ++i) idx[offsets[i + 1] - offsets[i] > (uint64_t)kMaxRowsSinglePass ? 1 : 0].push_back(i);
+    if (idx[0].empty() || idx[1].empty()) return kNotMixed;
+    const uint32_t np = ctx->n_prof;
+    struct Part {
+        std::vector<uint8_t> buf;
+        std::vector<uint64_t> off;
+        std::vector<uint32_t> score, rs, re, qs, qe, cig;
+        std::vector<uint8_t> status, tier, hz, sd;
+        std::vector<uint64_t> coff;
+    } part[2];
+    zoe_cuda_stats total{};
+    float total_ms = 0.f, dp_ms = 0.f;
+    uint32_t launches = 0;
+    uint64_t need = 0;
+    int rc_cap = 0;
+    for (int w = 0; w < 2; ++w) {
+        Part &q = part[w];
+        q.off.push_back(0);
+        for (uint64_t i : idx[w]) {
+            q.buf.insert(q.buf.end(), streamed_concat + offsets[i], streamed_concat + offsets[i + 1]);
+            q.off.push_back(q.buf.size());
+        }
+        if (q.buf.empty()) q.buf.push_back(0);
+        const size_t pairs = idx[w].size() * np;
+        for (auto *v : {&q.score, &q.rs, &q.re, &q.qs, &q.qe}) v->assign(pairs, 0);
+        for (auto *v : {&q.status, &q.tier, &q.hz, &q.sd}) v->assign(pairs, 0);
+        q.coff.assign(pairs + 1, 0);
+        q.cig.assign(std::max<uint64_t>(cigar_cap, 1), 0);
+        int rc = both_strands
+                     ? zoe_cuda_sw_align_both_strands_batch(ctx, q.buf.data(), q.off.data(), idx[w].size(), q.score.data(),
+                                                            q.status.data(), q.tier.data(), q.rs.data(), q.re.data(),
+                                                            q.qs.data(), q.qe.data(), q.cig.data(), q.coff.data(), cigar_cap,
+                                                            q.hz.data(), q.sd.data())
+                     : zoe_cuda_sw_align_batch(ctx, q.buf.data(), q.off.data(), idx[w].size(), q.score.data(), q.status.data(),
+                                               q.tier.data(), q.rs.data(), q.re.data(), q.qs.data(), q.qe.data(), q.cig.data(),
+                                               q.coff.data(), cigar_cap, q.hz.data());
+        if (rc == ZOE_CUDA_E_CIGAR_CAP) {
+            rc_cap = rc;
+            need += q.coff[0];
+            continue;
+        }
+        if (rc) return rc;
+        need += q.coff[pairs];
+        const zoe_cuda_stats &st = ctx->stats;
+        total.pairs += st.pairs; total.cells += st.cells; total.tier8 += st.tier8; total.tier16 += st.tier16;
+        total.tier32 += st.tier32; total.overflowed += st.overflowed; total.unmapped += st.unmapped;
+        total.rerun_wide += st.rerun_wide; total.hazard += st.hazard; total.window_fallback += st.window_fallback;
+        total.window_pinned += st.window_pinned;
+        total_ms += ctx->last_total_ms;
+        dp_ms += ctx->last_dp_ms;
+        launches += ctx->last_launches.load();
+    }
+    if (rc_cap || need > cigar_cap) {
+        cigar_off[0] = need;
+        return fail(ctx, ZOE_CUDA_E_CIGAR_CAP, "CIGAR buffer too small: need at least %llu words, have %llu",
+                    (unsigned long long)need, (unsigned long long)cigar_cap);
+    }
+    uint64_t pos = 0;
+    size_t cursor[2] = {0, 0};
+    for (uint64_t i = 0; i < n; ++i) {
+        const int w = offsets[i + 1] - offsets[i] > (uint64_t)kMaxRowsSinglePass ? 1 : 0;
+        const Part &q = part[w];
+        const size_t src = cursor[w]++ * np, dst = (size_t)i * np;
+        for (uint32_t j = 0; j < np; ++j) {
+            if (score) score[dst + j] = q.score[src + j];
+            if (status) status[dst + j] = q.status[src + j];
+            if (tier) tier[dst + j] = q.tier[src + j];
+            if (ref_start) ref_start[dst + j] = q.rs[src + j];
+            if (ref_end) ref_end[dst + j] = q.re[src + j];
+            if (query_start) query_start[dst + j] = q.qs[src + j];
+            if (query_end) query_end[dst + j] = q.qe[src + j];
+            if (hazard) hazard[dst + j] = q.hz[src + j];
+            if (strand) strand[dst + j] = q.sd[src + j];
+            cigar_off[dst + j] = pos;
+            const uint64_t a = q.coff[src + j], b = q.coff[src + j + 1];
+            if (b > a) memcpy(cigar + pos, q.cig.data() + a, (b - a) * sizeof(uint32_t));
+            pos += b - a;
+        }
+    }
+    cigar_off[(size_t)n * np] = pos;
+    ctx->stats = total;
+    ctx->last_total_ms = total_ms;
+    ctx->last_dp_ms = dp_ms;
+    ctx->last_launches = launches;
+    ctx->staged = false;
+    return 0;
+}
+
 }  // namespace
 
 // =================================================================================================
@@ -2738,6 +3171,10 @@ void zoe_cuda_destroy(zoe_cuda_ctx *ctx) {
                           &d.tp_blob, &d.tp_ctr, &d.tp_cigoff, &d.tp_bw, &d.tp_list, &d.tp_cig, &d.sn_refs, &d.sn_roff, &d.sn_qry, &d.sn_qoff, &d.sn_out, &d.long_ids, &d.long_bnd,
                           &d.long_queue, &d.ckpt, &d.ckpt_base, &d.win_hist, &d.win_bucket, &d.win_items, &d.win_nitems, &d.win_pitems, &d.win_pnitems, &d.win_amb, &d.starts, &d.cig_bsum})
             b->release();
+        for (DevBuf *b : {&d.xs_seq, &d.xs_off, &d.strand, &d.sel_cig_count, &d.sel_cig_off, &d.sel_cig_out, &d.sel_ctr})
+            b->release();
+        for (DevBuf &b : d.sel32) b.release();
+        for (DevBuf &b : d.sel8) b.release();
         if (d.ev_begin) cudaEventDestroy(d.ev_begin);
         if (d.ev_end) cudaEventDestroy(d.ev_end);
         if (d.ev_k0) cudaEventDestroy(d.ev_k0);
@@ -2978,16 +3415,7 @@ int zoe_cuda_sw_score_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_concat, c
     begin_call(ctx);
     int rc = prepare_batch(ctx, streamed_concat, offsets, n);
     if (rc) return rc;
-    auto d2h = [&](Device &d) -> int {  // queued behind the kernels on the device's stream
-        if (d.n_count == 0) return 0;
-        CU(ctx, cudaSetDevice(d.id));
-        size_t first = (size_t)d.n_first * ctx->n_prof, pairs = (size_t)d.n_count * ctx->n_prof;
-        if (score)
-            CU(ctx, cudaMemcpyAsync(score + first, d.score.p, pairs * sizeof(uint32_t), cudaMemcpyDeviceToHost, d.stream));
-        if (status) CU(ctx, cudaMemcpyAsync(status + first, d.status.p, pairs, cudaMemcpyDeviceToHost, d.stream));
-        if (tier) CU(ctx, cudaMemcpyAsync(tier + first, d.tier.p, pairs, cudaMemcpyDeviceToHost, d.stream));
-        return 0;
-    };
+    auto d2h = [&](Device &d) { return queue_score_d2h(ctx, d, score, status, tier); };
     // Large batches are cut into sub-batches that alternate between the two streams of a GPU, so the H2D copy of the
     // next sub-batch and the D2H copy of the previous one overlap the kernels of the current one.  Not for the long-row
     // path (its copies are negligible next to its kernels) nor when packed lanes may overflow (the 32-bit re-run
@@ -3065,8 +3493,7 @@ int zoe_cuda_sw_align_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_concat, c
     int rc = stage_on_devices(ctx, streamed_concat, offsets, n, /*split=*/true);
     if (rc) return rc;
     dbg.lap("align: stage");
-    // A batch that mixes long (> 1024 residues) and short sequences is split: the short ones take the fast pipelines,
-    // the long ones the long-row path (run_align_on_device, long_mode); results are merged in the caller's order.
+    // A batch that mixes long (> 1024 residues) and short sequences is split (align_split_long_short).
     // Detected from the lengths the staging pass collects anyway (a separate pass that lists the indices of 1M reads
     // cost 3-4 ms of host time in front of every call); the upload already queued for the whole batch is drained and dropped.
     if (n > 0 && ctx->staged_max_len > (uint32_t)kMaxRowsSinglePass && ctx->staged_min_len <= (uint32_t)kMaxRowsSinglePass) {
@@ -3077,88 +3504,9 @@ int zoe_cuda_sw_align_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_concat, c
             d.copy_pending = false;
         }
         ctx->staged = false;
-        std::vector<uint64_t> idx[2];  // [0] short, [1] long
-        for (uint64_t i = 0; i < n; ++i) idx[offsets[i + 1] - offsets[i] > (uint64_t)kMaxRowsSinglePass ? 1 : 0].push_back(i);
-        if (!idx[0].empty() && !idx[1].empty()) {
-            const uint32_t np = ctx->n_prof;
-            struct Part {
-                std::vector<uint8_t> buf;
-                std::vector<uint64_t> off;
-                std::vector<uint32_t> score, rs, re, qs, qe, cig;
-                std::vector<uint8_t> status, tier, hz;
-                std::vector<uint64_t> coff;
-            } part[2];
-            zoe_cuda_stats total{};
-            float total_ms = 0.f, dp_ms = 0.f;
-            uint32_t launches = 0;
-            uint64_t need = 0;
-            int rc_cap = 0;
-            for (int w = 0; w < 2; ++w) {
-                Part &q = part[w];
-                q.off.push_back(0);
-                for (uint64_t i : idx[w]) {
-                    q.buf.insert(q.buf.end(), streamed_concat + offsets[i], streamed_concat + offsets[i + 1]);
-                    q.off.push_back(q.buf.size());
-                }
-                if (q.buf.empty()) q.buf.push_back(0);
-                const size_t pairs = idx[w].size() * np;
-                for (auto *v : {&q.score, &q.rs, &q.re, &q.qs, &q.qe}) v->assign(pairs, 0);
-                for (auto *v : {&q.status, &q.tier, &q.hz}) v->assign(pairs, 0);
-                q.coff.assign(pairs + 1, 0);
-                q.cig.assign(std::max<uint64_t>(cigar_cap, 1), 0);
-                int rc = zoe_cuda_sw_align_batch(ctx, q.buf.data(), q.off.data(), idx[w].size(), q.score.data(), q.status.data(),
-                                                 q.tier.data(), q.rs.data(), q.re.data(), q.qs.data(), q.qe.data(), q.cig.data(),
-                                                 q.coff.data(), cigar_cap, q.hz.data());
-                if (rc == ZOE_CUDA_E_CIGAR_CAP) {
-                    rc_cap = rc;
-                    need += q.coff[0];
-                    continue;
-                }
-                if (rc) return rc;
-                need += q.coff[pairs];
-                const zoe_cuda_stats &st = ctx->stats;
-                total.pairs += st.pairs; total.cells += st.cells; total.tier8 += st.tier8; total.tier16 += st.tier16;
-                total.tier32 += st.tier32; total.overflowed += st.overflowed; total.unmapped += st.unmapped;
-                total.rerun_wide += st.rerun_wide; total.hazard += st.hazard; total.window_fallback += st.window_fallback;
-                total.window_pinned += st.window_pinned;
-                total_ms += ctx->last_total_ms;
-                dp_ms += ctx->last_dp_ms;
-                launches += ctx->last_launches.load();
-            }
-            if (rc_cap || need > cigar_cap) {
-                cigar_off[0] = need;
-                return fail(ctx, ZOE_CUDA_E_CIGAR_CAP, "CIGAR buffer too small: need at least %llu words, have %llu",
-                            (unsigned long long)need, (unsigned long long)cigar_cap);
-            }
-            uint64_t pos = 0;
-            size_t cursor[2] = {0, 0};
-            for (uint64_t i = 0; i < n; ++i) {
-                const int w = offsets[i + 1] - offsets[i] > (uint64_t)kMaxRowsSinglePass ? 1 : 0;
-                const Part &q = part[w];
-                const size_t src = cursor[w]++ * np, dst = (size_t)i * np;
-                for (uint32_t j = 0; j < np; ++j) {
-                    if (score) score[dst + j] = q.score[src + j];
-                    if (status) status[dst + j] = q.status[src + j];
-                    if (tier) tier[dst + j] = q.tier[src + j];
-                    if (ref_start) ref_start[dst + j] = q.rs[src + j];
-                    if (ref_end) ref_end[dst + j] = q.re[src + j];
-                    if (query_start) query_start[dst + j] = q.qs[src + j];
-                    if (query_end) query_end[dst + j] = q.qe[src + j];
-                    if (hazard) hazard[dst + j] = q.hz[src + j];
-                    cigar_off[dst + j] = pos;
-                    const uint64_t a = q.coff[src + j], b = q.coff[src + j + 1];
-                    if (b > a) memcpy(cigar + pos, q.cig.data() + a, (b - a) * sizeof(uint32_t));
-                    pos += b - a;
-                }
-            }
-            cigar_off[(size_t)n * np] = pos;
-            ctx->stats = total;
-            ctx->last_total_ms = total_ms;
-            ctx->last_dp_ms = dp_ms;
-            ctx->last_launches = launches;
-            ctx->staged = false;
-            return 0;
-        }
+        rc = align_split_long_short(ctx, false, streamed_concat, offsets, n, score, status, tier, ref_start, ref_end,
+                                    query_start, query_end, cigar, cigar_off, cigar_cap, hazard, nullptr);
+        if (rc != kNotMixed) return rc;
     }
     rc = for_each_device(ctx, [&](Device &d) { return run_align_on_device(ctx, d, cigar_cap); });
     if (rc) return rc;
@@ -3182,22 +3530,8 @@ int zoe_cuda_sw_score_ranges_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_co
     if (rc) return rc;
     rc = for_each_device(ctx, [&](Device &d) { return run_ranges_on_device(ctx, d); });
     if (rc) return rc;
-    for (Device &d : ctx->devs) {
-        if (d.n_count == 0) continue;
-        CU(ctx, cudaSetDevice(d.id));
-        size_t first = (size_t)d.n_first * ctx->n_prof, pairs = (size_t)d.n_count * ctx->n_prof;
-        auto d2h = [&](void *dst, const DevBuf &src, size_t elem) -> cudaError_t {
-            if (!dst) return cudaSuccess;
-            return cudaMemcpyAsync((uint8_t *)dst + first * elem, src.p, pairs * elem, cudaMemcpyDeviceToHost, d.stream);
-        };
-        CU(ctx, d2h(score, d.score, 4));
-        CU(ctx, d2h(status, d.status, 1));
-        CU(ctx, d2h(tier, d.tier, 1));
-        CU(ctx, d2h(ref_start, d.ref_start, 4));
-        CU(ctx, d2h(ref_end, d.ref_end, 4));
-        CU(ctx, d2h(query_start, d.query_start, 4));
-        CU(ctx, d2h(query_end, d.query_end, 4));
-    }
+    rc = queue_ranges_d2h(ctx, score, status, tier, ref_start, ref_end, query_start, query_end);
+    if (rc) return rc;
     rc = sync_and_time(ctx);
     if (rc) return rc;
     return gather_stats(ctx);
@@ -3251,6 +3585,79 @@ int zoe_cuda_run_3pass_staged(zoe_cuda_ctx *ctx) {
     rc = sync_and_time(ctx);
     if (rc) return rc;
     return gather_stats(ctx);
+}
+
+int zoe_cuda_sw_score_both_strands_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_concat, const uint64_t *offsets,
+                                         uint64_t n, uint32_t *score, uint8_t *status, uint8_t *tier, uint8_t *strand) {
+    if (!ctx) return ZOE_CUDA_E_BAD_ARG;
+    begin_call(ctx);
+    DoubledView view(ctx);
+    int rc = stage_both_strands(ctx, view, streamed_concat, offsets, n, /*pair_limit=*/false);
+    if (rc) return rc;
+    uint64_t no_cigar = 0;
+    for (Device &d : ctx->devs) {
+        rc = run_score_on_device(ctx, d);
+        if (rc) return rc;
+        rc = select_strands(ctx, d, StrandOutputs::Score, &no_cigar);
+        if (rc) return rc;
+    }
+    view.leave();
+    for (Device &d : ctx->devs) {
+        rc = queue_score_d2h(ctx, d, score, status, tier);
+        if (rc) return rc;
+    }
+    rc = queue_strand_d2h(ctx, strand);
+    if (rc) return rc;
+    rc = sync_and_time(ctx);
+    if (rc) return rc;
+    view.ok = true;
+    return gather_both_strands_stats(ctx);
+}
+
+int zoe_cuda_sw_score_ranges_both_strands_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_concat, const uint64_t *offsets,
+                                                uint64_t n, uint32_t *score, uint8_t *status, uint8_t *tier,
+                                                uint32_t *ref_start, uint32_t *ref_end, uint32_t *query_start,
+                                                uint32_t *query_end, uint8_t *strand) {
+    if (!ctx) return ZOE_CUDA_E_BAD_ARG;
+    begin_call(ctx);
+    DoubledView view(ctx);
+    int rc = stage_both_strands(ctx, view, streamed_concat, offsets, n, /*pair_limit=*/true);
+    if (rc) return rc;
+    rc = for_each_device(ctx, [&](Device &d) { return run_ranges_on_device(ctx, d); });
+    if (rc) return rc;
+    uint64_t no_cigar = 0;
+    for (Device &d : ctx->devs) {
+        rc = select_strands(ctx, d, StrandOutputs::Ranges, &no_cigar);
+        if (rc) return rc;
+    }
+    view.leave();
+    rc = queue_ranges_d2h(ctx, score, status, tier, ref_start, ref_end, query_start, query_end);
+    if (rc) return rc;
+    rc = queue_strand_d2h(ctx, strand);
+    if (rc) return rc;
+    rc = sync_and_time(ctx);
+    if (rc) return rc;
+    view.ok = true;
+    return gather_both_strands_stats(ctx);
+}
+
+int zoe_cuda_sw_align_both_strands_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_concat, const uint64_t *offsets,
+                                         uint64_t n, uint32_t *score, uint8_t *status, uint8_t *tier, uint32_t *ref_start,
+                                         uint32_t *ref_end, uint32_t *query_start, uint32_t *query_end, uint32_t *cigar,
+                                         uint64_t *cigar_off, uint64_t cigar_cap, uint8_t *hazard, uint8_t *strand) {
+    if (!ctx) return ZOE_CUDA_E_BAD_ARG;
+    return align_both_strands(ctx, false, streamed_concat, offsets, n, score, status, tier, ref_start, ref_end, query_start,
+                              query_end, cigar, cigar_off, cigar_cap, hazard, strand);
+}
+
+int zoe_cuda_sw_align_3pass_both_strands_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_concat, const uint64_t *offsets,
+                                               uint64_t n, uint32_t *score, uint8_t *status, uint8_t *tier,
+                                               uint32_t *ref_start, uint32_t *ref_end, uint32_t *query_start,
+                                               uint32_t *query_end, uint32_t *cigar, uint64_t *cigar_off, uint64_t cigar_cap,
+                                               uint8_t *strand) {
+    if (!ctx) return ZOE_CUDA_E_BAD_ARG;
+    return align_both_strands(ctx, true, streamed_concat, offsets, n, score, status, tier, ref_start, ref_end, query_start,
+                              query_end, cigar, cigar_off, cigar_cap, nullptr, strand);
 }
 
 int zoe_cuda_sneaky_snake_batch(zoe_cuda_ctx *ctx, const uint8_t *refs, const uint64_t *ref_offsets, const uint8_t *queries,

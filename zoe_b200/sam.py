@@ -5,6 +5,10 @@ Mirrors (paths relative to the zoe repository):
     ``AlignmentStates::to_cigar_unchecked``, RNEXT ``*``, PNEXT 0, TLEN 0, ``AS:i:<score>``)
   * ``SamData::unmapped``        src/data/records/sam/mod.rs:201-214  (FLAG 4, POS 0, MAPQ 255, CIGAR/SEQ/QUAL ``*``)
   * ``Display for SamData``      src/data/records/sam/std_traits.rs:3-43 (tab-separated, missing SEQ/QUAL as ``*``)
+
+Results of the both-strand search pass their strands as ``strand``: a reverse-strand pair is written as SAM writes a read
+that maps to the reverse strand -- FLAG bit 16 set, SEQ reverse-complemented, QUAL reversed (its POS and CIGAR already
+refer to the reverse complement).
 """
 from __future__ import annotations
 
@@ -14,7 +18,7 @@ from typing import Iterable, List, Optional, Sequence
 import numpy as np
 
 from . import _lib
-from .alignment import Alignment, MaybeAligned
+from .alignment import Alignment, MaybeAligned, Strand, reverse_complement
 
 _OPS = {0: "M", 1: "I", 2: "D", 4: "S"}
 
@@ -54,16 +58,26 @@ class SamData:
         return s
 
 
+def _oriented(reverse: bool, flag: int, seq: bytes, qual: bytes):
+    """FLAG, SEQ and QUAL of a record on the forward strand, or on the reverse strand (FLAG 16)."""
+    if not reverse:
+        return flag, seq, qual
+    return flag | 16, reverse_complement(seq), qual if qual == b"*" else qual[::-1]
+
+
 def sam_records(result: Sequence[Sequence[MaybeAligned]], qnames: Sequence[str], rnames: Sequence[str],
-                seqs: Sequence[bytes], quals: Optional[Sequence[bytes]] = None, mapq: int = 255, flag: int = 0):
+                seqs: Sequence[bytes], quals: Optional[Sequence[bytes]] = None, mapq: int = 255, flag: int = 0,
+                strand: Optional[Sequence[Sequence[Strand]]] = None):
     """``CudaProfiles.sw_align_batch(SeqSrc.Query(reads))`` -> one :class:`SamData` per (read, reference) pair;
-    pairs that are not ``Some`` become ``SamData::unmapped`` records."""
+    pairs that are not ``Some`` become ``SamData::unmapped`` records.  ``strand[i][j]`` (the both-strand search):
+    ``Strand.Reverse`` pairs become reverse-strand records."""
     out = []
     for i, row in enumerate(result):
         for j, m in enumerate(row):
             if m.is_some():
-                out.append(SamData.from_alignment(m.unwrap(), qnames[i], flag, rnames[j], mapq, bytes(seqs[i]),
-                                                  bytes(quals[i]) if quals is not None else b"*"))
+                f, seq, qual = _oriented(strand is not None and strand[i][j] is Strand.Reverse, flag, bytes(seqs[i]),
+                                         bytes(quals[i]) if quals is not None else b"*")
+                out.append(SamData.from_alignment(m.unwrap(), qnames[i], f, rnames[j], mapq, seq, qual))
             else:
                 out.append(SamData.unmapped(qnames[i], rnames[j]))
     return out
@@ -71,9 +85,10 @@ def sam_records(result: Sequence[Sequence[MaybeAligned]], qnames: Sequence[str],
 
 def sam_lines_from_arrays(a: dict, n_profiled: int, qnames: Sequence[str], rnames: Sequence[str], buf: np.ndarray,
                           offs: np.ndarray, quals: Optional[Sequence[bytes]] = None, mapq: int = 255,
-                          flag: int = 0) -> Iterable[str]:
+                          flag: int = 0, strand: Optional[np.ndarray] = None) -> Iterable[str]:
     """The same records straight from ``CudaProfiles.align_arrays`` (no per-pair Python objects): yields SAM lines in
-    pair order (read-major)."""
+    pair order (read-major).  ``strand`` (flat, pair index; e.g. ``align_both_strands_arrays(...)["strand"]``): pairs
+    with strand 1 become reverse-strand records."""
     n = len(offs) - 1
     cig, coff = a["cigar"], a["cigar_off"]
     for i in range(n):
@@ -86,6 +101,7 @@ def sam_lines_from_arrays(a: dict, n_profiled: int, qnames: Sequence[str], rname
                 continue
             words = cig[int(coff[k]):int(coff[k + 1])]
             cigar = "".join(f"{int(w) >> 4}{_OPS[int(w) & 15]}" for w in words)
-            rec = SamData(qnames[i], flag, rnames[j], int(a["ref_start"][k]) + 1, mapq, cigar, seq, qual,
+            f, s, q = _oriented(strand is not None and int(strand[k]) == 1, flag, seq, qual)
+            rec = SamData(qnames[i], f, rnames[j], int(a["ref_start"][k]) + 1, mapq, cigar, s, q,
                           opt_fields=[f"AS:i:{int(a['score'][k])}"])
             yield str(rec)
