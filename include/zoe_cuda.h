@@ -174,6 +174,36 @@ int zoe_cuda_sw_align_3pass_both_strands_batch(zoe_cuda_ctx *ctx, const uint8_t 
                                                uint32_t *query_end, uint32_t *cigar, uint64_t *cigar_off, uint64_t cigar_cap,
                                                uint8_t *strand);
 
+/* Best-hit search: each streamed sequence's best profiled sequence and strand, chosen on the device; the align entry
+ * point aligns only that pair.  For streamed sequence i:
+ *   candidates  (j, s) for every profiled j, with s = 0 (seq_i as given) and, when both_strands is set, also s = 1
+ *               (revcomp(seq_i), the complement table of the both-strand search).  Each candidate's result is what the
+ *               single-strand score call returns for that pair.
+ *   selection   the both-strand rank -- Overflowed > Some(score), ordered by score, > Unmapped -- and the highest rank
+ *               wins; ties go to the smallest j, then to the forward strand.  A sequence whose candidates are all Unmapped
+ *               (a 0-length one too) gets hit 0, strand 0, Unmapped.
+ *   hit, strand, score, status, tier   the winner and its score-call result.
+ *   runner_up   the largest Some score among candidates with j != hit (either strand); 0 when there is none and when
+ *               the winner is not Some.  It is the SAM XS value.
+ * The align entry point returns, for the selected pair (seq_i, or revcomp(seq_i) when strand is 1, against hit),
+ * exactly what zoe_cuda_sw_align_batch returns (three_pass: zoe_cuda_sw_align_3pass_batch, hazard 0): score, status,
+ * tier, ranges, CIGAR, hazard.  Coordinates and CIGAR of a reverse winner refer to revcomp(seq_i).  Winners that are not
+ * Some are not aligned: zero ranges, empty CIGAR.
+ * Every output has n entries (cigar_off n + 1) and may be NULL, except cigar_off, and cigar when cigar_cap > 0.
+ * ZOE_CUDA_E_CIGAR_CAP writes the selected pairs' total need to cigar_off[0].  Limits are those of the score call the
+ * search runs (with both_strands, those of zoe_cuda_sw_score_both_strands_batch).  zoe_cuda_last_stats: pairs and cells
+ * count the score pass over every candidate plus the aligned pairs; the tier / overflowed / unmapped counters count the
+ * score pass; hazard, window and tp_* count the alignments.  A call leaves nothing staged and the profiled set as it was,
+ * error or not (DESIGN.md 4.9). */
+int zoe_cuda_sw_score_best_hit_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_concat, const uint64_t *offsets,
+                                     uint64_t n, int both_strands, uint32_t *hit, uint8_t *strand, uint32_t *score,
+                                     uint8_t *status, uint8_t *tier, uint32_t *runner_up);
+int zoe_cuda_sw_align_best_hit_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_concat, const uint64_t *offsets,
+                                     uint64_t n, int both_strands, int three_pass, uint32_t *hit, uint8_t *strand,
+                                     uint32_t *score, uint8_t *status, uint8_t *tier, uint32_t *runner_up,
+                                     uint32_t *ref_start, uint32_t *ref_end, uint32_t *query_start, uint32_t *query_end,
+                                     uint32_t *cigar, uint64_t *cigar_off, uint64_t cigar_cap, uint8_t *hazard);
+
 /* Batched sneaky_snake(reference, query, threshold) (src/alignment/sneaky_snake.rs:78-131): the SneakySnake
  * pre-alignment filter for pair i = (reference i, query i).  out[i]: 1 = Some(true) (edits within
  * floor(len(query) * threshold)), 0 = Some(false), 2 = None (threshold outside 0..=1, or the length difference exceeds

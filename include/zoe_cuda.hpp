@@ -172,6 +172,57 @@ class CudaProfiles {
         return with_strand(align(seqs, true, &strand), strand);
     }
 
+    // Best-hit search (zoe_cuda.h): per streamed sequence, its best profiled sequence and strand (both_strands), the
+    // alignment of that pair and the runner-up score (SAM XS).
+    struct BestHit {
+        uint32_t index = 0;
+        Strand strand = Strand::Forward;
+        MaybeAligned<Alignment> result;
+        uint32_t runner_up = 0;
+    };
+    std::vector<BestHit> sw_align_best_hit(const std::vector<std::string> &seqs, bool both_strands = false,
+                                           bool three_pass = false) {
+        std::vector<uint8_t> buf;
+        std::vector<uint64_t> off;
+        pack(seqs, buf, off);
+        const size_t n = seqs.size();
+        std::vector<uint32_t> hit(n + 1), score(n + 1), ru(n + 1), rs(n + 1), re(n + 1), qs(n + 1), qe(n + 1);
+        std::vector<uint8_t> strand(n + 1), status(n + 1), tier(n + 1);
+        std::vector<uint64_t> coff(n + 2);
+        std::vector<uint32_t> cig(16 * n + 1024);
+        auto call = [&]() {
+            return zoe_cuda_sw_align_best_hit_batch(ctx_, buf.data(), off.data(), n, both_strands ? 1 : 0, three_pass ? 1 : 0,
+                                                    hit.data(), strand.data(), score.data(), status.data(), tier.data(),
+                                                    ru.data(), rs.data(), re.data(), qs.data(), qe.data(), cig.data(),
+                                                    coff.data(), cig.size(), nullptr);
+        };
+        int rc = call();
+        if (rc == ZOE_CUDA_E_CIGAR_CAP) {
+            cig.resize(coff[0] + 16);
+            rc = call();
+        }
+        check(rc);
+        static const char ops[] = {'M', 'I', 'D', '?', 'S'};
+        std::vector<BestHit> out(n);
+        for (size_t i = 0; i < n; ++i) {
+            BestHit &b = out[i];
+            b.index = hit[i];
+            b.strand = static_cast<Strand>(strand[i]);
+            b.runner_up = ru[i];
+            b.result.status = static_cast<Status>(status[i]);
+            if (!b.result.is_some()) continue;
+            Alignment &a = b.result.value;
+            a.score = score[i];
+            a.ref_range = {rs[i], re[i]};
+            a.query_range = {qs[i], qe[i]};
+            for (uint64_t w = coff[i]; w < coff[i + 1]; ++w) a.states.push_back({cig[w] >> 4, ops[cig[w] & 7]});
+            const bool streamed_is_query = streamed_are_ == SeqSrc::Query;
+            a.ref_len = (uint32_t)(streamed_is_query ? targets_[b.index].size() : seqs[i].size());
+            a.query_len = (uint32_t)(streamed_is_query ? seqs[i].size() : targets_[b.index].size());
+        }
+        return out;
+    }
+
   private:
     template <class T>
     static std::vector<std::pair<T, Strand>> with_strand(std::vector<T> v, const std::vector<uint8_t> &strand) {

@@ -96,6 +96,16 @@ unsafe extern "C" {
         status: *mut u8, tier: *mut u8, ref_start: *mut u32, ref_end: *mut u32, query_start: *mut u32,
         query_end: *mut u32, cigar: *mut u32, cigar_off: *mut u64, cigar_cap: u64, strand: *mut u8,
     ) -> c_int;
+    pub fn zoe_cuda_sw_score_best_hit_batch(
+        ctx: *mut zoe_cuda_ctx, streamed_concat: *const u8, offsets: *const u64, n: u64, both_strands: c_int,
+        hit: *mut u32, strand: *mut u8, score: *mut u32, status: *mut u8, tier: *mut u8, runner_up: *mut u32,
+    ) -> c_int;
+    pub fn zoe_cuda_sw_align_best_hit_batch(
+        ctx: *mut zoe_cuda_ctx, streamed_concat: *const u8, offsets: *const u64, n: u64, both_strands: c_int,
+        three_pass: c_int, hit: *mut u32, strand: *mut u8, score: *mut u32, status: *mut u8, tier: *mut u8,
+        runner_up: *mut u32, ref_start: *mut u32, ref_end: *mut u32, query_start: *mut u32, query_end: *mut u32,
+        cigar: *mut u32, cigar_off: *mut u64, cigar_cap: u64, hazard: *mut u8,
+    ) -> c_int;
     pub fn zoe_cuda_run_ranges_staged(ctx: *mut zoe_cuda_ctx) -> c_int;
     pub fn zoe_cuda_run_3pass_staged(ctx: *mut zoe_cuda_ctx) -> c_int;
     pub fn zoe_cuda_stage_streamed(ctx: *mut zoe_cuda_ctx, streamed_concat: *const u8, offsets: *const u64, n: u64) -> c_int;

@@ -25,6 +25,17 @@ pub enum Strand {
     Reverse = 1,
 }
 
+/// One sequence's result of the best-hit search: the chosen profiled sequence `index` and `strand`, that pair's
+/// alignment (of the reverse complement for `Strand::Reverse`), and the best `Some` score against any other profiled
+/// sequence (0 if none; SAM `XS`).
+#[derive(Debug)]
+pub struct BestHit {
+    pub index:     usize,
+    pub strand:    Strand,
+    pub result:    MaybeAligned<Alignment<u32>>,
+    pub runner_up: u32,
+}
+
 #[derive(Debug)]
 pub enum CudaError {
     Profile(ProfileError),
@@ -135,6 +146,58 @@ impl CudaProfiles {
         let mut sd = vec![0u8; seqs.len() * self.profiled_lens.len()];
         let out = self.align(seqs, true, Some(&mut sd))?;
         Ok(out.into_iter().zip(sd).map(|(m, d)| (m, strand(d))).collect())
+    }
+
+    /// Best-hit search: one `BestHit` per sequence -- its best profiled sequence (and strand, with `both_strands`) by the
+    /// both-strand rank, ties to the smallest index and then `Strand::Forward`; the alignment of that pair as
+    /// `sw_align_batch` (`three_pass`: `sw_align_3pass_batch`) aligns it; the runner-up score (SAM XS).
+    pub fn sw_align_best_hit_batch(&self, seqs: &[&[u8]], both_strands: bool, three_pass: bool) -> Result<Vec<BestHit>, CudaError> {
+        let (concat, offsets) = pack(seqs);
+        let n = seqs.len();
+        let (mut hit, mut score, mut ru) = (vec![0u32; n + 1], vec![0u32; n + 1], vec![0u32; n + 1]);
+        let (mut sd, mut status, mut tier) = (vec![0u8; n + 1], vec![0u8; n + 1], vec![0u8; n + 1]);
+        let (mut rs, mut re, mut qs, mut qe) = (vec![0u32; n + 1], vec![0u32; n + 1], vec![0u32; n + 1], vec![0u32; n + 1]);
+        let mut coff = vec![0u64; n + 2];
+        let mut cigar = vec![0u32; 16 * n + 1024];
+        loop {
+            let rc = unsafe {
+                sys::zoe_cuda_sw_align_best_hit_batch(self.ctx, concat.as_ptr(), offsets.as_ptr(), n as u64,
+                    both_strands as std::os::raw::c_int, three_pass as std::os::raw::c_int, hit.as_mut_ptr(), sd.as_mut_ptr(),
+                    score.as_mut_ptr(), status.as_mut_ptr(), tier.as_mut_ptr(), ru.as_mut_ptr(), rs.as_mut_ptr(),
+                    re.as_mut_ptr(), qs.as_mut_ptr(), qe.as_mut_ptr(), cigar.as_mut_ptr(), coff.as_mut_ptr(),
+                    cigar.len() as u64, std::ptr::null_mut())
+            };
+            if rc == sys::ZOE_CUDA_E_CIGAR_CAP {
+                cigar.resize(coff[0] as usize + 16, 0);
+                continue;
+            }
+            self.check(rc, 0, 0)?;
+            break;
+        }
+        const OPS: [u8; 5] = [b'M', b'I', b'D', b'?', b'S'];
+        Ok(seqs.iter().enumerate().map(|(i, seq)| {
+            let j = hit[i] as usize;
+            let result = match status[i] {
+                sys::ZOE_CUDA_SOME => {
+                    let ciglets = cigar[coff[i] as usize..coff[i + 1] as usize]
+                        .iter()
+                        .map(|w| Ciglet { inc: (w >> 4) as usize, op: OPS[(w & 7) as usize] });
+                    let (ref_len, query_len) =
+                        if self.profiled_is_query { (seq.len(), self.profiled_lens[j]) } else { (self.profiled_lens[j], seq.len()) };
+                    MaybeAligned::Some(Alignment {
+                        score: score[i],
+                        ref_range: rs[i] as usize..re[i] as usize,
+                        query_range: qs[i] as usize..qe[i] as usize,
+                        states: AlignmentStates::from_ciglets_unchecked(ciglets),
+                        ref_len,
+                        query_len,
+                    })
+                }
+                sys::ZOE_CUDA_OVERFLOWED => MaybeAligned::Overflowed,
+                _ => MaybeAligned::Unmapped,
+            };
+            BestHit { index: j, strand: strand(sd[i]), result, runner_up: ru[i] }
+        }).collect())
     }
 
     /// `strand`: the both-strand entry points, the strand of every pair written there.

@@ -5,6 +5,7 @@ Host-side mirror of the zoe interface for this path (``alignment``), the data ta
 """
 from .alignment import (  # noqa: F401
     Alignment,
+    BestHit,
     CudaProfiles,
     MaybeAligned,
     ProfileError,

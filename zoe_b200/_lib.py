@@ -22,6 +22,7 @@ SYMBOLS = [
     "zoe_cuda_run_3pass_staged", "zoe_cuda_sneaky_snake_batch", "zoe_cuda_set_memory_budget",
     "zoe_cuda_sw_score_both_strands_batch", "zoe_cuda_sw_score_ranges_both_strands_batch",
     "zoe_cuda_sw_align_both_strands_batch", "zoe_cuda_sw_align_3pass_both_strands_batch",
+    "zoe_cuda_sw_score_best_hit_batch", "zoe_cuda_sw_align_best_hit_batch",
 ]
 
 
@@ -72,6 +73,9 @@ def load() -> C.CDLL:
     lib.zoe_cuda_sw_score_ranges_both_strands_batch.argtypes = lib.zoe_cuda_sw_score_ranges_batch.argtypes + [u8p]
     lib.zoe_cuda_sw_align_both_strands_batch.argtypes = lib.zoe_cuda_sw_align_batch.argtypes + [u8p]
     lib.zoe_cuda_sw_align_3pass_both_strands_batch.argtypes = lib.zoe_cuda_sw_align_3pass_batch.argtypes + [u8p]
+    lib.zoe_cuda_sw_score_best_hit_batch.argtypes = [p, u8p, u64p, C.c_uint64, C.c_int, u32p, u8p, u32p, u8p, u8p, u32p]
+    lib.zoe_cuda_sw_align_best_hit_batch.argtypes = [p, u8p, u64p, C.c_uint64, C.c_int, C.c_int, u32p, u8p, u32p, u8p, u8p,
+                                                     u32p, u32p, u32p, u32p, u32p, u32p, u64p, C.c_uint64, u8p]
     lib.zoe_cuda_sneaky_snake_batch.argtypes = [p, u8p, u64p, u8p, u64p, C.c_uint64, C.c_float, u8p]
     lib.zoe_cuda_stage_streamed.argtypes = [p, u8p, u64p, C.c_uint64]
     lib.zoe_cuda_run_score_staged.argtypes = [p]

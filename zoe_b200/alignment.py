@@ -164,6 +164,18 @@ def _p(a: np.ndarray, ty):
     return a.ctypes.data_as(C.POINTER(ty))
 
 
+@dataclass(frozen=True)
+class BestHit:
+    """One streamed sequence's result of the best-hit search: the chosen profiled sequence ``index`` and ``strand``, the
+    alignment of that pair (of the reverse complement for ``Strand.Reverse``), and ``runner_up``, the best Some score
+    against any other profiled sequence (0 if none; SAM ``XS``)."""
+
+    index: int
+    strand: Strand
+    result: MaybeAligned
+    runner_up: int
+
+
 class CudaProfiles:
     """A set of profiled sequences resident on one or more B200s.
 
@@ -540,3 +552,81 @@ class CudaProfiles:
     def sw_align_3pass_both_strands_batch(self, src: SeqSrc):
         """The 3-pass alignment (:meth:`sw_align_3pass_batch`) of the both-strand search."""
         return self.sw_align_both_strands_batch(src, three_pass=True)
+
+    # ---- best-hit search: each streamed sequence's best profiled sequence and strand, chosen on the device ----
+    def sw_score_best_hit_arrays(self, buf: np.ndarray, offs: np.ndarray, both_strands: bool = False):
+        """Per streamed sequence (flat arrays of ``n``): ``hit`` (u32), ``strand`` (u8), the winner's ``score`` /
+        ``status`` / ``tier`` and ``runner_up`` (u32), as ``zoe_cuda_sw_score_best_hit_batch`` defines them."""
+        n = len(offs) - 1
+        out = self._best_hit_outputs(n)
+        self._check(self._lib.zoe_cuda_sw_score_best_hit_batch(
+            self._h, _p(buf, C.c_uint8), _p(offs, C.c_uint64), n, int(both_strands), _p(out["hit"], C.c_uint32),
+            _p(out["strand"], C.c_uint8), _p(out["score"], C.c_uint32), _p(out["status"], C.c_uint8),
+            _p(out["tier"], C.c_uint8), _p(out["runner_up"], C.c_uint32)))
+        return {k: v[:n] for k, v in out.items()}
+
+    def align_best_hit_arrays(self, buf: np.ndarray, offs: np.ndarray, both_strands: bool = False,
+                              three_pass: bool = False, cigar_cap: Optional[int] = None):
+        """:meth:`sw_score_best_hit_arrays` plus the alignment of each selected pair: ``ref_start`` ... ``query_end``,
+        ``hazard``, ``cigar`` and ``cigar_off`` (``n + 1``), indexed by streamed sequence."""
+        n = len(offs) - 1
+        m = max(n, 1)
+        out = self._best_hit_outputs(n)
+        out.update({k: np.zeros(m, dtype=np.uint32) for k in ("ref_start", "ref_end", "query_start", "query_end")})
+        out["hazard"] = np.zeros(m, dtype=np.uint8)
+        out["cigar_off"] = np.zeros(m + 1, dtype=np.uint64)
+        cap = int(cigar_cap) if cigar_cap else max(16 * m, 1024)
+        for _ in range(2):
+            out["cigar"] = np.zeros(cap, dtype=np.uint32)
+            rc = self._lib.zoe_cuda_sw_align_best_hit_batch(
+                self._h, _p(buf, C.c_uint8), _p(offs, C.c_uint64), n, int(both_strands), int(three_pass),
+                _p(out["hit"], C.c_uint32), _p(out["strand"], C.c_uint8), _p(out["score"], C.c_uint32),
+                _p(out["status"], C.c_uint8), _p(out["tier"], C.c_uint8), _p(out["runner_up"], C.c_uint32),
+                _p(out["ref_start"], C.c_uint32), _p(out["ref_end"], C.c_uint32), _p(out["query_start"], C.c_uint32),
+                _p(out["query_end"], C.c_uint32), _p(out["cigar"], C.c_uint32), _p(out["cigar_off"], C.c_uint64),
+                len(out["cigar"]), _p(out["hazard"], C.c_uint8))
+            if rc == _lib.E_CIGAR_CAP:
+                cap = int(out["cigar_off"][0]) + 16
+                continue
+            self._check(rc)
+            break
+        else:
+            self._check(rc)
+        for k in out:
+            if k not in ("cigar", "cigar_off"):
+                out[k] = out[k][:n]
+        out["cigar_off"] = out["cigar_off"][:n + 1]
+        return out
+
+    @staticmethod
+    def _best_hit_outputs(n: int) -> dict:
+        m = max(n, 1)
+        return {"hit": np.zeros(m, dtype=np.uint32), "strand": np.zeros(m, dtype=np.uint8),
+                "score": np.zeros(m, dtype=np.uint32), "status": np.zeros(m, dtype=np.uint8),
+                "tier": np.zeros(m, dtype=np.uint8), "runner_up": np.zeros(m, dtype=np.uint32)}
+
+    def sw_align_best_hit_batch(self, src: SeqSrc, both_strands: bool = False, three_pass: bool = False):
+        """One :class:`BestHit` per streamed sequence: its best profiled sequence (and strand, with ``both_strands``),
+        aligned as :meth:`sw_align_batch` aligns that pair."""
+        self._check_src(src)
+        seqs = [bytes(s) for s in src.seq]
+        buf, offs = _pack(seqs)
+        return self._best_hit_rows(seqs, self.align_best_hit_arrays(buf, offs, both_strands, three_pass))
+
+    def _best_hit_rows(self, seqs: Sequence[bytes], a: dict):
+        out = []
+        for i, s in enumerate(seqs):
+            j, strand = int(a["hit"][i]), Strand(int(a["strand"][i]))
+            st = int(a["status"][i])
+            if st != _lib.SOME:
+                m = self._maybe(st, None)
+            else:
+                lo, hi = int(a["cigar_off"][i]), int(a["cigar_off"][i + 1])
+                cig = "".join(f"{int(w) >> 4}{_CIGAR_OPS[int(w) & 15]}" for w in a["cigar"][lo:hi])
+                streamed_len, prof_len = len(s), len(self.targets[j])
+                ref_len, query_len = (streamed_len, prof_len) if self.profiled_is_query else (prof_len, streamed_len)
+                m = MaybeAligned.some(Alignment(
+                    int(a["score"][i]), (int(a["ref_start"][i]), int(a["ref_end"][i])),
+                    (int(a["query_start"][i]), int(a["query_end"][i])), cig, ref_len, query_len))
+            out.append(BestHit(j, strand, m, int(a["runner_up"][i])))
+        return out

@@ -34,6 +34,7 @@
 #include "sw_3pass.cuh"
 #include "sneaky_snake.cuh"
 #include "strands.cuh"
+#include "best_hit.cuh"
 
 using namespace zoe_cuda;
 
@@ -117,6 +118,11 @@ struct Device {
     // both-strand search (strands.cuh): the doubled batch is built here and swapped into rseq / roff; the selected
     // strand's per-pair outputs are gathered into the sel_* buffers and swapped into the ones the fetch paths read
     DevBuf xs_seq, xs_off, strand, sel32[5], sel8[3], sel_cig_count, sel_cig_off, sel_cig_out, sel_ctr;
+    // best-hit search (best_hit.cuh): the staged batch moves to bh_seq / bh_off while each bucket's compact batch is
+    // gathered into rseq / roff; bh_out* / bh_hit / bh_strand / bh_runner are the per-read outputs of the shard, bh_acc
+    // collects the buckets' CIGAR words
+    DevBuf bh_seq, bh_off, bh_key, bh_tab, bh_list, bh_llen, bh_loff, bh_hit, bh_strand, bh_runner, bh_out32[5], bh_out8[3];
+    DevBuf bh_cig_count, bh_cig_src, bh_acc, bh_cig_off, bh_cig;
     uint64_t n_first = 0, n_count = 0;  // shard of the streamed batch owned by this device
     uint64_t rseq_bytes = 0;
     bool timed_kernel = false;
@@ -620,6 +626,84 @@ int upload_scoring_and_profiled(zoe_cuda_ctx *ctx) {
         CU(ctx, cudaStreamSynchronize(d.stream));
     }
     return 0;
+}
+
+// The host-side derivation of a profiled set (offsets validated by the caller; max_len its longest sequence): symbol
+// codes, visiting order, dense symbol table, wk and the column groups, then the upload to every device.  Invalidates the
+// launch plans and everything the devices cached about the previous set.
+int install_profiled(zoe_cuda_ctx *ctx, const uint8_t *concat, const uint64_t *offsets, uint32_t n, uint32_t max_len) {
+    const uint64_t total = offsets[n] - offsets[0];
+    ctx->plans.clear();
+    ctx->profiled_epoch++;
+    ctx->n_prof = n;
+    ctx->max_prof_len = max_len;
+    ctx->prof_bytes.assign(concat + offsets[0], concat + offsets[n]);
+    ctx->prof_off.resize(n + 1);
+    ctx->coff.resize(n + 1);
+    for (uint32_t j = 0; j <= n; ++j) {
+        ctx->prof_off[j] = offsets[j] - offsets[0];
+        ctx->coff[j] = (uint32_t)ctx->prof_off[j];
+    }
+    // visiting order for the two-stream score kernel: longest first, so paired sweeps have similar lengths
+    ctx->corder.resize(n);
+    for (uint32_t j = 0; j < n; ++j) ctx->corder[j] = j;
+    std::stable_sort(ctx->corder.begin(), ctx->corder.end(), [&](uint32_t a, uint32_t b) {
+        return ctx->coff[a + 1] - ctx->coff[a] > ctx->coff[b + 1] - ctx->coff[b];
+    });
+    // dense column-symbol codes: only the symbols that occur in the profiled set get a table row
+    int dense[64];
+    for (int i = 0; i < 64; ++i) dense[i] = -1;
+    std::vector<int> sym_of_dense;
+    ctx->ccodes.resize(total);
+    for (uint64_t i = 0; i < total; ++i) {
+        int s = ctx->lut[ctx->prof_bytes[i]];
+        if (dense[s] < 0) {
+            dense[s] = (int)sym_of_dense.size();
+            sym_of_dense.push_back(s);
+        }
+        ctx->ccodes[i] = (uint8_t)dense[s];
+    }
+    ctx->n_csym = (int)sym_of_dense.size();
+    // wk[c][r] = weights[streamed symbol r][profiled symbol c]  (profile.rs:290-291: the profile row is
+    // indexed by the streamed symbol, the lane by the profiled residue)
+    ctx->wk.assign((size_t)ctx->n_csym * ctx->S, 0);
+    for (int c = 0; c < ctx->n_csym; ++c)
+        for (int r = 0; r < ctx->S; ++r) ctx->wk[(size_t)c * ctx->S + r] = ctx->weights[(size_t)r * ctx->S + sym_of_dense[c]];
+    // regroup a panel that does not fit the staging area (see launch_score)
+    ctx->groups.clear();
+    ctx->ccodes_g.clear();
+    ctx->coff_g.clear();
+    ctx->corder_g.clear();
+    if (total > kColsSmemLimit && n > 1) {
+        uint32_t j = 0;
+        while (j < n) {
+            zoe_cuda_ctx::ColGroup g{};
+            g.j0 = j;
+            g.byte_start = (uint32_t)ctx->ccodes_g.size();
+            g.coff_start = (uint32_t)ctx->corder_g.size();
+            uint32_t bytes = 0;
+            while (j < n && (bytes == 0 || bytes + (ctx->coff[j + 1] - ctx->coff[j]) <= kColsSmemLimit)) {
+                ctx->coff_g.push_back(bytes);
+                bytes += ctx->coff[j + 1] - ctx->coff[j];
+                ++j;
+            }
+            ctx->coff_g.push_back(bytes);
+            g.n = j - g.j0;
+            g.bytes = bytes;
+            ctx->ccodes_g.insert(ctx->ccodes_g.end(), ctx->ccodes.begin() + ctx->coff[g.j0], ctx->ccodes.begin() + ctx->coff[j]);
+            ctx->ccodes_g.resize((ctx->ccodes_g.size() + 15) & ~(size_t)15, 0);  // next group starts 16-byte aligned (TMA)
+            std::vector<uint32_t> order(g.n);
+            for (uint32_t q = 0; q < g.n; ++q) order[q] = q;
+            std::stable_sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) {
+                return ctx->coff[g.j0 + a + 1] - ctx->coff[g.j0 + a] > ctx->coff[g.j0 + b + 1] - ctx->coff[g.j0 + b];
+            });
+            ctx->corder_g.insert(ctx->corder_g.end(), order.begin(), order.end());
+            ctx->groups.push_back(g);
+        }
+        ctx->ccodes_g.resize(ctx->ccodes_g.size() + 16, 0);
+        if (ctx->groups.size() < 2) ctx->groups.clear();
+    }
+    return upload_scoring_and_profiled(ctx);
 }
 
 // Split [0, n) over the devices by contiguous index range (SURVEY.md 8(e)); no collective.
@@ -2822,6 +2906,28 @@ int stage_both_strands(zoe_cuda_ctx *ctx, DoubledView &view, const uint8_t *conc
     return 0;
 }
 
+// Queues the exclusive scan of n 32-bit counts into off[0, n] (off[n] = the total, also left in *base, which is zeroed
+// first): the CIGAR offset scan of the align pipeline.
+int scan_counts(zoe_cuda_ctx *ctx, Device &d, const uint32_t *cnt, uint64_t n, uint64_t *off, unsigned long long *base) {
+    CU(ctx, cudaMemsetAsync(base, 0, sizeof(unsigned long long), d.stream));
+    if (n >= (1u << 16)) {
+        const uint32_t nbk = (uint32_t)((n + 1023) / 1024);
+        CU(ctx, d.cig_bsum.reserve((size_t)nbk * sizeof(unsigned long long)));
+        cigar_block_sum_kernel<<<nbk, 1024, 0, d.stream>>>(cnt, 0, n, d.cig_bsum.as<unsigned long long>());
+        CU(ctx, cudaGetLastError());
+        cigar_scan_sums_kernel<<<1, 1024, 0, d.stream>>>(d.cig_bsum.as<unsigned long long>(), nbk, base, off + n);
+        CU(ctx, cudaGetLastError());
+        cigar_block_scan_kernel<<<nbk, 1024, 0, d.stream>>>(cnt, 0, n, d.cig_bsum.as<unsigned long long>(), off);
+        CU(ctx, cudaGetLastError());
+        ctx->last_launches += 3;
+    } else {
+        cigar_scan_kernel<<<1, 1024, 0, d.stream>>>(cnt, 0, n, off, base);
+        CU(ctx, cudaGetLastError());
+        ctx->last_launches++;
+    }
+    return 0;
+}
+
 enum class StrandOutputs { Score, Ranges, Align, ThreePass };
 
 // Strand selection on one device (doubled view): gathers the selected strand's per-pair outputs into the buffers the
@@ -2866,24 +2972,8 @@ int select_strands(zoe_cuda_ctx *ctx, Device &d, StrandOutputs kind, uint64_t *c
     CU(ctx, d.sel_cig_off.reserve((n_out + 1) * sizeof(uint64_t)));
     CU(ctx, d.sel_ctr.reserve(sizeof(unsigned long long)));
     unsigned long long *base = d.sel_ctr.as<unsigned long long>();
-    CU(ctx, cudaMemsetAsync(base, 0, sizeof(unsigned long long), d.stream));
-    const uint32_t *cnt = d.sel_cig_count.as<uint32_t>();
-    uint64_t *off = d.sel_cig_off.as<uint64_t>();
-    if (n_out >= (1u << 16)) {
-        const uint32_t nbk = (uint32_t)((n_out + 1023) / 1024);
-        CU(ctx, d.cig_bsum.reserve((size_t)nbk * sizeof(unsigned long long)));
-        cigar_block_sum_kernel<<<nbk, 1024, 0, d.stream>>>(cnt, 0, n_out, d.cig_bsum.as<unsigned long long>());
-        CU(ctx, cudaGetLastError());
-        cigar_scan_sums_kernel<<<1, 1024, 0, d.stream>>>(d.cig_bsum.as<unsigned long long>(), nbk, base, off + n_out);
-        CU(ctx, cudaGetLastError());
-        cigar_block_scan_kernel<<<nbk, 1024, 0, d.stream>>>(cnt, 0, n_out, d.cig_bsum.as<unsigned long long>(), off);
-        CU(ctx, cudaGetLastError());
-        ctx->last_launches += 3;
-    } else {
-        cigar_scan_kernel<<<1, 1024, 0, d.stream>>>(cnt, 0, n_out, off, base);
-        CU(ctx, cudaGetLastError());
-        ctx->last_launches++;
-    }
+    int rc = scan_counts(ctx, d, d.sel_cig_count.as<uint32_t>(), n_out, d.sel_cig_off.as<uint64_t>(), base);
+    if (rc) return rc;
     unsigned long long need = 0;
     CU(ctx, cudaMemcpyAsync(&need, base, sizeof(need), cudaMemcpyDeviceToHost, d.stream));
     CU(ctx, cudaStreamSynchronize(d.stream));
@@ -3109,6 +3199,403 @@ int align_split_long_short(zoe_cuda_ctx *ctx, bool both_strands, const uint8_t *
     return 0;
 }
 
+// ---------------------------------------------------------------------------------------------
+// best-hit search (best_hit.cuh, DESIGN.md 4.9): the score pass over every candidate -> per-read selection -> for the
+// align entry point, buckets of Some winners by (hit, length class), each aligned by the unchanged pipelines under a
+// profiled view of its one sequence -> per-read outputs and one CIGAR stream in read order
+// ---------------------------------------------------------------------------------------------
+// The host state of a profiled set, set aside while a one-sequence view is installed.
+struct PanelState {
+    uint32_t n_prof = 0, max_prof_len = 0;
+    int n_csym = 0;
+    std::vector<uint8_t> prof_bytes, ccodes, ccodes_g;
+    std::vector<uint64_t> prof_off;
+    std::vector<uint32_t> coff, corder, coff_g, corder_g;
+    std::vector<int8_t> wk;
+    std::vector<zoe_cuda_ctx::ColGroup> groups;
+    void swap_with(zoe_cuda_ctx *ctx) {
+        std::swap(n_prof, ctx->n_prof);
+        std::swap(max_prof_len, ctx->max_prof_len);
+        std::swap(n_csym, ctx->n_csym);
+        prof_bytes.swap(ctx->prof_bytes);
+        ccodes.swap(ctx->ccodes);
+        ccodes_g.swap(ctx->ccodes_g);
+        prof_off.swap(ctx->prof_off);
+        coff.swap(ctx->coff);
+        corder.swap(ctx->corder);
+        coff_g.swap(ctx->coff_g);
+        corder_g.swap(ctx->corder_g);
+        wk.swap(ctx->wk);
+        groups.swap(ctx->groups);
+    }
+};
+
+// Installs the profiled set {j} of the context's panel for one bucket, and restores the panel on leave() or on
+// destruction, error or not.  Both directions derive and upload the set as zoe_cuda_set_profiled does (bump
+// profiled_epoch, clear the plans).  The kernels are not pointed at a slice of the panel's buffers: the codes are
+// staged by TMA from 16-byte-aligned starts, the dense symbol table and wk belong to the whole set, and flag_base /
+// ckpt_base are cached against the epoch.
+struct ProfiledView {
+    zoe_cuda_ctx *ctx;
+    bool active = false;
+    PanelState panel;
+    explicit ProfiledView(zoe_cuda_ctx *c) : ctx(c) {}
+    ProfiledView(const ProfiledView &) = delete;
+    ProfiledView &operator=(const ProfiledView &) = delete;
+    int enter(uint32_t j) {
+        if (!active) {
+            panel.swap_with(ctx);
+            active = true;
+        }
+        const uint64_t off[2] = {panel.prof_off[j], panel.prof_off[j + 1]};
+        return install_profiled(ctx, panel.prof_bytes.data(), off, 1, (uint32_t)(off[1] - off[0]));
+    }
+    int leave() {
+        if (!active) return 0;
+        panel.swap_with(ctx);
+        active = false;
+        ctx->plans.clear();
+        ctx->profiled_epoch++;
+        return upload_scoring_and_profiled(ctx);
+    }
+    ~ProfiledView() { leave(); }
+};
+
+// Per-read selection on one device (real view; the score pass's results are resident in d.score / d.status / d.tier).
+int select_best_hits(zoe_cuda_ctx *ctx, Device &d, uint32_t n_strands) {
+    const uint64_t n = d.n_count;
+    if (n == 0) return 0;
+    CU(ctx, cudaSetDevice(d.id));
+    for (DevBuf *b : {&d.bh_hit, &d.bh_runner, &d.bh_out32[0]}) CU(ctx, b->reserve(n * sizeof(uint32_t)));
+    for (DevBuf *b : {&d.bh_strand, &d.bh_out8[0], &d.bh_out8[1]}) CU(ctx, b->reserve(n));
+    BestHitSelectParams p{};
+    p.score = d.score.as<uint32_t>();
+    p.status = d.status.as<uint8_t>();
+    p.tier = d.tier.as<uint8_t>();
+    p.n = n;
+    p.n_prof = ctx->n_prof;
+    p.n_strands = n_strands;
+    p.hit = d.bh_hit.as<uint32_t>();
+    p.score_out = d.bh_out32[0].as<uint32_t>();
+    p.runner_up = d.bh_runner.as<uint32_t>();
+    p.strand = d.bh_strand.as<uint8_t>();
+    p.status_out = d.bh_out8[0].as<uint8_t>();
+    p.tier_out = d.bh_out8[1].as<uint8_t>();
+    // a thread per read while a read's candidates fit one warp's width, a warp per read beyond
+    if ((uint64_t)ctx->n_prof * n_strands <= 32) {
+        const uint32_t blocks = (uint32_t)std::min<uint64_t>((n + 255) / 256, (uint64_t)d.sm_count * 8);
+        best_hit_select_kernel<1><<<blocks, 256, 0, d.stream>>>(p);
+    } else {
+        const uint32_t blocks = (uint32_t)std::min<uint64_t>((n + 7) / 8, (uint64_t)d.sm_count * 16);
+        best_hit_select_kernel<32><<<blocks, 256, 0, d.stream>>>(p);
+    }
+    CU(ctx, cudaGetLastError());
+    ctx->last_launches++;
+    return 0;
+}
+
+// Buckets one device's Some winners (best_hit_bucket_*_kernel), zeroes the outputs of the reads no bucket aligns, and
+// reads the bucket table back into tab (kBhStart + 1 rows of n_keys words).
+int bucket_best_hits(zoe_cuda_ctx *ctx, Device &d, uint32_t n_strands, bool split_long, uint32_t n_keys,
+                     std::vector<unsigned long long> &tab) {
+    tab.assign((size_t)(kBhStart + 1) * n_keys, 0);
+    const uint64_t n = d.n_count;
+    if (n == 0) return 0;
+    CU(ctx, cudaSetDevice(d.id));
+    CU(ctx, d.bh_key.reserve(n * sizeof(uint32_t)));
+    CU(ctx, d.bh_list.reserve(n * sizeof(uint32_t)));
+    CU(ctx, d.bh_tab.reserve(((size_t)kBhTabRows * n_keys + 1) * sizeof(unsigned long long)));
+    for (DevBuf *b : {&d.bh_out32[1], &d.bh_out32[2], &d.bh_out32[3], &d.bh_out32[4], &d.bh_cig_count}) {
+        CU(ctx, b->reserve(n * sizeof(uint32_t)));
+        CU(ctx, cudaMemsetAsync(b->p, 0, n * sizeof(uint32_t), d.stream));
+    }
+    CU(ctx, d.bh_out8[2].reserve(n));
+    CU(ctx, cudaMemsetAsync(d.bh_out8[2].p, 0, n, d.stream));
+    CU(ctx, d.bh_cig_src.reserve(n * sizeof(uint64_t)));
+    unsigned long long *t = d.bh_tab.as<unsigned long long>();
+    CU(ctx, cudaMemsetAsync(t, 0, ((size_t)kBhTabRows * n_keys + 1) * sizeof(unsigned long long), d.stream));
+    CU(ctx, cudaMemsetAsync(t + (size_t)kBhMin * n_keys, 0xff, (size_t)n_keys * sizeof(unsigned long long), d.stream));
+    const size_t smem = (size_t)4 * n_keys * sizeof(unsigned long long);
+    const bool use_smem = smem <= 48 * 1024;
+    const uint32_t blocks = (uint32_t)std::min<uint64_t>((n + 255) / 256, (uint64_t)d.sm_count * 4);
+    best_hit_bucket_count_kernel<<<blocks, 256, use_smem ? smem : 0, d.stream>>>(
+        d.bh_hit.as<uint32_t>(), d.bh_out8[0].as<uint8_t>(), d.roff.as<uint64_t>(), n_strands, n, split_long, n_keys,
+        use_smem, d.bh_key.as<uint32_t>(), t);
+    CU(ctx, cudaGetLastError());
+    best_hit_bucket_scan_kernel<<<1, 32, 0, d.stream>>>(t, n_keys);
+    CU(ctx, cudaGetLastError());
+    best_hit_bucket_scatter_kernel<<<blocks, 256, 0, d.stream>>>(d.bh_key.as<uint32_t>(), n, n_keys, t,
+                                                                 d.bh_list.as<uint32_t>());
+    CU(ctx, cudaGetLastError());
+    ctx->last_launches += 3;
+    CU(ctx, cudaMemcpyAsync(tab.data(), t, tab.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, d.stream));
+    CU(ctx, cudaStreamSynchronize(d.stream));
+    // compact-batch offsets of every listed read, in list order (bucket b's batch: loff[start_b, start_b + count_b])
+    uint64_t m = 0;
+    for (uint32_t k = 0; k < n_keys; ++k) m += tab[(size_t)kBhCount * n_keys + k];
+    CU(ctx, d.bh_llen.reserve(std::max<uint64_t>(m, 1) * sizeof(uint32_t)));
+    CU(ctx, d.bh_loff.reserve((m + 1) * sizeof(uint64_t)));
+    if (m) {
+        best_hit_list_len_kernel<<<(uint32_t)((m + 255) / 256), 256, 0, d.stream>>>(
+            d.bh_list.as<uint32_t>(), m, d.roff.as<uint64_t>(), n_strands, d.bh_llen.as<uint32_t>());
+        CU(ctx, cudaGetLastError());
+        ctx->last_launches++;
+    }
+    return scan_counts(ctx, d, d.bh_llen.as<uint32_t>(), m, d.bh_loff.as<uint64_t>(), t + (size_t)kBhTabRows * n_keys);
+}
+
+// Grows b to `bytes`, keeping its first `used` bytes.
+int reserve_keep(zoe_cuda_ctx *ctx, Device &d, DevBuf &b, size_t used, size_t bytes) {
+    if (bytes <= b.cap) return 0;
+    DevBuf nb;
+    CU(ctx, nb.reserve(bytes));
+    if (used) CU(ctx, cudaMemcpyAsync(nb.p, b.p, used, cudaMemcpyDeviceToDevice, d.stream));
+    CU(ctx, cudaStreamSynchronize(d.stream));
+    b.release();
+    b = nb;
+    return 0;
+}
+
+// One bucket on one device, under the bucket's host view: gather its reads into rseq / roff, align them against the
+// one profiled sequence, scatter the outputs to read order and move the CIGAR words to bh_acc at *acc_used.
+int align_bucket(zoe_cuda_ctx *ctx, Device &d, bool three_pass, uint32_t n_strands, uint64_t start, uint64_t max_len,
+                 uint64_t cigar_cap, uint64_t *acc_used) {
+    if (d.n_count == 0) return 0;
+    CU(ctx, cudaSetDevice(d.id));
+    const uint64_t cnt = d.n_count;
+    CU(ctx, d.rseq.reserve(d.rseq_bytes + 16));
+    CU(ctx, d.roff.reserve((cnt + 1) * sizeof(uint64_t)));
+    const uint32_t blocks = (uint32_t)std::min<uint64_t>((cnt + 7) / 8, (uint64_t)d.sm_count * 16);
+    best_hit_gather_kernel<<<blocks, 256, 0, d.stream>>>(d.bh_seq.as<uint8_t>(), d.bh_off.as<uint64_t>(), n_strands,
+                                                         d.bh_strand.as<uint8_t>(), d.bh_list.as<uint32_t>() + start,
+                                                         d.bh_loff.as<uint64_t>() + start, cnt, d.rseq.as<uint8_t>(),
+                                                         d.roff.as<uint64_t>());
+    CU(ctx, cudaGetLastError());
+    ctx->last_launches++;
+    // The bucket's CIGARs are part of what the caller receives, so the caller's capacity bounds them; a bucket that
+    // overflows it makes the call fail with ZOE_CUDA_E_CIGAR_CAP and needs no re-run.  (A pair's CIGAR has at most
+    // rows + columns + 4 words: small buckets reserve no more.)
+    const uint64_t cap = std::min<uint64_t>(cigar_cap, cnt * (max_len + ctx->max_prof_len + 4));
+    int rc = three_pass ? run_3pass_on_device(ctx, d, cap) : run_align_on_device(ctx, d, cap);
+    if (rc) return rc;
+    const uint64_t words = d.cig_total;
+    if (words > cap && cap < cigar_cap)
+        return fail(ctx, ZOE_CUDA_E_STATE, "internal error: best-hit bucket CIGAR bound exceeded (%llu words)",
+                    (unsigned long long)words);
+    const bool copy = *acc_used + words <= cigar_cap;
+    if (copy) {
+        rc = reserve_keep(ctx, d, d.bh_acc, *acc_used * sizeof(uint32_t), std::max<uint64_t>(*acc_used + words, 1) * sizeof(uint32_t));
+        if (rc) return rc;
+    }
+    BestHitScatterParams p{};
+    DevBuf *in32[5] = {&d.score, &d.ref_start, &d.ref_end, &d.query_start, &d.query_end};
+    DevBuf *in8[3] = {&d.status, &d.tier, &d.hazard};
+    for (int k = 0; k < 5; ++k) {
+        p.in32[k] = in32[k]->as<uint32_t>();
+        p.out32[k] = d.bh_out32[k].as<uint32_t>();
+    }
+    for (int k = 0; k < 3; ++k) {
+        p.in8[k] = (k == 2 && three_pass) ? nullptr : in8[k]->as<uint8_t>();
+        p.out8[k] = d.bh_out8[k].as<uint8_t>();
+    }
+    p.list = d.bh_list.as<uint32_t>() + start;
+    p.count = cnt;
+    p.cig_off = d.cig_off.as<uint64_t>();
+    p.cig_out = d.cig_out.as<uint32_t>();
+    p.cig_count = d.bh_cig_count.as<uint32_t>();
+    p.cig_src = d.bh_cig_src.as<uint64_t>();
+    p.acc = d.bh_acc.as<uint32_t>();
+    p.acc_base = *acc_used;
+    p.copy = copy && words > 0;
+    best_hit_scatter_kernel<<<blocks, 256, 0, d.stream>>>(p);
+    CU(ctx, cudaGetLastError());
+    ctx->last_launches++;
+    *acc_used += words;
+    return 0;
+}
+
+// The best-hit entry points.  align = false: score pass + selection only.
+int best_hit(zoe_cuda_ctx *ctx, bool align, bool both_strands, bool three_pass, const uint8_t *concat,
+             const uint64_t *offsets, uint64_t n, uint32_t *hit, uint8_t *strand, uint32_t *score, uint8_t *status,
+             uint8_t *tier, uint32_t *runner_up, uint32_t *ref_start, uint32_t *ref_end, uint32_t *query_start,
+             uint32_t *query_end, uint32_t *cigar, uint64_t *cigar_off, uint64_t cigar_cap, uint8_t *hazard) {
+    if (align && (!cigar_off || (!cigar && cigar_cap))) return fail(ctx, ZOE_CUDA_E_BAD_ARG, "null CIGAR outputs");
+    begin_call(ctx);
+    DoubledView view(ctx);  // (entered only with both strands; drains every stream on an error return)
+    int rc = both_strands ? stage_both_strands(ctx, view, concat, offsets, n, /*pair_limit=*/false)
+                          : stage_on_devices(ctx, concat, offsets, n, /*split=*/false);
+    if (rc) return rc;
+    for (Device &d : ctx->devs) {
+        rc = run_score_on_device(ctx, d);
+        if (rc) return rc;
+    }
+    if (align) {
+        // the score pass's counters (every candidate) are read before the align stage reuses them; gather_stats reads
+        // them with a copy that does not wait for the library's streams
+        for (Device &d : ctx->devs) {
+            CU(ctx, cudaSetDevice(d.id));
+            CU(ctx, cudaStreamSynchronize(d.stream));
+        }
+        rc = gather_stats(ctx);
+        if (rc) return rc;
+    }
+    view.leave();
+    const uint32_t S = both_strands ? 2 : 1;
+    for (Device &d : ctx->devs) {
+        rc = select_best_hits(ctx, d, S);
+        if (rc) return rc;
+    }
+    const size_t nd = ctx->devs.size();
+    std::vector<uint64_t> acc_used(nd, 0);
+    if (align) {
+        const bool split_long = !three_pass;
+        const uint32_t P = ctx->n_prof, K = split_long ? 2 * P : P;
+        std::vector<std::vector<unsigned long long>> tab(nd);
+        std::vector<uint64_t> first(nd), count(nd);
+        for (size_t k = 0; k < nd; ++k) {
+            Device &d = ctx->devs[k];
+            rc = bucket_best_hits(ctx, d, S, split_long, K, tab[k]);
+            if (rc) return rc;
+            first[k] = d.n_first;
+            count[k] = d.n_count;
+            std::swap(d.rseq, d.bh_seq);
+            std::swap(d.roff, d.bh_off);
+        }
+        const uint64_t real_n = ctx->staged_n;
+        uint64_t aligned = 0, aligned_cells = 0;
+        {
+            ProfiledView pv(ctx);
+            for (uint32_t key = 0; key < K; ++key) {
+                uint64_t total = 0, residues = 0, longest = 0, shortest = ~0ull;
+                auto at = [&](size_t k, int row) { return (uint64_t)tab[k][(size_t)row * K + key]; };
+                for (size_t k = 0; k < nd; ++k) {
+                    if (at(k, kBhCount) == 0) continue;
+                    total += at(k, kBhCount);
+                    residues += at(k, kBhSum);
+                    longest = std::max<uint64_t>(longest, at(k, kBhMax));
+                    shortest = std::min<uint64_t>(shortest, at(k, kBhMin));
+                }
+                if (total == 0) continue;  // a profiled sequence no read chose
+                rc = pv.enter(split_long ? key / 2 : key);
+                if (rc) return rc;
+                // the host view of the bucket's batch: the devices' buckets back to back
+                ctx->staged_n = total;
+                ctx->staged_max_len = (uint32_t)longest;
+                ctx->staged_min_len = (uint32_t)shortest;
+                ctx->staged_cells = residues * ctx->max_prof_len;
+                ctx->staged_len.clear();
+                if (longest > (uint64_t)kMaxRowsSinglePass) ctx->staged_len.resize(total);
+                uint64_t pos = 0;
+                for (size_t k = 0; k < nd; ++k) {
+                    Device &d = ctx->devs[k];
+                    d.n_first = pos;
+                    d.n_count = at(k, kBhCount);
+                    d.rseq_bytes = at(k, kBhSum);
+                    d.copy_pending = false;
+                    if (!ctx->staged_len.empty() && d.n_count) {
+                        // the long-row path orders its tasks by length: a long bucket's lengths come from the caller's
+                        // offsets (such reads are few)
+                        std::vector<uint32_t> ids(d.n_count);
+                        CU(ctx, cudaSetDevice(d.id));
+                        CU(ctx, cudaMemcpy(ids.data(), d.bh_list.as<uint32_t>() + at(k, kBhStart), d.n_count * sizeof(uint32_t),
+                                           cudaMemcpyDeviceToHost));
+                        for (uint64_t t = 0; t < d.n_count; ++t) {
+                            const uint64_t i = first[k] + ids[t];
+                            ctx->staged_len[pos + t] = (uint32_t)(offsets[i + 1] - offsets[i]);
+                        }
+                    }
+                    pos += d.n_count;
+                }
+                rc = for_each_device(ctx, [&](Device &d) {
+                    const size_t k = (size_t)(&d - ctx->devs.data());
+                    return align_bucket(ctx, d, three_pass, S, at(k, kBhStart), at(k, kBhMax), cigar_cap, &acc_used[k]);
+                });
+                if (rc) return rc;
+                aligned += total;
+                aligned_cells += ctx->staged_cells;
+            }
+            rc = pv.leave();
+            if (rc) return rc;
+        }
+        ctx->staged_n = real_n;
+        for (size_t k = 0; k < nd; ++k) {
+            ctx->devs[k].n_first = first[k];
+            ctx->devs[k].n_count = count[k];
+        }
+        uint64_t need = 0;
+        for (uint64_t u : acc_used) need += u;
+        if (need > cigar_cap) {
+            cigar_off[0] = need;
+            sync_and_time(ctx);
+            return fail(ctx, ZOE_CUDA_E_CIGAR_CAP, "CIGAR buffer too small: the best hits need %llu words, have %llu",
+                        (unsigned long long)need, (unsigned long long)cigar_cap);
+        }
+        // the CIGAR stream in read order
+        for (size_t k = 0; k < nd; ++k) {
+            Device &d = ctx->devs[k];
+            if (d.n_count == 0) continue;
+            CU(ctx, cudaSetDevice(d.id));
+            CU(ctx, d.bh_cig_off.reserve((d.n_count + 1) * sizeof(uint64_t)));
+            CU(ctx, d.bh_cig.reserve(std::max<uint64_t>(acc_used[k], 1) * sizeof(uint32_t)));
+            rc = scan_counts(ctx, d, d.bh_cig_count.as<uint32_t>(), d.n_count, d.bh_cig_off.as<uint64_t>(),
+                             d.bh_tab.as<unsigned long long>() + (size_t)kBhTabRows * K);
+            if (rc) return rc;
+            if (acc_used[k]) {
+                const uint32_t blocks = (uint32_t)std::min<uint64_t>((d.n_count + 7) / 8, (uint64_t)d.sm_count * 16);
+                best_hit_cigar_gather_kernel<<<blocks, 256, 0, d.stream>>>(d.bh_acc.as<uint32_t>(), d.bh_cig_src.as<uint64_t>(),
+                                                                          d.bh_cig_count.as<uint32_t>(), d.n_count,
+                                                                          d.bh_cig_off.as<uint64_t>(), d.bh_cig.as<uint32_t>());
+                CU(ctx, cudaGetLastError());
+                ctx->last_launches++;
+            }
+        }
+        ctx->stats.pairs += aligned;
+        ctx->stats.cells += aligned_cells;
+    }
+    // per-read outputs (and the CIGAR stream) to the caller
+    uint64_t cig_base = 0;
+    for (size_t k = 0; k < nd; ++k) {
+        Device &d = ctx->devs[k];
+        if (d.n_count == 0) continue;
+        CU(ctx, cudaSetDevice(d.id));
+        const size_t first = d.n_first, cnt = d.n_count;
+        auto d2h = [&](void *dst, const DevBuf &src, size_t elem) -> cudaError_t {
+            if (!dst) return cudaSuccess;
+            return cudaMemcpyAsync((uint8_t *)dst + first * elem, src.p, cnt * elem, cudaMemcpyDeviceToHost, d.stream);
+        };
+        CU(ctx, d2h(hit, d.bh_hit, 4));
+        CU(ctx, d2h(strand, d.bh_strand, 1));
+        CU(ctx, d2h(score, d.bh_out32[0], 4));
+        CU(ctx, d2h(status, d.bh_out8[0], 1));
+        CU(ctx, d2h(tier, d.bh_out8[1], 1));
+        CU(ctx, d2h(runner_up, d.bh_runner, 4));
+        if (!align) continue;
+        CU(ctx, d2h(ref_start, d.bh_out32[1], 4));
+        CU(ctx, d2h(ref_end, d.bh_out32[2], 4));
+        CU(ctx, d2h(query_start, d.bh_out32[3], 4));
+        CU(ctx, d2h(query_end, d.bh_out32[4], 4));
+        CU(ctx, d2h(hazard, d.bh_out8[2], 1));
+        CU(ctx, cudaMemcpyAsync(cigar_off + first, d.bh_cig_off.p, (cnt + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost,
+                                d.stream));
+        if (acc_used[k])
+            CU(ctx, cudaMemcpyAsync(cigar + cig_base, d.bh_cig.p, acc_used[k] * sizeof(uint32_t), cudaMemcpyDeviceToHost,
+                                    d.stream));
+        CU(ctx, cudaStreamSynchronize(d.stream));
+        if (cig_base)
+            for (size_t i = 0; i <= cnt; ++i) cigar_off[first + i] += cig_base;
+        cig_base += acc_used[k];
+    }
+    if (align && n == 0) cigar_off[0] = 0;
+    rc = sync_and_time(ctx);
+    if (rc) return rc;
+    view.ok = true;
+    if (align) return 0;
+    rc = gather_stats(ctx);  // (real view: pairs and cells of one strand)
+    ctx->stats.pairs *= S;
+    ctx->stats.cells *= S;
+    return rc;
+}
+
 }  // namespace
 
 // =================================================================================================
@@ -3175,6 +3662,11 @@ void zoe_cuda_destroy(zoe_cuda_ctx *ctx) {
             b->release();
         for (DevBuf &b : d.sel32) b.release();
         for (DevBuf &b : d.sel8) b.release();
+        for (DevBuf *b : {&d.bh_seq, &d.bh_off, &d.bh_key, &d.bh_tab, &d.bh_list, &d.bh_llen, &d.bh_loff, &d.bh_hit,
+                          &d.bh_strand, &d.bh_runner, &d.bh_cig_count, &d.bh_cig_src, &d.bh_acc, &d.bh_cig_off, &d.bh_cig})
+            b->release();
+        for (DevBuf &b : d.bh_out32) b.release();
+        for (DevBuf &b : d.bh_out8) b.release();
         if (d.ev_begin) cudaEventDestroy(d.ev_begin);
         if (d.ev_end) cudaEventDestroy(d.ev_end);
         if (d.ev_k0) cudaEventDestroy(d.ev_k0);
@@ -3269,77 +3761,7 @@ int zoe_cuda_set_profiled(zoe_cuda_ctx *ctx, const uint8_t *concat, const uint64
         if (len == 0) return fail(ctx, ZOE_CUDA_E_EMPTY_SEQUENCE, "profiled sequence %u is empty", j);
         max_len = std::max<uint32_t>(max_len, (uint32_t)len);
     }
-    ctx->plans.clear();
-    ctx->profiled_epoch++;
-    ctx->n_prof = n;
-    ctx->max_prof_len = max_len;
-    ctx->prof_bytes.assign(concat + offsets[0], concat + offsets[n]);
-    ctx->prof_off.resize(n + 1);
-    ctx->coff.resize(n + 1);
-    for (uint32_t j = 0; j <= n; ++j) {
-        ctx->prof_off[j] = offsets[j] - offsets[0];
-        ctx->coff[j] = (uint32_t)ctx->prof_off[j];
-    }
-    // visiting order for the two-stream score kernel: longest first, so paired sweeps have similar lengths
-    ctx->corder.resize(n);
-    for (uint32_t j = 0; j < n; ++j) ctx->corder[j] = j;
-    std::stable_sort(ctx->corder.begin(), ctx->corder.end(), [&](uint32_t a, uint32_t b) {
-        return ctx->coff[a + 1] - ctx->coff[a] > ctx->coff[b + 1] - ctx->coff[b];
-    });
-    // dense column-symbol codes: only the symbols that occur in the profiled set get a table row
-    int dense[64];
-    for (int i = 0; i < 64; ++i) dense[i] = -1;
-    std::vector<int> sym_of_dense;
-    ctx->ccodes.resize(total);
-    for (uint64_t i = 0; i < total; ++i) {
-        int s = ctx->lut[ctx->prof_bytes[i]];
-        if (dense[s] < 0) {
-            dense[s] = (int)sym_of_dense.size();
-            sym_of_dense.push_back(s);
-        }
-        ctx->ccodes[i] = (uint8_t)dense[s];
-    }
-    ctx->n_csym = (int)sym_of_dense.size();
-    // wk[c][r] = weights[streamed symbol r][profiled symbol c]  (profile.rs:290-291: the profile row is
-    // indexed by the streamed symbol, the lane by the profiled residue)
-    ctx->wk.assign((size_t)ctx->n_csym * ctx->S, 0);
-    for (int c = 0; c < ctx->n_csym; ++c)
-        for (int r = 0; r < ctx->S; ++r) ctx->wk[(size_t)c * ctx->S + r] = ctx->weights[(size_t)r * ctx->S + sym_of_dense[c]];
-    // regroup a panel that does not fit the staging area (see launch_score)
-    ctx->groups.clear();
-    ctx->ccodes_g.clear();
-    ctx->coff_g.clear();
-    ctx->corder_g.clear();
-    if (total > kColsSmemLimit && n > 1) {
-        uint32_t j = 0;
-        while (j < n) {
-            zoe_cuda_ctx::ColGroup g{};
-            g.j0 = j;
-            g.byte_start = (uint32_t)ctx->ccodes_g.size();
-            g.coff_start = (uint32_t)ctx->corder_g.size();
-            uint32_t bytes = 0;
-            while (j < n && (bytes == 0 || bytes + (ctx->coff[j + 1] - ctx->coff[j]) <= kColsSmemLimit)) {
-                ctx->coff_g.push_back(bytes);
-                bytes += ctx->coff[j + 1] - ctx->coff[j];
-                ++j;
-            }
-            ctx->coff_g.push_back(bytes);
-            g.n = j - g.j0;
-            g.bytes = bytes;
-            ctx->ccodes_g.insert(ctx->ccodes_g.end(), ctx->ccodes.begin() + ctx->coff[g.j0], ctx->ccodes.begin() + ctx->coff[j]);
-            ctx->ccodes_g.resize((ctx->ccodes_g.size() + 15) & ~(size_t)15, 0);  // next group starts 16-byte aligned (TMA)
-            std::vector<uint32_t> order(g.n);
-            for (uint32_t q = 0; q < g.n; ++q) order[q] = q;
-            std::stable_sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) {
-                return ctx->coff[g.j0 + a + 1] - ctx->coff[g.j0 + a] > ctx->coff[g.j0 + b + 1] - ctx->coff[g.j0 + b];
-            });
-            ctx->corder_g.insert(ctx->corder_g.end(), order.begin(), order.end());
-            ctx->groups.push_back(g);
-        }
-        ctx->ccodes_g.resize(ctx->ccodes_g.size() + 16, 0);
-        if (ctx->groups.size() < 2) ctx->groups.clear();
-    }
-    int rc = upload_scoring_and_profiled(ctx);
+    int rc = install_profiled(ctx, concat, offsets, n, max_len);
     if (rc) return rc;
     ctx->have_profiled = true;
     ctx->staged = false;
@@ -3658,6 +4080,24 @@ int zoe_cuda_sw_align_3pass_both_strands_batch(zoe_cuda_ctx *ctx, const uint8_t 
     if (!ctx) return ZOE_CUDA_E_BAD_ARG;
     return align_both_strands(ctx, true, streamed_concat, offsets, n, score, status, tier, ref_start, ref_end, query_start,
                               query_end, cigar, cigar_off, cigar_cap, nullptr, strand);
+}
+
+int zoe_cuda_sw_score_best_hit_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_concat, const uint64_t *offsets,
+                                     uint64_t n, int both_strands, uint32_t *hit, uint8_t *strand, uint32_t *score,
+                                     uint8_t *status, uint8_t *tier, uint32_t *runner_up) {
+    if (!ctx) return ZOE_CUDA_E_BAD_ARG;
+    return best_hit(ctx, false, both_strands != 0, false, streamed_concat, offsets, n, hit, strand, score, status, tier,
+                    runner_up, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 0, nullptr);
+}
+
+int zoe_cuda_sw_align_best_hit_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_concat, const uint64_t *offsets,
+                                     uint64_t n, int both_strands, int three_pass, uint32_t *hit, uint8_t *strand,
+                                     uint32_t *score, uint8_t *status, uint8_t *tier, uint32_t *runner_up,
+                                     uint32_t *ref_start, uint32_t *ref_end, uint32_t *query_start, uint32_t *query_end,
+                                     uint32_t *cigar, uint64_t *cigar_off, uint64_t cigar_cap, uint8_t *hazard) {
+    if (!ctx) return ZOE_CUDA_E_BAD_ARG;
+    return best_hit(ctx, true, both_strands != 0, three_pass != 0, streamed_concat, offsets, n, hit, strand, score, status,
+                    tier, runner_up, ref_start, ref_end, query_start, query_end, cigar, cigar_off, cigar_cap, hazard);
 }
 
 int zoe_cuda_sneaky_snake_batch(zoe_cuda_ctx *ctx, const uint8_t *refs, const uint64_t *ref_offsets, const uint8_t *queries,

@@ -6,6 +6,9 @@ Mirrors (paths relative to the zoe repository):
   * ``SamData::unmapped``        src/data/records/sam/mod.rs:201-214  (FLAG 4, POS 0, MAPQ 255, CIGAR/SEQ/QUAL ``*``)
   * ``Display for SamData``      src/data/records/sam/std_traits.rs:3-43 (tab-separated, missing SEQ/QUAL as ``*``)
 
+Results of the best-hit search (``CudaProfiles.align_best_hit_arrays``) become one primary record per read:
+``sam_lines_best_hit``.
+
 Results of the both-strand search pass their strands as ``strand``: a reverse-strand pair is written as SAM writes a read
 that maps to the reverse strand -- FLAG bit 16 set, SEQ reverse-complemented, QUAL reversed (its POS and CIGAR already
 refer to the reverse complement).
@@ -105,3 +108,27 @@ def sam_lines_from_arrays(a: dict, n_profiled: int, qnames: Sequence[str], rname
             rec = SamData(qnames[i], f, rnames[j], int(a["ref_start"][k]) + 1, mapq, cigar, s, q,
                           opt_fields=[f"AS:i:{int(a['score'][k])}"])
             yield str(rec)
+
+
+def sam_lines_best_hit(a: dict, qnames: Sequence[str], rnames: Sequence[str], buf: np.ndarray, offs: np.ndarray,
+                       quals: Optional[Sequence[bytes]] = None, mapq: int = 255, flag: int = 0) -> Iterable[str]:
+    """One SAM line per read from ``CudaProfiles.align_best_hit_arrays``: a Some winner maps to ``rnames[hit]`` at
+    ``ref_start + 1`` with its CIGAR and ``AS:i:score``, plus ``XS:i:runner_up`` when the runner-up is above 0; a strand-1
+    winner is a reverse-strand record (FLAG 16, reverse-complemented SEQ, reversed QUAL).  Any other read is
+    ``SamData::unmapped`` with RNAME ``*``."""
+    n = len(offs) - 1
+    cig, coff = a["cigar"], a["cigar_off"]
+    for i in range(n):
+        if int(a["status"][i]) != _lib.SOME:
+            yield str(SamData.unmapped(qnames[i], "*"))
+            continue
+        seq = bytes(buf[int(offs[i]):int(offs[i + 1])])
+        qual = bytes(quals[i]) if quals is not None else b"*"
+        words = cig[int(coff[i]):int(coff[i + 1])]
+        cigar = "".join(f"{int(w) >> 4}{_OPS[int(w) & 15]}" for w in words)
+        f, s, q = _oriented(int(a["strand"][i]) == 1, flag, seq, qual)
+        tags = [f"AS:i:{int(a['score'][i])}"]
+        if int(a["runner_up"][i]) > 0:
+            tags.append(f"XS:i:{int(a['runner_up'][i])}")
+        yield str(SamData(qnames[i], f, rnames[int(a["hit"][i])], int(a["ref_start"][i]) + 1, mapq, cigar, s, q,
+                          opt_fields=tags))
