@@ -204,6 +204,53 @@ int zoe_cuda_sw_align_best_hit_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_
                                      uint32_t *ref_start, uint32_t *ref_end, uint32_t *query_start, uint32_t *query_end,
                                      uint32_t *cigar, uint64_t *cigar_off, uint64_t cigar_cap, uint8_t *hazard);
 
+/* Paired-end best-hit search: each read pair's profiled sequence and orientation, chosen on the device from both mates;
+ * the align entry point aligns both mates there and reports proper pairs and TLEN.
+ *   layout      n_pairs pairs: mate 1 of pair i is sequence i of the mate-1 batch, mate 2 sequence i of the mate-2
+ *               batch.  hit, proper and tlen have n_pairs entries; every other output is per mate, 2 n_pairs entries
+ *               at index 2i + m (m = 0 for mate 1, 1 for mate 2); cigar_off has 2 n_pairs + 1 entries and the CIGAR
+ *               stream is in that order.
+ *   candidates  the library is FR, as Illumina paired-end is: the mates come from opposite strands.  Pair i has the
+ *               candidates (j, o) for every profiled j and o in {0, 1}; under (j, o) mate 1 is on strand o and mate 2 on
+ *               strand 1 - o (strand 1: the reverse complement, with the complement table of the both-strand search).
+ *               A mate's result under a candidate is what the single-strand score call returns for that sequence
+ *               against j.
+ *   selection   each candidate's key is first the number of Overflowed mates (0-2), then the sum of its two mates'
+ *               Some scores; the highest key wins, ties go to the smallest j, then to o = 0.  A candidate whose mates
+ *               are both Unmapped has key (0, 0); a pair whose candidates all have key (0, 0) -- 0-length mates
+ *               included -- gets hit 0, o = 0 and two Unmapped mates.
+ *   strand, score, status, tier   each mate's result under the winning candidate.
+ *   runner_up   per mate: its largest Some score among candidates with j != hit, on either strand; 0 when the mate is
+ *               not Some (the best-hit XS definition, per mate).
+ * The align entry point gives each mate that is Some under the winner exactly what zoe_cuda_sw_align_batch returns for
+ * (the mate, or its reverse complement on strand 1, against hit); three_pass: zoe_cuda_sw_align_3pass_batch, hazard 0.
+ * A mate that is not Some gets zero ranges and an empty CIGAR.  Coordinates and CIGAR of a strand-1 mate refer to its
+ * reverse complement, as in the both-strand search.  A mate's panel range is [ref_start, ref_end) when
+ * profiled_is_query is 0 and [query_start, query_end) when it is 1.
+ *   tlen        when both mates are Some, extent = max(ends) - min(starts); tlen is +extent when mate 1's start is
+ *               smaller, or the starts are equal and o = 0, else -extent.  It is mate 1's TLEN (a 32-bit int); mate
+ *               2's is -tlen.
+ *               0 when the mates are not both Some.
+ *   proper      1 iff both mates are Some, the forward-strand mate's start is at most the reverse-strand mate's start
+ *               (the mates point inward) and min_insert <= extent <= max_insert.
+ * min_insert > max_insert fails with ZOE_CUDA_E_BAD_ARG.  Every output may be NULL, except cigar_off, and cigar when
+ * cigar_cap > 0; ZOE_CUDA_E_CIGAR_CAP writes the exact need to cigar_off[0].  Limits are those of
+ * zoe_cuda_sw_score_both_strands_batch applied to the 2 n_pairs mates.  zoe_cuda_last_stats counts as the best-hit
+ * search does: the score pass over every candidate (4 n_pairs x n_profiled strand-pairs) plus the aligned mates.  A
+ * call leaves nothing staged and the profiled set as it was, error or not.  Not covered: RF / FF libraries, mate rescue
+ * (re-aligning an unmapped mate near its mapped mate), MAPQ, and supplementary or secondary records (DESIGN.md 4.10). */
+int zoe_cuda_sw_score_paired_best_hit_batch(zoe_cuda_ctx *ctx, const uint8_t *mate1_concat, const uint64_t *mate1_offsets,
+                                            const uint8_t *mate2_concat, const uint64_t *mate2_offsets, uint64_t n_pairs,
+                                            uint32_t *hit, uint8_t *strand, uint32_t *score, uint8_t *status, uint8_t *tier,
+                                            uint32_t *runner_up);
+int zoe_cuda_sw_align_paired_best_hit_batch(zoe_cuda_ctx *ctx, const uint8_t *mate1_concat, const uint64_t *mate1_offsets,
+                                            const uint8_t *mate2_concat, const uint64_t *mate2_offsets, uint64_t n_pairs,
+                                            int three_pass, uint32_t min_insert, uint32_t max_insert, uint32_t *hit,
+                                            uint8_t *proper, int *tlen, uint8_t *strand, uint32_t *score, uint8_t *status,
+                                            uint8_t *tier, uint32_t *runner_up, uint32_t *ref_start, uint32_t *ref_end,
+                                            uint32_t *query_start, uint32_t *query_end, uint32_t *cigar, uint64_t *cigar_off,
+                                            uint64_t cigar_cap, uint8_t *hazard);
+
 /* Batched sneaky_snake(reference, query, threshold) (src/alignment/sneaky_snake.rs:78-131): the SneakySnake
  * pre-alignment filter for pair i = (reference i, query i).  out[i]: 1 = Some(true) (edits within
  * floor(len(query) * threshold)), 0 = Some(false), 2 = None (threshold outside 0..=1, or the length difference exceeds

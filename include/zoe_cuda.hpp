@@ -202,28 +202,82 @@ class CudaProfiles {
             rc = call();
         }
         check(rc);
-        static const char ops[] = {'M', 'I', 'D', '?', 'S'};
         std::vector<BestHit> out(n);
+        for (size_t i = 0; i < n; ++i)
+            out[i] = best_hit_at(i, hit[i], seqs[i], strand, score, status, ru, rs, re, qs, qe, coff, cig);
+        return out;
+    }
+
+    // Paired-end best-hit search (zoe_cuda.h), an FR library: per read pair (mates1[i], mates2[i]), the profiled sequence
+    // and orientation both mates support best, each mate's alignment, proper-pair flag and mate 1's TLEN.
+    struct PairedHit {
+        uint32_t index = 0;
+        bool proper = false;
+        int32_t tlen = 0;
+        BestHit mate1, mate2;
+    };
+    std::vector<PairedHit> sw_align_paired_best_hit(const std::vector<std::string> &mates1,
+                                                    const std::vector<std::string> &mates2, uint32_t min_insert,
+                                                    uint32_t max_insert, bool three_pass = false) {
+        if (mates1.size() != mates2.size()) throw std::invalid_argument("mate lists differ in length");
+        std::vector<uint8_t> buf1, buf2;
+        std::vector<uint64_t> off1, off2;
+        pack(mates1, buf1, off1);
+        pack(mates2, buf2, off2);
+        const size_t n = mates1.size(), m = 2 * n + 1;
+        std::vector<uint32_t> hit(n + 1), score(m), ru(m), rs(m), re(m), qs(m), qe(m);
+        std::vector<int> tlen(n + 1);
+        std::vector<uint8_t> proper(n + 1), strand(m), status(m), tier(m);
+        std::vector<uint64_t> coff(m + 1);
+        std::vector<uint32_t> cig(16 * m + 1024);
+        auto call = [&]() {
+            return zoe_cuda_sw_align_paired_best_hit_batch(
+                ctx_, buf1.data(), off1.data(), buf2.data(), off2.data(), n, three_pass ? 1 : 0, min_insert, max_insert,
+                hit.data(), proper.data(), tlen.data(), strand.data(), score.data(), status.data(), tier.data(), ru.data(),
+                rs.data(), re.data(), qs.data(), qe.data(), cig.data(), coff.data(), cig.size(), nullptr);
+        };
+        int rc = call();
+        if (rc == ZOE_CUDA_E_CIGAR_CAP) {
+            cig.resize(coff[0] + 16);
+            rc = call();
+        }
+        check(rc);
+        std::vector<PairedHit> out(n);
         for (size_t i = 0; i < n; ++i) {
-            BestHit &b = out[i];
-            b.index = hit[i];
-            b.strand = static_cast<Strand>(strand[i]);
-            b.runner_up = ru[i];
-            b.result.status = static_cast<Status>(status[i]);
-            if (!b.result.is_some()) continue;
-            Alignment &a = b.result.value;
-            a.score = score[i];
-            a.ref_range = {rs[i], re[i]};
-            a.query_range = {qs[i], qe[i]};
-            for (uint64_t w = coff[i]; w < coff[i + 1]; ++w) a.states.push_back({cig[w] >> 4, ops[cig[w] & 7]});
-            const bool streamed_is_query = streamed_are_ == SeqSrc::Query;
-            a.ref_len = (uint32_t)(streamed_is_query ? targets_[b.index].size() : seqs[i].size());
-            a.query_len = (uint32_t)(streamed_is_query ? seqs[i].size() : targets_[b.index].size());
+            out[i].index = hit[i];
+            out[i].proper = proper[i] != 0;
+            out[i].tlen = tlen[i];
+            out[i].mate1 = best_hit_at(2 * i, hit[i], mates1[i], strand, score, status, ru, rs, re, qs, qe, coff, cig);
+            out[i].mate2 = best_hit_at(2 * i + 1, hit[i], mates2[i], strand, score, status, ru, rs, re, qs, qe, coff, cig);
         }
         return out;
     }
 
   private:
+    // Entry k of a best-hit or paired call's per-sequence outputs, for streamed sequence seq placed on profiled j.
+    BestHit best_hit_at(size_t k, uint32_t j, const std::string &seq, const std::vector<uint8_t> &strand,
+                        const std::vector<uint32_t> &score, const std::vector<uint8_t> &status,
+                        const std::vector<uint32_t> &ru, const std::vector<uint32_t> &rs, const std::vector<uint32_t> &re,
+                        const std::vector<uint32_t> &qs, const std::vector<uint32_t> &qe,
+                        const std::vector<uint64_t> &coff, const std::vector<uint32_t> &cig) const {
+        static const char ops[] = {'M', 'I', 'D', '?', 'S'};
+        BestHit b;
+        b.index = j;
+        b.strand = static_cast<Strand>(strand[k]);
+        b.runner_up = ru[k];
+        b.result.status = static_cast<Status>(status[k]);
+        if (!b.result.is_some()) return b;
+        Alignment &a = b.result.value;
+        a.score = score[k];
+        a.ref_range = {rs[k], re[k]};
+        a.query_range = {qs[k], qe[k]};
+        for (uint64_t w = coff[k]; w < coff[k + 1]; ++w) a.states.push_back({cig[w] >> 4, ops[cig[w] & 7]});
+        const bool streamed_is_query = streamed_are_ == SeqSrc::Query;
+        a.ref_len = (uint32_t)(streamed_is_query ? targets_[j].size() : seq.size());
+        a.query_len = (uint32_t)(streamed_is_query ? seq.size() : targets_[j].size());
+        return b;
+    }
+
     template <class T>
     static std::vector<std::pair<T, Strand>> with_strand(std::vector<T> v, const std::vector<uint8_t> &strand) {
         std::vector<std::pair<T, Strand>> out;

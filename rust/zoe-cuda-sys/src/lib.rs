@@ -106,6 +106,18 @@ unsafe extern "C" {
         runner_up: *mut u32, ref_start: *mut u32, ref_end: *mut u32, query_start: *mut u32, query_end: *mut u32,
         cigar: *mut u32, cigar_off: *mut u64, cigar_cap: u64, hazard: *mut u8,
     ) -> c_int;
+    pub fn zoe_cuda_sw_score_paired_best_hit_batch(
+        ctx: *mut zoe_cuda_ctx, mate1_concat: *const u8, mate1_offsets: *const u64, mate2_concat: *const u8,
+        mate2_offsets: *const u64, n_pairs: u64, hit: *mut u32, strand: *mut u8, score: *mut u32, status: *mut u8,
+        tier: *mut u8, runner_up: *mut u32,
+    ) -> c_int;
+    pub fn zoe_cuda_sw_align_paired_best_hit_batch(
+        ctx: *mut zoe_cuda_ctx, mate1_concat: *const u8, mate1_offsets: *const u64, mate2_concat: *const u8,
+        mate2_offsets: *const u64, n_pairs: u64, three_pass: c_int, min_insert: u32, max_insert: u32, hit: *mut u32,
+        proper: *mut u8, tlen: *mut c_int, strand: *mut u8, score: *mut u32, status: *mut u8, tier: *mut u8,
+        runner_up: *mut u32, ref_start: *mut u32, ref_end: *mut u32, query_start: *mut u32, query_end: *mut u32,
+        cigar: *mut u32, cigar_off: *mut u64, cigar_cap: u64, hazard: *mut u8,
+    ) -> c_int;
     pub fn zoe_cuda_run_ranges_staged(ctx: *mut zoe_cuda_ctx) -> c_int;
     pub fn zoe_cuda_run_3pass_staged(ctx: *mut zoe_cuda_ctx) -> c_int;
     pub fn zoe_cuda_stage_streamed(ctx: *mut zoe_cuda_ctx, streamed_concat: *const u8, offsets: *const u64, n: u64) -> c_int;

@@ -36,6 +36,18 @@ pub struct BestHit {
     pub runner_up: u32,
 }
 
+/// One read pair's result of the paired-end best-hit search (an FR library): the profiled sequence `index` both mates
+/// were placed on, `proper` (the mates point inward within the insert bounds), `tlen` (mate 1's SAM TLEN; mate 2's is
+/// `-tlen`) and each mate's `BestHit`, whose `strand` is the mate's strand in the chosen orientation.
+#[derive(Debug)]
+pub struct PairedHit {
+    pub index:  usize,
+    pub proper: bool,
+    pub tlen:   i32,
+    pub mate1:  BestHit,
+    pub mate2:  BestHit,
+}
+
 #[derive(Debug)]
 pub enum CudaError {
     Profile(ProfileError),
@@ -174,30 +186,81 @@ impl CudaProfiles {
             self.check(rc, 0, 0)?;
             break;
         }
-        const OPS: [u8; 5] = [b'M', b'I', b'D', b'?', b'S'];
         Ok(seqs.iter().enumerate().map(|(i, seq)| {
             let j = hit[i] as usize;
-            let result = match status[i] {
-                sys::ZOE_CUDA_SOME => {
-                    let ciglets = cigar[coff[i] as usize..coff[i + 1] as usize]
-                        .iter()
-                        .map(|w| Ciglet { inc: (w >> 4) as usize, op: OPS[(w & 7) as usize] });
-                    let (ref_len, query_len) =
-                        if self.profiled_is_query { (seq.len(), self.profiled_lens[j]) } else { (self.profiled_lens[j], seq.len()) };
-                    MaybeAligned::Some(Alignment {
-                        score: score[i],
-                        ref_range: rs[i] as usize..re[i] as usize,
-                        query_range: qs[i] as usize..qe[i] as usize,
-                        states: AlignmentStates::from_ciglets_unchecked(ciglets),
-                        ref_len,
-                        query_len,
-                    })
-                }
-                sys::ZOE_CUDA_OVERFLOWED => MaybeAligned::Overflowed,
-                _ => MaybeAligned::Unmapped,
-            };
+            let result = self.hit_alignment(seq, j, status[i], score[i], [rs[i], re[i], qs[i], qe[i]],
+                                            &cigar[coff[i] as usize..coff[i + 1] as usize]);
             BestHit { index: j, strand: strand(sd[i]), result, runner_up: ru[i] }
         }).collect())
+    }
+
+    /// Paired-end best-hit search: one `PairedHit` per read pair `(mates1[i], mates2[i])`.  The pair's profiled
+    /// sequence and orientation maximise (Overflowed mates, sum of the mates' Some scores), ties to the smallest index
+    /// and then to mate 1 forward; each mate is aligned as `sw_align_batch` (`three_pass`: `sw_align_3pass_batch`)
+    /// aligns it, or its reverse complement on `Strand::Reverse`.  `proper` and `tlen` use the insert bounds.
+    pub fn sw_align_paired_best_hit_batch(&self, mates1: &[&[u8]], mates2: &[&[u8]], three_pass: bool, min_insert: u32,
+                                          max_insert: u32) -> Result<Vec<PairedHit>, CudaError> {
+        assert_eq!(mates1.len(), mates2.len(), "mate lists differ in length");
+        let ((c1, o1), (c2, o2)) = (pack(mates1), pack(mates2));
+        let n = mates1.len();
+        let m = 2 * n + 1;
+        let (mut hit, mut proper, mut tlen) = (vec![0u32; n + 1], vec![0u8; n + 1], vec![0i32; n + 1]);
+        let (mut score, mut ru) = (vec![0u32; m], vec![0u32; m]);
+        let (mut sd, mut status, mut tier) = (vec![0u8; m], vec![0u8; m], vec![0u8; m]);
+        let (mut rs, mut re, mut qs, mut qe) = (vec![0u32; m], vec![0u32; m], vec![0u32; m], vec![0u32; m]);
+        let mut coff = vec![0u64; m + 1];
+        let mut cigar = vec![0u32; 16 * m + 1024];
+        loop {
+            let rc = unsafe {
+                sys::zoe_cuda_sw_align_paired_best_hit_batch(self.ctx, c1.as_ptr(), o1.as_ptr(), c2.as_ptr(), o2.as_ptr(),
+                    n as u64, three_pass as std::os::raw::c_int, min_insert, max_insert, hit.as_mut_ptr(),
+                    proper.as_mut_ptr(), tlen.as_mut_ptr(), sd.as_mut_ptr(), score.as_mut_ptr(), status.as_mut_ptr(),
+                    tier.as_mut_ptr(), ru.as_mut_ptr(), rs.as_mut_ptr(), re.as_mut_ptr(), qs.as_mut_ptr(), qe.as_mut_ptr(),
+                    cigar.as_mut_ptr(), coff.as_mut_ptr(), cigar.len() as u64, std::ptr::null_mut())
+            };
+            if rc == sys::ZOE_CUDA_E_CIGAR_CAP {
+                cigar.resize(coff[0] as usize + 16, 0);
+                continue;
+            }
+            self.check(rc, 0, 0)?;
+            break;
+        }
+        let mate = |k: usize, seq: &[u8], j: usize| BestHit {
+            index: j,
+            strand: strand(sd[k]),
+            result: self.hit_alignment(seq, j, status[k], score[k], [rs[k], re[k], qs[k], qe[k]],
+                                       &cigar[coff[k] as usize..coff[k + 1] as usize]),
+            runner_up: ru[k],
+        };
+        Ok((0..n).map(|i| {
+            let j = hit[i] as usize;
+            PairedHit { index: j, proper: proper[i] != 0, tlen: tlen[i], mate1: mate(2 * i, mates1[i], j),
+                        mate2: mate(2 * i + 1, mates2[i], j) }
+        }).collect())
+    }
+
+    /// One best-hit or paired result's alignment against profiled sequence `j`; `ranges` = ref_start, ref_end,
+    /// query_start, query_end.
+    fn hit_alignment(&self, seq: &[u8], j: usize, status: u8, score: u32, ranges: [u32; 4], words: &[u32])
+                     -> MaybeAligned<Alignment<u32>> {
+        const OPS: [u8; 5] = [b'M', b'I', b'D', b'?', b'S'];
+        match status {
+            sys::ZOE_CUDA_SOME => {
+                let ciglets = words.iter().map(|w| Ciglet { inc: (w >> 4) as usize, op: OPS[(w & 7) as usize] });
+                let (ref_len, query_len) =
+                    if self.profiled_is_query { (seq.len(), self.profiled_lens[j]) } else { (self.profiled_lens[j], seq.len()) };
+                MaybeAligned::Some(Alignment {
+                    score,
+                    ref_range: ranges[0] as usize..ranges[1] as usize,
+                    query_range: ranges[2] as usize..ranges[3] as usize,
+                    states: AlignmentStates::from_ciglets_unchecked(ciglets),
+                    ref_len,
+                    query_len,
+                })
+            }
+            sys::ZOE_CUDA_OVERFLOWED => MaybeAligned::Overflowed,
+            _ => MaybeAligned::Unmapped,
+        }
     }
 
     /// `strand`: the both-strand entry points, the strand of every pair written there.

@@ -8,6 +8,7 @@ from .alignment import (  # noqa: F401
     BestHit,
     CudaProfiles,
     MaybeAligned,
+    PairedHit,
     ProfileError,
     ScoreAndRanges,
     SeqSrc,

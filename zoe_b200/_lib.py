@@ -23,6 +23,7 @@ SYMBOLS = [
     "zoe_cuda_sw_score_both_strands_batch", "zoe_cuda_sw_score_ranges_both_strands_batch",
     "zoe_cuda_sw_align_both_strands_batch", "zoe_cuda_sw_align_3pass_both_strands_batch",
     "zoe_cuda_sw_score_best_hit_batch", "zoe_cuda_sw_align_best_hit_batch",
+    "zoe_cuda_sw_score_paired_best_hit_batch", "zoe_cuda_sw_align_paired_best_hit_batch",
 ]
 
 
@@ -76,6 +77,11 @@ def load() -> C.CDLL:
     lib.zoe_cuda_sw_score_best_hit_batch.argtypes = [p, u8p, u64p, C.c_uint64, C.c_int, u32p, u8p, u32p, u8p, u8p, u32p]
     lib.zoe_cuda_sw_align_best_hit_batch.argtypes = [p, u8p, u64p, C.c_uint64, C.c_int, C.c_int, u32p, u8p, u32p, u8p, u8p,
                                                      u32p, u32p, u32p, u32p, u32p, u32p, u64p, C.c_uint64, u8p]
+    lib.zoe_cuda_sw_score_paired_best_hit_batch.argtypes = [p, u8p, u64p, u8p, u64p, C.c_uint64, u32p, u8p, u32p, u8p,
+                                                            u8p, u32p]
+    lib.zoe_cuda_sw_align_paired_best_hit_batch.argtypes = [p, u8p, u64p, u8p, u64p, C.c_uint64, C.c_int, C.c_uint32,
+                                                            C.c_uint32, u32p, u8p, C.POINTER(C.c_int32), u8p, u32p, u8p,
+                                                            u8p, u32p, u32p, u32p, u32p, u32p, u32p, u64p, C.c_uint64, u8p]
     lib.zoe_cuda_sneaky_snake_batch.argtypes = [p, u8p, u64p, u8p, u64p, C.c_uint64, C.c_float, u8p]
     lib.zoe_cuda_stage_streamed.argtypes = [p, u8p, u64p, C.c_uint64]
     lib.zoe_cuda_run_score_staged.argtypes = [p]

@@ -176,6 +176,19 @@ class BestHit:
     runner_up: int
 
 
+@dataclass(frozen=True)
+class PairedHit:
+    """One read pair's result of the paired-end best-hit search: the profiled sequence ``index`` both mates were placed
+    on, ``proper`` (the mates point inward within the insert bounds), ``tlen`` (mate 1's SAM TLEN; mate 2's is
+    ``-tlen``) and a :class:`BestHit` per mate, whose ``strand`` is the mate's strand in the chosen orientation."""
+
+    index: int
+    proper: bool
+    tlen: int
+    mate1: BestHit
+    mate2: BestHit
+
+
 class CudaProfiles:
     """A set of profiled sequences resident on one or more B200s.
 
@@ -630,3 +643,78 @@ class CudaProfiles:
                     (int(a["query_start"][i]), int(a["query_end"][i])), cig, ref_len, query_len))
             out.append(BestHit(j, strand, m, int(a["runner_up"][i])))
         return out
+
+    # ---- paired-end best-hit search: each read pair's profiled sequence and orientation, chosen from both mates ----
+    def sw_score_paired_best_hit_arrays(self, buf1: np.ndarray, offs1: np.ndarray, buf2: np.ndarray, offs2: np.ndarray):
+        """``hit`` per pair (``n`` entries) and, per mate at index ``2 i + m``, ``strand``, ``score``, ``status``,
+        ``tier`` and ``runner_up``, as ``zoe_cuda_sw_score_paired_best_hit_batch`` defines them.  Mate 1 of pair ``i`` is
+        sequence ``i`` of (buf1, offs1), mate 2 sequence ``i`` of (buf2, offs2)."""
+        n = self._pair_count(offs1, offs2)
+        out = self._best_hit_outputs(2 * n)
+        out["hit"] = np.zeros(max(n, 1), dtype=np.uint32)
+        self._check(self._lib.zoe_cuda_sw_score_paired_best_hit_batch(
+            self._h, _p(buf1, C.c_uint8), _p(offs1, C.c_uint64), _p(buf2, C.c_uint8), _p(offs2, C.c_uint64), n,
+            _p(out["hit"], C.c_uint32), _p(out["strand"], C.c_uint8), _p(out["score"], C.c_uint32),
+            _p(out["status"], C.c_uint8), _p(out["tier"], C.c_uint8), _p(out["runner_up"], C.c_uint32)))
+        return {k: v[:n] if k == "hit" else v[:2 * n] for k, v in out.items()}
+
+    def align_paired_best_hit_arrays(self, buf1: np.ndarray, offs1: np.ndarray, buf2: np.ndarray, offs2: np.ndarray,
+                                     three_pass: bool = False, *, min_insert: int, max_insert: int,
+                                     cigar_cap: Optional[int] = None):
+        """:meth:`sw_score_paired_best_hit_arrays` plus ``proper`` (u8) and ``tlen`` (i32) per pair and, per mate,
+        its alignment: ``ref_start`` ... ``query_end``, ``hazard``, ``cigar`` and ``cigar_off`` (``2 n + 1``)."""
+        n = self._pair_count(offs1, offs2)
+        m = max(2 * n, 1)
+        out = self._best_hit_outputs(2 * n)
+        out["hit"] = np.zeros(max(n, 1), dtype=np.uint32)
+        out["proper"] = np.zeros(max(n, 1), dtype=np.uint8)
+        out["tlen"] = np.zeros(max(n, 1), dtype=np.int32)
+        out.update({k: np.zeros(m, dtype=np.uint32) for k in ("ref_start", "ref_end", "query_start", "query_end")})
+        out["hazard"] = np.zeros(m, dtype=np.uint8)
+        out["cigar_off"] = np.zeros(m + 1, dtype=np.uint64)
+        cap = int(cigar_cap) if cigar_cap else max(16 * m, 1024)
+        for _ in range(2):
+            out["cigar"] = np.zeros(cap, dtype=np.uint32)
+            rc = self._lib.zoe_cuda_sw_align_paired_best_hit_batch(
+                self._h, _p(buf1, C.c_uint8), _p(offs1, C.c_uint64), _p(buf2, C.c_uint8), _p(offs2, C.c_uint64), n,
+                int(three_pass), int(min_insert), int(max_insert), _p(out["hit"], C.c_uint32),
+                _p(out["proper"], C.c_uint8), _p(out["tlen"], C.c_int32), _p(out["strand"], C.c_uint8),
+                _p(out["score"], C.c_uint32), _p(out["status"], C.c_uint8), _p(out["tier"], C.c_uint8),
+                _p(out["runner_up"], C.c_uint32), _p(out["ref_start"], C.c_uint32), _p(out["ref_end"], C.c_uint32),
+                _p(out["query_start"], C.c_uint32), _p(out["query_end"], C.c_uint32), _p(out["cigar"], C.c_uint32),
+                _p(out["cigar_off"], C.c_uint64), len(out["cigar"]), _p(out["hazard"], C.c_uint8))
+            if rc == _lib.E_CIGAR_CAP:
+                cap = int(out["cigar_off"][0]) + 16
+                continue
+            self._check(rc)
+            break
+        else:
+            self._check(rc)
+        for k in out:
+            if k in ("hit", "proper", "tlen"):
+                out[k] = out[k][:n]
+            elif k != "cigar":
+                out[k] = out[k][:2 * n + 1] if k == "cigar_off" else out[k][:2 * n]
+        return out
+
+    @staticmethod
+    def _pair_count(offs1: np.ndarray, offs2: np.ndarray) -> int:
+        if len(offs1) != len(offs2):
+            raise ValueError(f"mate batches differ in size: {len(offs1) - 1} and {len(offs2) - 1} sequences")
+        return len(offs1) - 1
+
+    def sw_align_paired_best_hit_batch(self, mates1: Sequence[bytes], mates2: Sequence[bytes], three_pass: bool = False,
+                                       *, min_insert: int, max_insert: int):
+        """One :class:`PairedHit` per read pair ``(mates1[i], mates2[i])`` (an FR library): the profiled sequence and
+        orientation that the two mates support best together, each mate aligned as :meth:`sw_align_batch` aligns it
+        (its reverse complement when its strand is ``Strand.Reverse``)."""
+        m1, m2 = [bytes(s) for s in mates1], [bytes(s) for s in mates2]
+        if len(m1) != len(m2):
+            raise ValueError(f"mate lists differ in length: {len(m1)} and {len(m2)}")
+        (buf1, offs1), (buf2, offs2) = _pack(m1), _pack(m2)
+        a = self.align_paired_best_hit_arrays(buf1, offs1, buf2, offs2, three_pass, min_insert=min_insert,
+                                              max_insert=max_insert)
+        mates = [s for pair in zip(m1, m2) for s in pair]
+        rows = self._best_hit_rows(mates, dict(a, hit=np.repeat(a["hit"], 2)))
+        return [PairedHit(int(a["hit"][i]), bool(a["proper"][i]), int(a["tlen"][i]), rows[2 * i], rows[2 * i + 1])
+                for i in range(len(m1))]

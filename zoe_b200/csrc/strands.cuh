@@ -29,24 +29,54 @@ __host__ __device__ constexpr uint8_t complement_base(uint8_t c) {
     }
 }
 
-// Doubles a staged shard of n sequences: out sequence 2i is sequence i, 2i+1 its reverse complement, at offsets
-// 2 off[i] and 2 off[i] + len_i (off2 gets 2n + 1 entries).  One warp per sequence; memory-bound.
-__global__ void __launch_bounds__(256) strand_expand_kernel(const uint8_t *__restrict__ seq, const uint64_t *__restrict__ off,
-                                                            uint64_t n, uint8_t *__restrict__ seq2, uint64_t *__restrict__ off2) {
+// Source mappings of strand_expand_kernel.  at(i) gives expanded read i's bytes, its length and its position in the
+// concatenation of all n reads; total(n) is that concatenation's length.
+// One staged shard: read i is sequence i.
+struct ExpandSingle {
+    const uint8_t *seq;
+    const uint64_t *off;  // n + 1 entries
+    __device__ __forceinline__ const uint8_t *at(uint64_t i, uint64_t *pos, uint64_t *len) const {
+        *pos = off[i];
+        *len = off[i + 1] - *pos;
+        return seq + *pos;
+    }
+    __device__ __forceinline__ uint64_t total(uint64_t n) const { return off[n]; }
+};
+
+// A staged shard of read pairs (paired.cuh): the mate-1 sequences, then the mate-2 sequences at seq + off1[n_pairs].
+// Read 2i + m is mate m of pair i, so the reads are the mates interleaved by pair.
+struct ExpandPairs {
+    const uint8_t *seq;
+    const uint64_t *off1, *off2;  // n_pairs + 1 entries each, each relative to its own mates' first byte
+    uint64_t n_pairs;
+    __device__ __forceinline__ const uint8_t *at(uint64_t i, uint64_t *pos, uint64_t *len) const {
+        const uint64_t p = i >> 1, a1 = off1[p], l1 = off1[p + 1] - a1, a2 = off2[p];
+        *pos = a1 + a2 + ((i & 1) ? l1 : 0);
+        *len = (i & 1) ? off2[p + 1] - a2 : l1;
+        return (i & 1) ? seq + off1[n_pairs] + a2 : seq + a1;
+    }
+    __device__ __forceinline__ uint64_t total(uint64_t) const { return off1[n_pairs] + off2[n_pairs]; }
+};
+
+// Doubles n reads of a staged shard: out sequence 2i is read i, 2i+1 its reverse complement, at offsets 2 pos_i and
+// 2 pos_i + len_i (off2 gets 2n + 1 entries).  One warp per read; memory-bound.
+template <class Src>
+__global__ void __launch_bounds__(256) strand_expand_kernel(const Src src, uint64_t n, uint8_t *__restrict__ seq2,
+                                                            uint64_t *__restrict__ off2) {
     const uint64_t warps = (uint64_t)gridDim.x * (blockDim.x >> 5);
     const uint32_t lane = threadIdx.x & 31;
     for (uint64_t i = (uint64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); i < n; i += warps) {
-        const uint64_t a = off[i], len = off[i + 1] - a;
-        const uint8_t *src = seq + a;
+        uint64_t a, len;
+        const uint8_t *s = src.at(i, &a, &len);
         uint8_t *fwd = seq2 + 2 * a, *rev = fwd + len;
         for (uint64_t k = lane; k < len; k += 32) {
-            fwd[k] = src[k];
-            rev[k] = complement_base(src[len - 1 - k]);
+            fwd[k] = s[k];
+            rev[k] = complement_base(s[len - 1 - k]);
         }
         if (lane == 0) {
             off2[2 * i] = 2 * a;
             off2[2 * i + 1] = 2 * a + len;
-            if (i + 1 == n) off2[2 * n] = 2 * off[n];
+            if (i + 1 == n) off2[2 * n] = 2 * src.total(n);
         }
     }
 }

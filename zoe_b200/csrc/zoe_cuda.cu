@@ -35,6 +35,7 @@
 #include "sneaky_snake.cuh"
 #include "strands.cuh"
 #include "best_hit.cuh"
+#include "paired.cuh"
 
 using namespace zoe_cuda;
 
@@ -123,6 +124,8 @@ struct Device {
     // collects the buckets' CIGAR words
     DevBuf bh_seq, bh_off, bh_key, bh_tab, bh_list, bh_llen, bh_loff, bh_hit, bh_strand, bh_runner, bh_out32[5], bh_out8[3];
     DevBuf bh_cig_count, bh_cig_src, bh_acc, bh_cig_off, bh_cig;
+    // paired-end best-hit search (paired.cuh): the per-pair outputs (the per-mate ones are the bh_* buffers)
+    DevBuf pr_hit, pr_proper, pr_tlen;
     uint64_t n_first = 0, n_count = 0;  // shard of the streamed batch owned by this device
     uint64_t rseq_bytes = 0;
     bool timed_kernel = false;
@@ -721,6 +724,20 @@ __global__ void rebase_offsets_kernel(uint64_t *off, uint64_t n, uint64_t base) 
     if (i < n) off[i] -= base;
 }
 
+// Validates a batch's offsets and widens [*min_len, *max_len] and *tot by its sequences' lengths.
+int check_offsets(zoe_cuda_ctx *ctx, const uint64_t *offsets, uint64_t n, uint32_t *max_len, uint32_t *min_len,
+                  uint64_t *tot) {
+    for (uint64_t i = 0; i < n; ++i) {
+        if (offsets[i + 1] < offsets[i]) return fail(ctx, ZOE_CUDA_E_BAD_ARG, "offsets must be non-decreasing");
+        uint64_t len = offsets[i + 1] - offsets[i];
+        if (len > 0x7fffffffULL) return fail(ctx, ZOE_CUDA_E_BAD_ARG, "sequence too long");
+        *max_len = std::max<uint32_t>(*max_len, (uint32_t)len);
+        *min_len = std::min<uint32_t>(*min_len, (uint32_t)len);
+        *tot += len;
+    }
+    return 0;
+}
+
 // Validates a batch, records its global properties (count, longest / shortest sequence, cells) and shards it.
 int prepare_batch(zoe_cuda_ctx *ctx, const uint8_t *concat, const uint64_t *offsets, uint64_t n) {
     if (!ctx->have_profiled) return fail(ctx, ZOE_CUDA_E_STATE, "set_profiled must be called before a batch");
@@ -728,14 +745,8 @@ int prepare_batch(zoe_cuda_ctx *ctx, const uint8_t *concat, const uint64_t *offs
     if (n >= 0x7fffffffULL) return fail(ctx, ZOE_CUDA_E_BAD_ARG, "batch too large");
     uint32_t max_len = 0, min_len = n ? 0xffffffffu : 0u;
     uint64_t tot = 0;
-    for (uint64_t i = 0; i < n; ++i) {
-        if (offsets[i + 1] < offsets[i]) return fail(ctx, ZOE_CUDA_E_BAD_ARG, "offsets must be non-decreasing");
-        uint64_t len = offsets[i + 1] - offsets[i];
-        if (len > 0x7fffffffULL) return fail(ctx, ZOE_CUDA_E_BAD_ARG, "sequence too long");
-        max_len = std::max<uint32_t>(max_len, (uint32_t)len);
-        min_len = std::min<uint32_t>(min_len, (uint32_t)len);
-        tot += len;
-    }
+    int rc = check_offsets(ctx, offsets, n, &max_len, &min_len, &tot);
+    if (rc) return rc;
     ctx->staged_min_len = min_len;
     uint64_t prof_total = ctx->prof_off[ctx->n_prof];
     ctx->staged_n = n;
@@ -776,6 +787,7 @@ uint32_t first_part_tasks(const Device &d, uint32_t n_tasks, uint32_t total_grou
 // kernel instead of in front of it (config 3: 3.3 ms of a 70 ms call).  [An earlier version polled a "bytes arrived" word
 // inside the kernels: the extra control flow cost the two-stream score kernel 67 register moves per 76 cell pairs in its
 // steady loop, 292 -> 318 ms on config 2; measured and dropped.]
+int reserve_batch_outputs(zoe_cuda_ctx *ctx, Device &d);
 int stage_device(zoe_cuda_ctx *ctx, Device &d, const uint8_t *concat, const uint64_t *offsets, bool record_begin = true,
                  bool split = false) {
     CU(ctx, cudaSetDevice(d.id));
@@ -824,6 +836,11 @@ int stage_device(zoe_cuda_ctx *ctx, Device &d, const uint8_t *concat, const uint
     } else if (d.rseq_bytes) {
         CU(ctx, cudaMemcpyAsync(d.rseq.p, concat + b0, d.rseq_bytes, cudaMemcpyHostToDevice, d.stream));
     }
+    return reserve_batch_outputs(ctx, d);
+}
+
+// The score pass's per-pair buffers for the device's shard.
+int reserve_batch_outputs(zoe_cuda_ctx *ctx, Device &d) {
     size_t pairs = (size_t)d.n_count * ctx->n_prof;
     CU(ctx, d.best.reserve(pairs * sizeof(int32_t)));
     CU(ctx, d.score.reserve(pairs * sizeof(uint32_t)));
@@ -2867,15 +2884,22 @@ int check_both_strands_limits(zoe_cuda_ctx *ctx, uint64_t n, bool pair_limit) {
 }
 
 // Queues the strand expansion of the device's staged shard and swaps the doubled batch into rseq / roff.  The pair
-// buffers staging sized for the real shard are grown for the doubled one.
-int expand_strands(zoe_cuda_ctx *ctx, Device &d) {
+// buffers staging sized for the real shard are grown for the doubled one.  paired: the shard is a pair shard staged by
+// stage_pairs (its reads are the mates, interleaved by pair).
+int expand_strands(zoe_cuda_ctx *ctx, Device &d, bool paired = false) {
     if (d.n_count == 0) return 0;
     CU(ctx, cudaSetDevice(d.id));
     CU(ctx, d.xs_seq.reserve(2 * d.rseq_bytes + 16));
     CU(ctx, d.xs_off.reserve((2 * d.n_count + 1) * sizeof(uint64_t)));
     const uint32_t blocks = (uint32_t)std::min<uint64_t>((d.n_count + 7) / 8, (uint64_t)d.sm_count * 16);
-    strand_expand_kernel<<<blocks, 256, 0, d.stream>>>(d.rseq.as<uint8_t>(), d.roff.as<uint64_t>(), d.n_count,
-                                                       d.xs_seq.as<uint8_t>(), d.xs_off.as<uint64_t>());
+    if (paired) {
+        const uint64_t np = d.n_count / 2;
+        const ExpandPairs src{d.rseq.as<uint8_t>(), d.roff.as<uint64_t>(), d.roff.as<uint64_t>() + np + 1, np};
+        strand_expand_kernel<<<blocks, 256, 0, d.stream>>>(src, d.n_count, d.xs_seq.as<uint8_t>(), d.xs_off.as<uint64_t>());
+    } else {
+        const ExpandSingle src{d.rseq.as<uint8_t>(), d.roff.as<uint64_t>()};
+        strand_expand_kernel<<<blocks, 256, 0, d.stream>>>(src, d.n_count, d.xs_seq.as<uint8_t>(), d.xs_off.as<uint64_t>());
+    }
     CU(ctx, cudaGetLastError());
     ctx->last_launches++;
     std::swap(d.rseq, d.xs_seq);
@@ -2902,6 +2926,73 @@ int stage_both_strands(zoe_cuda_ctx *ctx, DoubledView &view, const uint8_t *conc
         rc = expand_strands(ctx, d);
         if (rc) return rc;
     }
+    view.enter();
+    return 0;
+}
+
+// Stages a paired batch: n pairs, mate 1 of pair i being sequence i of the first batch and mate 2 sequence i of the
+// second.  The host view is the 2n mates interleaved by pair (read 2i + m is mate m of pair i), sharded over pairs so
+// that no device splits a pair.  Each device gets its pair range of both batches with one upload per caller buffer
+// (the expansion reads the whole shard: no split upload), mate-1 bytes then mate-2 bytes in rseq and the two offset
+// arrays, each rebased to its own first byte, back to back in roff.  Then the strand expansion (ExpandPairs) and the
+// doubled view, as stage_both_strands: the devices hold the quadrupled batch, sequence 4i + 2m + s.
+int stage_pairs(zoe_cuda_ctx *ctx, DoubledView &view, const uint8_t *concat1, const uint64_t *offsets1,
+                const uint8_t *concat2, const uint64_t *offsets2, uint64_t n) {
+    if (!ctx->have_profiled) return fail(ctx, ZOE_CUDA_E_STATE, "set_profiled must be called before a batch");
+    if (n > 0 && (!concat1 || !offsets1 || !concat2 || !offsets2)) return fail(ctx, ZOE_CUDA_E_BAD_ARG, "null batch pointers");
+    int rc = check_both_strands_limits(ctx, 2 * std::min<uint64_t>(n, 0x7fffffffULL), false);
+    if (rc) return rc;
+    uint32_t max_len = 0, min_len = n ? 0xffffffffu : 0u;
+    uint64_t tot = 0;
+    rc = check_offsets(ctx, offsets1, n, &max_len, &min_len, &tot);
+    if (rc) return rc;
+    rc = check_offsets(ctx, offsets2, n, &max_len, &min_len, &tot);
+    if (rc) return rc;
+    ctx->staged_n = 2 * n;
+    ctx->staged_max_len = max_len;
+    ctx->staged_min_len = min_len;
+    ctx->staged_cells = tot * ctx->prof_off[ctx->n_prof];
+    ctx->staged_len.clear();
+    if (max_len > (uint32_t)kMaxRowsSinglePass) {
+        ctx->staged_len.resize(2 * n);
+        for (uint64_t i = 0; i < n; ++i) {
+            ctx->staged_len[2 * i] = (uint32_t)(offsets1[i + 1] - offsets1[i]);
+            ctx->staged_len[2 * i + 1] = (uint32_t)(offsets2[i + 1] - offsets2[i]);
+        }
+    }
+    ctx->alt_used = false;
+    shard(ctx, n);
+    for (Device &d : ctx->devs) {
+        const uint64_t a = d.n_first, np = d.n_count;
+        d.n_first = 2 * a;
+        d.n_count = 2 * np;
+        CU(ctx, cudaSetDevice(d.id));
+        CU(ctx, cudaEventRecord(d.ev_begin, d.stream));
+        d.copy_pending = false;
+        if (np == 0) continue;
+        const uint64_t a1 = offsets1[a], b1 = offsets1[a + np], a2 = offsets2[a], b2 = offsets2[a + np];
+        d.rseq_bytes = (b1 - a1) + (b2 - a2);
+        CU(ctx, d.rseq.reserve(d.rseq_bytes + 16));
+        CU(ctx, d.roff.reserve(2 * (np + 1) * sizeof(uint64_t)));
+        uint64_t *off = d.roff.as<uint64_t>();
+        CU(ctx, cudaMemcpyAsync(off, offsets1 + a, (np + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, d.stream));
+        CU(ctx, cudaMemcpyAsync(off + np + 1, offsets2 + a, (np + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, d.stream));
+        if (b1 > a1) CU(ctx, cudaMemcpyAsync(d.rseq.p, concat1 + a1, b1 - a1, cudaMemcpyHostToDevice, d.stream));
+        if (b2 > a2)
+            CU(ctx, cudaMemcpyAsync(d.rseq.as<uint8_t>() + (b1 - a1), concat2 + a2, b2 - a2, cudaMemcpyHostToDevice, d.stream));
+        const uint32_t blocks = (uint32_t)((np + 256) / 256);
+        for (int m = 0; m < 2; ++m) {
+            const uint64_t b0 = m == 0 ? a1 : a2;
+            if (b0 == 0) continue;
+            rebase_offsets_kernel<<<blocks, 256, 0, d.stream>>>(off + m * (np + 1), np + 1, b0);
+            CU(ctx, cudaGetLastError());
+        }
+        rc = reserve_batch_outputs(ctx, d);
+        if (rc) return rc;
+        rc = expand_strands(ctx, d, /*paired=*/true);
+        if (rc) return rc;
+    }
+    ctx->staged = true;
     view.enter();
     return 0;
 }
@@ -3294,6 +3385,65 @@ int select_best_hits(zoe_cuda_ctx *ctx, Device &d, uint32_t n_strands) {
     return 0;
 }
 
+// Pair selection on one device (paired search, real view: the device's reads are the mates of its pairs): the winner
+// of every pair to pr_hit and each mate's result under it to the per-read buffers select_best_hits fills.
+int select_pairs(zoe_cuda_ctx *ctx, Device &d) {
+    const uint64_t n = d.n_count, np = n / 2;
+    if (n == 0) return 0;
+    CU(ctx, cudaSetDevice(d.id));
+    for (DevBuf *b : {&d.bh_hit, &d.bh_runner, &d.bh_out32[0]}) CU(ctx, b->reserve(n * sizeof(uint32_t)));
+    for (DevBuf *b : {&d.bh_strand, &d.bh_out8[0], &d.bh_out8[1]}) CU(ctx, b->reserve(n));
+    CU(ctx, d.pr_hit.reserve(np * sizeof(uint32_t)));
+    PairSelectParams p{};
+    p.score = d.score.as<uint32_t>();
+    p.status = d.status.as<uint8_t>();
+    p.tier = d.tier.as<uint8_t>();
+    p.n_pairs = np;
+    p.n_prof = ctx->n_prof;
+    p.pair_hit = d.pr_hit.as<uint32_t>();
+    p.hit = d.bh_hit.as<uint32_t>();
+    p.score_out = d.bh_out32[0].as<uint32_t>();
+    p.runner_up = d.bh_runner.as<uint32_t>();
+    p.strand = d.bh_strand.as<uint8_t>();
+    p.status_out = d.bh_out8[0].as<uint8_t>();
+    p.tier_out = d.bh_out8[1].as<uint8_t>();
+    // a thread per pair while a pair's 2 n_prof candidates fit one warp's width, a warp per pair beyond
+    if ((uint64_t)ctx->n_prof * 2 <= 32) {
+        const uint32_t blocks = (uint32_t)std::min<uint64_t>((np + 255) / 256, (uint64_t)d.sm_count * 8);
+        pair_select_kernel<1><<<blocks, 256, 0, d.stream>>>(p);
+    } else {
+        const uint32_t blocks = (uint32_t)std::min<uint64_t>((np + 7) / 8, (uint64_t)d.sm_count * 16);
+        pair_select_kernel<32><<<blocks, 256, 0, d.stream>>>(p);
+    }
+    CU(ctx, cudaGetLastError());
+    ctx->last_launches++;
+    return 0;
+}
+
+// tlen and proper of one device's pairs from its per-mate outputs (in mate order).
+int finalize_pairs(zoe_cuda_ctx *ctx, Device &d, uint32_t min_insert, uint32_t max_insert) {
+    const uint64_t np = d.n_count / 2;
+    if (np == 0) return 0;
+    CU(ctx, cudaSetDevice(d.id));
+    CU(ctx, d.pr_proper.reserve(np));
+    CU(ctx, d.pr_tlen.reserve(np * sizeof(int32_t)));
+    PairFinalizeParams p{};
+    p.status = d.bh_out8[0].as<uint8_t>();
+    p.strand = d.bh_strand.as<uint8_t>();
+    p.start = d.bh_out32[ctx->profiled_is_query ? 3 : 1].as<uint32_t>();
+    p.end = d.bh_out32[ctx->profiled_is_query ? 4 : 2].as<uint32_t>();
+    p.n_pairs = np;
+    p.min_insert = min_insert;
+    p.max_insert = max_insert;
+    p.proper = d.pr_proper.as<uint8_t>();
+    p.tlen = d.pr_tlen.as<int32_t>();
+    const uint32_t blocks = (uint32_t)std::min<uint64_t>((np + 255) / 256, (uint64_t)d.sm_count * 8);
+    pair_finalize_kernel<<<blocks, 256, 0, d.stream>>>(p);
+    CU(ctx, cudaGetLastError());
+    ctx->last_launches++;
+    return 0;
+}
+
 // Buckets one device's Some winners (best_hit_bucket_*_kernel), zeroes the outputs of the reads no bucket aligns, and
 // reads the bucket table back into tab (kBhStart + 1 rows of n_keys words).
 int bucket_best_hits(zoe_cuda_ctx *ctx, Device &d, uint32_t n_strands, bool split_long, uint32_t n_keys,
@@ -3414,16 +3564,31 @@ int align_bucket(zoe_cuda_ctx *ctx, Device &d, bool three_pass, uint32_t n_stran
     return 0;
 }
 
-// The best-hit entry points.  align = false: score pass + selection only.
+// What the paired entry points add to the best-hit search: the mate-2 batch, the insert bounds and the per-pair
+// outputs (hit then has one entry per pair).
+struct PairedArgs {
+    const uint8_t *concat2;
+    const uint64_t *offsets2;
+    uint32_t min_insert, max_insert;
+    uint8_t *proper;
+    int32_t *tlen;
+};
+
+// The best-hit entry points.  align = false: score pass + selection only.  pair: the paired search, n pairs (concat /
+// offsets are mate 1); it runs on both strands, selects per pair and finishes with the pair outputs.
 int best_hit(zoe_cuda_ctx *ctx, bool align, bool both_strands, bool three_pass, const uint8_t *concat,
-             const uint64_t *offsets, uint64_t n, uint32_t *hit, uint8_t *strand, uint32_t *score, uint8_t *status,
-             uint8_t *tier, uint32_t *runner_up, uint32_t *ref_start, uint32_t *ref_end, uint32_t *query_start,
-             uint32_t *query_end, uint32_t *cigar, uint64_t *cigar_off, uint64_t cigar_cap, uint8_t *hazard) {
+             const uint64_t *offsets, uint64_t n, const PairedArgs *pair, uint32_t *hit, uint8_t *strand,
+             uint32_t *score, uint8_t *status, uint8_t *tier, uint32_t *runner_up, uint32_t *ref_start,
+             uint32_t *ref_end, uint32_t *query_start, uint32_t *query_end, uint32_t *cigar, uint64_t *cigar_off,
+             uint64_t cigar_cap, uint8_t *hazard) {
     if (align && (!cigar_off || (!cigar && cigar_cap))) return fail(ctx, ZOE_CUDA_E_BAD_ARG, "null CIGAR outputs");
+    if (pair && pair->min_insert > pair->max_insert)
+        return fail(ctx, ZOE_CUDA_E_BAD_ARG, "min_insert (%u) > max_insert (%u)", pair->min_insert, pair->max_insert);
     begin_call(ctx);
     DoubledView view(ctx);  // (entered only with both strands; drains every stream on an error return)
-    int rc = both_strands ? stage_both_strands(ctx, view, concat, offsets, n, /*pair_limit=*/false)
-                          : stage_on_devices(ctx, concat, offsets, n, /*split=*/false);
+    int rc = pair           ? stage_pairs(ctx, view, concat, offsets, pair->concat2, pair->offsets2, n)
+             : both_strands ? stage_both_strands(ctx, view, concat, offsets, n, /*pair_limit=*/false)
+                            : stage_on_devices(ctx, concat, offsets, n, /*split=*/false);
     if (rc) return rc;
     for (Device &d : ctx->devs) {
         rc = run_score_on_device(ctx, d);
@@ -3440,9 +3605,9 @@ int best_hit(zoe_cuda_ctx *ctx, bool align, bool both_strands, bool three_pass, 
         if (rc) return rc;
     }
     view.leave();
-    const uint32_t S = both_strands ? 2 : 1;
+    const uint32_t S = both_strands || pair ? 2 : 1;
     for (Device &d : ctx->devs) {
-        rc = select_best_hits(ctx, d, S);
+        rc = pair ? select_pairs(ctx, d) : select_best_hits(ctx, d, S);
         if (rc) return rc;
     }
     const size_t nd = ctx->devs.size();
@@ -3462,6 +3627,8 @@ int best_hit(zoe_cuda_ctx *ctx, bool align, bool both_strands, bool three_pass, 
             std::swap(d.roff, d.bh_off);
         }
         const uint64_t real_n = ctx->staged_n;
+        std::vector<uint32_t> read_len;  // per read when a read is long (prepare_batch, stage_pairs)
+        read_len.swap(ctx->staged_len);
         uint64_t aligned = 0, aligned_cells = 0;
         {
             ProfiledView pv(ctx);
@@ -3493,16 +3660,13 @@ int best_hit(zoe_cuda_ctx *ctx, bool align, bool both_strands, bool three_pass, 
                     d.rseq_bytes = at(k, kBhSum);
                     d.copy_pending = false;
                     if (!ctx->staged_len.empty() && d.n_count) {
-                        // the long-row path orders its tasks by length: a long bucket's lengths come from the caller's
-                        // offsets (such reads are few)
+                        // the long-row path orders its tasks by length: a long bucket's lengths come from the batch's
+                        // per-read lengths (such reads are few)
                         std::vector<uint32_t> ids(d.n_count);
                         CU(ctx, cudaSetDevice(d.id));
                         CU(ctx, cudaMemcpy(ids.data(), d.bh_list.as<uint32_t>() + at(k, kBhStart), d.n_count * sizeof(uint32_t),
                                            cudaMemcpyDeviceToHost));
-                        for (uint64_t t = 0; t < d.n_count; ++t) {
-                            const uint64_t i = first[k] + ids[t];
-                            ctx->staged_len[pos + t] = (uint32_t)(offsets[i + 1] - offsets[i]);
-                        }
+                        for (uint64_t t = 0; t < d.n_count; ++t) ctx->staged_len[pos + t] = read_len[first[k] + ids[t]];
                     }
                     pos += d.n_count;
                 }
@@ -3551,6 +3715,11 @@ int best_hit(zoe_cuda_ctx *ctx, bool align, bool both_strands, bool three_pass, 
         }
         ctx->stats.pairs += aligned;
         ctx->stats.cells += aligned_cells;
+        if (pair)
+            for (Device &d : ctx->devs) {
+                rc = finalize_pairs(ctx, d, pair->min_insert, pair->max_insert);
+                if (rc) return rc;
+            }
     }
     // per-read outputs (and the CIGAR stream) to the caller
     uint64_t cig_base = 0;
@@ -3563,7 +3732,20 @@ int best_hit(zoe_cuda_ctx *ctx, bool align, bool both_strands, bool three_pass, 
             if (!dst) return cudaSuccess;
             return cudaMemcpyAsync((uint8_t *)dst + first * elem, src.p, cnt * elem, cudaMemcpyDeviceToHost, d.stream);
         };
-        CU(ctx, d2h(hit, d.bh_hit, 4));
+        if (pair) {  // per-pair outputs: the device's pairs are its mates halved
+            auto pair_d2h = [&](void *dst, const DevBuf &src, size_t elem) -> cudaError_t {
+                if (!dst) return cudaSuccess;
+                return cudaMemcpyAsync((uint8_t *)dst + first / 2 * elem, src.p, cnt / 2 * elem, cudaMemcpyDeviceToHost,
+                                       d.stream);
+            };
+            CU(ctx, pair_d2h(hit, d.pr_hit, 4));
+            if (align) {
+                CU(ctx, pair_d2h(pair->proper, d.pr_proper, 1));
+                CU(ctx, pair_d2h(pair->tlen, d.pr_tlen, 4));
+            }
+        } else {
+            CU(ctx, d2h(hit, d.bh_hit, 4));
+        }
         CU(ctx, d2h(strand, d.bh_strand, 1));
         CU(ctx, d2h(score, d.bh_out32[0], 4));
         CU(ctx, d2h(status, d.bh_out8[0], 1));
@@ -4086,7 +4268,7 @@ int zoe_cuda_sw_score_best_hit_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_
                                      uint64_t n, int both_strands, uint32_t *hit, uint8_t *strand, uint32_t *score,
                                      uint8_t *status, uint8_t *tier, uint32_t *runner_up) {
     if (!ctx) return ZOE_CUDA_E_BAD_ARG;
-    return best_hit(ctx, false, both_strands != 0, false, streamed_concat, offsets, n, hit, strand, score, status, tier,
+    return best_hit(ctx, false, both_strands != 0, false, streamed_concat, offsets, n, nullptr, hit, strand, score, status, tier,
                     runner_up, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 0, nullptr);
 }
 
@@ -4096,8 +4278,31 @@ int zoe_cuda_sw_align_best_hit_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_
                                      uint32_t *ref_start, uint32_t *ref_end, uint32_t *query_start, uint32_t *query_end,
                                      uint32_t *cigar, uint64_t *cigar_off, uint64_t cigar_cap, uint8_t *hazard) {
     if (!ctx) return ZOE_CUDA_E_BAD_ARG;
-    return best_hit(ctx, true, both_strands != 0, three_pass != 0, streamed_concat, offsets, n, hit, strand, score, status,
+    return best_hit(ctx, true, both_strands != 0, three_pass != 0, streamed_concat, offsets, n, nullptr, hit, strand, score, status,
                     tier, runner_up, ref_start, ref_end, query_start, query_end, cigar, cigar_off, cigar_cap, hazard);
+}
+
+int zoe_cuda_sw_score_paired_best_hit_batch(zoe_cuda_ctx *ctx, const uint8_t *mate1_concat, const uint64_t *mate1_offsets,
+                                            const uint8_t *mate2_concat, const uint64_t *mate2_offsets, uint64_t n_pairs,
+                                            uint32_t *hit, uint8_t *strand, uint32_t *score, uint8_t *status, uint8_t *tier,
+                                            uint32_t *runner_up) {
+    if (!ctx) return ZOE_CUDA_E_BAD_ARG;
+    const PairedArgs pair{mate2_concat, mate2_offsets, 0, ~0u, nullptr, nullptr};
+    return best_hit(ctx, false, true, false, mate1_concat, mate1_offsets, n_pairs, &pair, hit, strand, score, status, tier,
+                    runner_up, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 0, nullptr);
+}
+
+int zoe_cuda_sw_align_paired_best_hit_batch(zoe_cuda_ctx *ctx, const uint8_t *mate1_concat, const uint64_t *mate1_offsets,
+                                            const uint8_t *mate2_concat, const uint64_t *mate2_offsets, uint64_t n_pairs,
+                                            int three_pass, uint32_t min_insert, uint32_t max_insert, uint32_t *hit,
+                                            uint8_t *proper, int *tlen, uint8_t *strand, uint32_t *score, uint8_t *status,
+                                            uint8_t *tier, uint32_t *runner_up, uint32_t *ref_start, uint32_t *ref_end,
+                                            uint32_t *query_start, uint32_t *query_end, uint32_t *cigar, uint64_t *cigar_off,
+                                            uint64_t cigar_cap, uint8_t *hazard) {
+    if (!ctx) return ZOE_CUDA_E_BAD_ARG;
+    const PairedArgs pair{mate2_concat, mate2_offsets, min_insert, max_insert, proper, tlen};
+    return best_hit(ctx, true, true, three_pass != 0, mate1_concat, mate1_offsets, n_pairs, &pair, hit, strand, score,
+                    status, tier, runner_up, ref_start, ref_end, query_start, query_end, cigar, cigar_off, cigar_cap, hazard);
 }
 
 int zoe_cuda_sneaky_snake_batch(zoe_cuda_ctx *ctx, const uint8_t *refs, const uint64_t *ref_offsets, const uint8_t *queries,

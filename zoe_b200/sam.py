@@ -9,6 +9,9 @@ Mirrors (paths relative to the zoe repository):
 Results of the best-hit search (``CudaProfiles.align_best_hit_arrays``) become one primary record per read:
 ``sam_lines_best_hit``.
 
+Results of the paired-end best-hit search (``CudaProfiles.align_paired_best_hit_arrays``) become two records per read
+pair, mate 1 first, with the paired FLAG bits, RNEXT, PNEXT and TLEN: ``sam_lines_paired``.
+
 Results of the both-strand search pass their strands as ``strand``: a reverse-strand pair is written as SAM writes a read
 that maps to the reverse strand -- FLAG bit 16 set, SEQ reverse-complemented, QUAL reversed (its POS and CIGAR already
 refer to the reverse complement).
@@ -132,3 +135,50 @@ def sam_lines_best_hit(a: dict, qnames: Sequence[str], rnames: Sequence[str], bu
             tags.append(f"XS:i:{int(a['runner_up'][i])}")
         yield str(SamData(qnames[i], f, rnames[int(a["hit"][i])], int(a["ref_start"][i]) + 1, mapq, cigar, s, q,
                           opt_fields=tags))
+
+
+def sam_lines_paired(a: dict, qnames: Sequence[str], rnames: Sequence[str], buf1: np.ndarray, offs1: np.ndarray,
+                     buf2: np.ndarray, offs2: np.ndarray, quals1: Optional[Sequence[bytes]] = None,
+                     quals2: Optional[Sequence[bytes]] = None, mapq: int = 255) -> Iterable[str]:
+    """Two SAM lines per read pair from ``CudaProfiles.align_paired_best_hit_arrays``, mate 1 then mate 2.
+
+    FLAG: 0x1 always, 0x2 for a proper pair, 0x4 / 0x8 when the record's own / its mate's result is not Some, 0x10 /
+    0x20 for its own / its mate's reverse strand when mapped, 0x40 for mate 1, 0x80 for mate 2.  A mapped mate is written
+    as :func:`sam_lines_best_hit` writes a read (RNAME ``rnames[hit]``, POS, CIGAR, oriented SEQ and QUAL, ``AS`` and
+    ``XS``), with RNEXT ``=`` and PNEXT at its mate's POS, and TLEN ``tlen`` for mate 1, ``-tlen`` for mate 2.  An
+    unmapped mate of a mapped one takes its mate's RNAME and POS (the SAM recommended practice), so both records'
+    PNEXT point there; it keeps its SEQ and QUAL as given.  A pair with no mapped mate gets RNAME ``*`` and POS 0
+    (FLAG 77 and 141)."""
+    cig, coff = a["cigar"], a["cigar_off"]
+    bufs, offs, quals = (buf1, buf2), (offs1, offs2), (quals1, quals2)
+    for i in range(len(offs1) - 1):
+        k = (2 * i, 2 * i + 1)
+        mapped = [int(a["status"][x]) == _lib.SOME for x in k]
+        rev = [int(a["strand"][x]) == 1 for x in k]
+        pos = [int(a["ref_start"][x]) + 1 if mapped[m] else 0 for m, x in enumerate(k)]
+        if mapped[0] != mapped[1]:  # the unmapped mate is placed at its mate
+            pos = [max(pos)] * 2
+        rname = rnames[int(a["hit"][i])] if any(mapped) else "*"
+        for m in range(2):
+            o = 1 - m
+            flag = 0x1 | (0x40 if m == 0 else 0x80)
+            flag |= 0x2 if int(a["proper"][i]) else 0
+            flag |= 0 if mapped[m] else 0x4
+            flag |= 0 if mapped[o] else 0x8
+            flag |= 0x10 if mapped[m] and rev[m] else 0
+            flag |= 0x20 if mapped[o] and rev[o] else 0
+            seq = bytes(bufs[m][int(offs[m][i]):int(offs[m][i + 1])])
+            qual = bytes(quals[m][i]) if quals[m] is not None else b"*"
+            rnext, pnext = ("=", pos[o]) if any(mapped) else ("*", 0)
+            if not mapped[m]:
+                yield str(SamData(qnames[i], flag, rname, pos[m], mapq, "", seq or b"*", qual or b"*", rnext, pnext, 0))
+                continue
+            x = k[m]
+            words = cig[int(coff[x]):int(coff[x + 1])]
+            cigar = "".join(f"{int(w) >> 4}{_OPS[int(w) & 15]}" for w in words)
+            _, s, q = _oriented(rev[m], 0, seq, qual)
+            tags = [f"AS:i:{int(a['score'][x])}"]
+            if int(a["runner_up"][x]) > 0:
+                tags.append(f"XS:i:{int(a['runner_up'][x])}")
+            tlen = int(a["tlen"][i]) if m == 0 else -int(a["tlen"][i])
+            yield str(SamData(qnames[i], flag, rname, pos[m], mapq, cigar, s, q, rnext, pnext, tlen, opt_fields=tags))

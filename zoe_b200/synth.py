@@ -54,6 +54,27 @@ def _mutate(rng, frag, sub, ins, dele, alphabet):
     return out
 
 
+def _read_errors(rng, frag, read_len, sub, indel):
+    """The read error model: an indel in ~``2*indel*read_len`` of the reads, then substitutions.  ``frag`` is
+    ``[n, span]`` with some slack past ``read_len`` so that deletions still leave ``read_len`` bases; returns
+    ``[n, read_len]``."""
+    span = frag.shape[1]
+    has_indel = rng.random(len(frag)) < (2 * indel * read_len)
+    for k in np.nonzero(has_indel)[0]:
+        f = frag[k]
+        pos = int(rng.integers(10, read_len - 10))
+        ln = int(rng.geometric(0.5))
+        if rng.random() < 0.5:
+            f2 = np.concatenate([f[:pos], random_dna(rng, ln), f[pos:]])[:span]
+        else:
+            f2 = np.concatenate([f[:pos], f[pos + ln:], random_dna(rng, ln)])[:span]
+        frag[k] = f2
+    frag = frag[:, :read_len].copy()
+    subs = rng.random(frag.shape) < sub
+    frag[subs] = _ACGT[rng.integers(0, 4, int(subs.sum()))]
+    return frag
+
+
 def illumina_reads(rng: np.random.Generator, targets, n_reads: int, read_len: int = 150, sub: float = 0.01,
                    indel: float = 0.001, random_frac: float = 0.05):
     """Fixed-length reads drawn from uniformly chosen targets, both strands, with a few errors.
@@ -71,27 +92,49 @@ def illumina_reads(rng: np.random.Generator, targets, n_reads: int, read_len: in
             continue
         tt = np.concatenate([t, random_dna(rng, span)])  # reads may run off the 3' end into noise
         start = rng.integers(0, max(1, lens[ti] - read_len + 1), idx.size)
-        frag = tt[start[:, None] + np.arange(span)[None, :]]
-        # indels on a subset
-        has_indel = rng.random(idx.size) < (2 * indel * read_len)
-        for k in np.nonzero(has_indel)[0]:
-            f = frag[k]
-            pos = int(rng.integers(10, read_len - 10))
-            ln = int(rng.geometric(0.5))
-            if rng.random() < 0.5:
-                f2 = np.concatenate([f[:pos], random_dna(rng, ln), f[pos:]])[:span]
-            else:
-                f2 = np.concatenate([f[:pos], f[pos + ln:], random_dna(rng, ln)])[:span]
-            frag[k] = f2
-        frag = frag[:, :read_len].copy()
-        subs = rng.random(frag.shape) < sub
-        frag[subs] = _ACGT[rng.integers(0, 4, int(subs.sum()))]
+        frag = _read_errors(rng, tt[start[:, None] + np.arange(span)[None, :]], read_len, sub, indel)
         rc = rng.random(idx.size) < 0.5
         frag[rc] = _COMP[frag[rc][:, ::-1]]
         reads[idx] = frag
     rnd = rng.random(n_reads) < random_frac
     reads[rnd] = _ACGT[rng.integers(0, 4, (int(rnd.sum()), read_len))]
     return reads
+
+
+def paired_reads(rng: np.random.Generator, targets, n_pairs: int, read_len: int = 150, insert_mean: float = 350.0,
+                 insert_sd: float = 50.0, sub: float = 0.01, indel: float = 0.001, random_frac: float = 0.05):
+    """Illumina-like FR read pairs.  Each pair's fragment comes from a uniformly chosen target, on a random strand, with
+    an insert length drawn from a normal distribution (at least ``read_len``, at most the target).  Mate 1 is the
+    fragment's first ``read_len`` bases, mate 2 the reverse complement of its last ``read_len`` bases; each mate then
+    gets the error model of :func:`illumina_reads`, and a ``random_frac`` of the mates are replaced by random reads.
+
+    Returns ``(mates1, mates2, truth)``: two ``[n_pairs, read_len]`` uint8 arrays and a dict of per-pair arrays,
+    ``target``, ``start`` (the fragment's first target position), ``insert`` and ``strand`` (1: the fragment is the
+    reverse complement of ``target[start:start + insert]``)."""
+    lens = np.array([len(t) for t in targets])
+    which = rng.integers(0, len(targets), n_pairs)
+    strand = rng.integers(0, 2, n_pairs).astype(np.uint8)
+    insert = np.minimum(np.maximum(np.rint(rng.normal(insert_mean, insert_sd, n_pairs)), read_len).astype(np.int64),
+                        lens[which])
+    start = (rng.random(n_pairs) * (lens[which] - insert + 1)).astype(np.int64)
+    mates = [np.empty((n_pairs, read_len), dtype=np.uint8) for _ in range(2)]
+    span = read_len + 8
+    for ti, t in enumerate(targets):
+        idx = np.nonzero(which == ti)[0]
+        if idx.size == 0:
+            continue
+        tt = np.concatenate([random_dna(rng, span), t, random_dna(rng, span)])  # reads may run off either end
+        s, e = start[idx] + span, start[idx] + insert[idx] + span
+        fwd = tt[s[:, None] + np.arange(span)[None, :]]            # the target's strand, read from the fragment start
+        rev = _COMP[tt[(e - 1)[:, None] - np.arange(span)[None, :]]]  # the other strand, read from the fragment end
+        rc = strand[idx] == 1
+        first, second = np.where(rc[:, None], rev, fwd), np.where(rc[:, None], fwd, rev)
+        mates[0][idx] = _read_errors(rng, first, read_len, sub, indel)
+        mates[1][idx] = _read_errors(rng, second, read_len, sub, indel)
+    for m in mates:
+        rnd = rng.random(n_pairs) < random_frac
+        m[rnd] = _ACGT[rng.integers(0, 4, (int(rnd.sum()), read_len))]
+    return mates[0], mates[1], {"target": which, "start": start, "insert": insert, "strand": strand}
 
 
 def fixed_len_batch(reads2d: np.ndarray):
