@@ -20,7 +20,57 @@ def osc(wm, go, ge):
     return O.Scoring(wm.weights, wm.mapping.index_map, go, ge)
 
 
+# ---- pass 3 routing, restated from sw_3pass.cuh and run_3pass_on_device (test_3pass_band_edges_gpu.py pins the constants) ----
+TP_RING = 32                 # kTpRing: (H, E) entries a banded attempt keeps in shared memory
+TP_BOX_CELLS = 65536         # scalar boxes above this many cells are "large"
+TP_WCAP_CAP = 24 * 1024      # row cells + 2 the warp kernel can hold at most (two int rows per warp in shared memory)
+
+
+def tp_ring_size(bw):
+    r = TP_RING
+    while r < 2 * bw + 2:
+        r *= 2
+    return r
+
+
+def tp_is_large(bw, rn, qn):
+    return tp_ring_size(bw) > TP_RING if bw else rn * qn > TP_BOX_CELLS
+
+
+def tp_row_cells(bw, qn):
+    return 2 * bw + 2 if bw else qn
+
+
+def tp_kernel(bw, rn, qn, thread_only=False):
+    """Which kernel runs an attempt at width `bw` (0: the scalar box): "warp" (tp_band_warp_kernel), "shared" (tp_dp_kernel,
+    banded, ring in shared memory), "global" (tp_dp_kernel, banded, ring in the pair's scratch) or "thread" (tp_dp_kernel,
+    scalar).  Every round's warp capacity covers the widest large row up to the cap, so the rule is per pair."""
+    if not thread_only and tp_is_large(bw, rn, qn) and tp_row_cells(bw, qn) + 2 <= TP_WCAP_CAP:
+        return "warp"
+    if bw == 0:
+        return "thread"
+    return "shared" if tp_ring_size(bw) <= TP_RING else "global"
+
+
+def tp_attempts(rn, qn, path):
+    """Widths pass 3 tries on a DP pair, in order (0 = the scalar box), from the oracle's box and path (1 | accepted
+    width << 8 banded, 2 scalar fallback): |rn - qn| + 1, doubled while it stays <= (qn - 1) / 2 (three_pass.rs:66-84)."""
+    assert path & 0xff in (1, 2), path
+    max_bw = (qn - 1) // 2
+    bw = abs(rn - qn) + 1
+    out = []
+    while 0 < bw <= max_bw:
+        out.append(bw)
+        if path & 0xff == 1 and bw == path >> 8:
+            return out
+        bw *= 2
+    assert path == 2, (rn, qn, path, out)  # an accepted width the doubling never tries
+    return out + [0]
+
+
 def check_3pass(targets, seqs, wm, go=-10, ge=-1, profiled_is_query=False, lanes=(32, 16, 8), policy=None):
+    """Every pair against the oracle; last_stats() against the oracle's paths, band attempts included.  Returns the stats
+    and, per DP pair, (i, j, rn, qn, path) with the box of passes 1-2 (rows streamed, columns profiled)."""
     targets = [bytes(t) for t in targets]
     seqs = [bytes(s) for s in seqs]
     prof = CudaProfiles(targets, wm, go, ge, lanes=lanes, profiled_is_query=profiled_is_query)
@@ -31,9 +81,12 @@ def check_3pass(targets, seqs, wm, go=-10, ge=-1, profiled_is_query=False, lanes
     stats = prof.last_stats()
     sc = osc(wm, go, ge)
     paths = {0: 0, 1: 0, 2: 0}
+    attempts = 0
+    dp = []
     for i, s in enumerate(seqs):
         for j, t in enumerate(targets):
-            if policy and policy[0] == policy[1]:  # a standalone StripedProfile<T, N, S>
+            standalone = policy and policy[0] == policy[1]  # a standalone StripedProfile<T, N, S>
+            if standalone:
                 rc, aln, path = O.striped_align_3pass(t, s, sc, policy[0], lanes[0], signed=not policy[2],
                                                       streamed_is_query=not profiled_is_query)
             else:
@@ -46,9 +99,20 @@ def check_3pass(targets, seqs, wm, go=-10, ge=-1, profiled_is_query=False, lanes
                 assert (a.score, a.ref_range, a.query_range, a.states, a.ref_len, a.query_len) == \
                        (aln.score, aln.ref_range, aln.query_range, aln.cigar, aln.ref_len, aln.query_len), (i, j, a, aln, path)
                 paths[path & 0xff] += 1
-    assert (stats["tp_nogaps"], stats["tp_banded"], stats["tp_scalar"]) == (paths[0], paths[1], paths[2]), (stats, paths)
+                if path & 0xff:
+                    # the box pass 3 ran on: the ranges of passes 1-2, un-inverted
+                    if standalone:
+                        _, _, rr, qr = O.striped_score_ranges(t, s, sc, policy[0], lanes[0], signed=not policy[2])
+                    else:
+                        _, _, rr, qr, _ = O.sw_score_ranges_from(t, s, sc, lanes=lanes,
+                                                                 first_bits=policy[0] if policy else 8)
+                    rn, qn = rr[1] - rr[0], qr[1] - qr[0]
+                    attempts += sum(1 for bw in tp_attempts(rn, qn, path) if bw)
+                    dp.append((i, j, rn, qn, path))
+    assert (stats["tp_nogaps"], stats["tp_banded"], stats["tp_scalar"], stats["tp_band_attempts"]) == \
+           (paths[0], paths[1], paths[2], attempts), (stats, paths, attempts)
     prof.close()
-    return stats
+    return stats, dp
 
 
 def test_doc_example():
@@ -65,7 +129,7 @@ def test_doc_example():
 
 def test_config3_sample():
     targets, reads = synth.config3(ROOT, n_reads=400, seed=92)
-    stats = check_3pass(targets, list(reads), W25)
+    stats, _ = check_3pass(targets, list(reads), W25)
     assert stats["tp_nogaps"] > 100 and stats["tp_banded"] > 5
 
 
@@ -89,8 +153,8 @@ def test_random_pairs_many_scorings_both_orientations():
                 s[2:2 + k2] = frag[:k2]
             seqs.append(s)
         seqs.append(np.zeros(0, dtype=np.uint8))
-        for st in (check_3pass(targets, seqs, wm, go, ge),
-                   check_3pass(targets[:2], seqs[:30], wm, go, ge, profiled_is_query=True, lanes=(16, 8, 4))):
+        for st, _ in (check_3pass(targets, seqs, wm, go, ge),
+                      check_3pass(targets[:2], seqs[:30], wm, go, ge, profiled_is_query=True, lanes=(16, 8, 4))):
             for k in tot:
                 tot[k] += st[k]
     assert all(v > 0 for v in tot.values()), tot
@@ -103,7 +167,7 @@ def test_long_gaps_force_band_doubling_and_scalar_fallback():
     seqs = [np.concatenate([t[20:80], t[120:180]]), np.concatenate([t[200:260], synth.random_dna(rng, 25), t[260:330]]),
             np.concatenate([t[10:60], t[64:110], t[118:170]]), t[5:8].copy(), t[300:302].copy(),
             np.concatenate([t[40:70], synth.random_dna(rng, 3), t[70:100], t[103:140]])]
-    stats = check_3pass([t], seqs, W42, -3, -1)
+    stats, _ = check_3pass([t], seqs, W42, -3, -1)
     assert stats["tp_band_attempts"] >= stats["tp_banded"]
     check_3pass([t], seqs, W42, -3, -1, profiled_is_query=True)
     check_3pass([t], seqs, W25)
@@ -130,7 +194,7 @@ def test_protein_and_width_policies():
     check_3pass(t, seqs, W25, policy=(8, 8, True), lanes=(16, 16, 16), profiled_is_query=True)
     check_3pass(t, seqs, W25, policy=(16, 16, True), lanes=(16, 16, 16))
     w = WeightMatrix.new(DNA_PROFILE_MAP, 127, -5, b"N")
-    stats = check_3pass([b"A" * 600], [b"A" * 600, b"A" * 300, b"A" * 100 + b"C" + b"A" * 100], w)
+    stats, _ = check_3pass([b"A" * 600], [b"A" * 600, b"A" * 300, b"A" * 100 + b"C" + b"A" * 100], w)
     assert stats["tier32"] == 1
 
 

@@ -89,7 +89,7 @@ def test_3pass_cigars_for_long_reads():
     rng = np.random.default_rng(25)
     genome = synth.random_dna(rng, 5000)
     reads = ont_reads(rng, genome, 7, 1100, 2600) + [synth.random_dna(rng, 1300), genome[500:1700].copy()]
-    stats = check_3pass([genome], reads, W25)
+    stats, _ = check_3pass([genome], reads, W25)
     assert stats["tp_banded"] > 0
     check_3pass([genome], reads[:3], W25, profiled_is_query=True)
     s = golden("CY137594.txt")
@@ -105,7 +105,7 @@ def test_3pass_warp_kernel_scalar_fallback_and_wide_bands():
     chimera = np.concatenate([g[100:700], g[1900:2500]])           # 1200 nt, a 1200-column deletion in the middle
     shifted = np.concatenate([g[200:900], synth.random_dna(rng, 300), g[900:1500]])  # a 300-nt insertion
     reads = [chimera, shifted] + ont_reads(rng, g, 3, 1100, 1600)
-    stats = check_3pass([g], reads, WeightMatrix.new_dna_matrix(2, -5, b"N"), go=-3, ge=-1)
+    stats, _ = check_3pass([g], reads, WeightMatrix.new_dna_matrix(2, -5, b"N"), go=-3, ge=-1)
     assert stats["tp_band_attempts"] > stats["tp_banded"]
 
 

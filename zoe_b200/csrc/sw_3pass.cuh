@@ -453,15 +453,11 @@ __global__ void __launch_bounds__(512) tp_band_warp_kernel(const ThreePassParams
             }
             __syncwarp();
         }
-        // the pair's best cell: max value, then the smallest row, then the smallest column
-        unsigned long long key = ((unsigned long long)(uint32_t)best << 40) |
-                                 ((unsigned long long)(0xFFFFFu - min(br, 0xFFFFFu)) << 20) | (unsigned long long)(0xFFFFFu - min(bc, 0xFFFFFu));
-        for (int d = 16; d >= 1; d >>= 1) {
-            const unsigned long long o = __shfl_xor_sync(ALL, key, d);
-            key = o > key ? o : key;
-        }
-        const int32_t s_best = (int32_t)(key >> 40);
-        const uint32_t r_end = 0xFFFFFu - (uint32_t)((key >> 20) & 0xFFFFFu), c_end = 0xFFFFFu - (uint32_t)(key & 0xFFFFFu);
+        // the pair's best cell: max value, then the smallest row, then the smallest column -- three reductions over full
+        // 32-bit values, so every row and score of a box is exact (no packed key to truncate them)
+        const int32_t s_best = __reduce_max_sync(ALL, best);
+        const uint32_t r_end = __reduce_min_sync(ALL, best == s_best ? br : 0xFFFFFFFFu);
+        const uint32_t c_end = __reduce_min_sync(ALL, best == s_best && br == r_end ? bc : 0xFFFFFFFFu);
         __threadfence_block();
         __syncwarp();
         if (lane == 0) {
