@@ -21,6 +21,7 @@
 #include <mutex>
 #include <string>
 #include <thread>
+#include <type_traits>
 #include <vector>
 
 #include "sw_align.cuh"
@@ -55,9 +56,22 @@ struct DebugTimer {  // host-side phase timing, printed when ZOE_CUDA_DEBUG is s
     }
 };
 
+// A device allocation, freed by its destructor (with its device current: see ~Device).  Move-only; a moved-from buffer
+// owns nothing.
 struct DevBuf {
     void *p = nullptr;
     size_t cap = 0;
+    DevBuf() = default;
+    DevBuf(DevBuf &&o) noexcept : p(std::exchange(o.p, nullptr)), cap(std::exchange(o.cap, 0)) {}
+    DevBuf &operator=(DevBuf &&o) noexcept {
+        if (this != &o) {
+            release();
+            p = std::exchange(o.p, nullptr);
+            cap = std::exchange(o.cap, 0);
+        }
+        return *this;
+    }
+    ~DevBuf() { release(); }
     cudaError_t reserve(size_t bytes) {
         if (bytes <= cap) return cudaSuccess;
         if (p) cudaFree(p);
@@ -78,27 +92,57 @@ struct DevBuf {
         return reinterpret_cast<T *>(p);
     }
 };
+static_assert(!std::is_copy_constructible_v<DevBuf>);
 
-struct Device {
+// The streams and events of a Device, destroyed after its buffers with the device current (~Device).  Move-only; a
+// moved-from set owns nothing.
+struct DeviceStreams {
+    cudaStream_t stream = nullptr;
+    // split upload (end-to-end calls): the first 1/8 of the sequences, then the rest, on `copy_stream`; the first kernel of
+    // the call runs on the first part while the second is still arriving
+    cudaStream_t copy_stream = nullptr;
+    cudaEvent_t ev_first = nullptr, ev_copied = nullptr;
+    cudaStream_t aux_stream = nullptr;  // align: the pin sweep of the ambiguous pairs runs beside the main window fill
+    cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
+    cudaEvent_t ev_begin = nullptr, ev_end = nullptr, ev_k0 = nullptr, ev_k1 = nullptr;
+    DeviceStreams() = default;
+    DeviceStreams(DeviceStreams &&o) noexcept
+        : stream(std::exchange(o.stream, nullptr)), copy_stream(std::exchange(o.copy_stream, nullptr)),
+          ev_first(std::exchange(o.ev_first, nullptr)), ev_copied(std::exchange(o.ev_copied, nullptr)),
+          aux_stream(std::exchange(o.aux_stream, nullptr)), ev_fork(std::exchange(o.ev_fork, nullptr)),
+          ev_join(std::exchange(o.ev_join, nullptr)), ev_begin(std::exchange(o.ev_begin, nullptr)),
+          ev_end(std::exchange(o.ev_end, nullptr)), ev_k0(std::exchange(o.ev_k0, nullptr)),
+          ev_k1(std::exchange(o.ev_k1, nullptr)) {}
+    ~DeviceStreams() {
+        for (cudaEvent_t e : {ev_begin, ev_end, ev_k0, ev_k1, ev_fork, ev_join})
+            if (e) cudaEventDestroy(e);
+        if (aux_stream) cudaStreamDestroy(aux_stream);
+        if (copy_stream) cudaStreamDestroy(copy_stream);
+        for (cudaEvent_t e : {ev_first, ev_copied})
+            if (e) cudaEventDestroy(e);
+        if (stream) cudaStreamDestroy(stream);
+    }
+};
+
+struct Device : DeviceStreams {
     int id = 0;
     int sm_count = 0;
     size_t free_at_create = 0;  // cudaMemGetInfo is slow (tens of ms on a 180 GB part): asked once
-    cudaStream_t stream = nullptr;
+    Device() = default;
+    Device(Device &&) = default;
+    // the buffers, then the streams and events, are freed with the device current; every one of them is created after
+    // `stream`, so a device without one (moved from, or not created) owns nothing
+    ~Device() {
+        if (stream) cudaSetDevice(id);
+    }
     // per-profiled-sequence base offsets (flag_base / ckpt_base) are a function of the profiled set, the kernel's (G, K) and
     // the checkpoint spacing: uploaded once and reused (a pageable-memory copy synchronises the stream: 0.4 ms per call)
     uint64_t flb_epoch = 0, ckb_epoch = 0;
     int flb_G = 0, flb_K = 0, ckb_G = 0, ckb_K = 0, ckb_cb = -1;
     bool ckpt_base_cached(uint64_t epoch, int G, int K, int cb) const { return ckb_epoch == epoch && ckb_G == G && ckb_K == K && ckb_cb == cb; }
     void ckpt_base_mark(uint64_t epoch, int G, int K, int cb) { ckb_epoch = epoch; ckb_G = G; ckb_K = K; ckb_cb = cb; }
-    // split upload (end-to-end calls): the first 1/8 of the sequences, then the rest, on `copy_stream`; the first kernel of
-    // the call runs on the first part while the second is still arriving
-    cudaStream_t copy_stream = nullptr;
-    cudaEvent_t ev_first = nullptr, ev_copied = nullptr;
-    bool copy_pending = false;
+    bool copy_pending = false;  // split upload: the second part is still arriving on copy_stream
     uint64_t seq_split = 0;  // sequences [0, seq_split) of the shard are in the first part (even)
-    cudaStream_t aux_stream = nullptr;  // align: the pin sweep of the ambiguous pairs runs beside the main window fill
-    cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-    cudaEvent_t ev_begin = nullptr, ev_end = nullptr, ev_k0 = nullptr, ev_k1 = nullptr;
     // scoring + profiled (replicated on every device)
     DevBuf ccodes, coff, wk, lut, corder;
     DevBuf ccodes_g, coff_g, corder_g;  // profiled set regrouped for panels beyond the shared-memory staging area
@@ -312,6 +356,28 @@ int fail(zoe_cuda_ctx *ctx, int code, const char *fmt, ...) {
             return fail(ctx, ZOE_CUDA_E_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e__), \
                         __FILE__, __LINE__);                                                       \
     } while (0)
+
+// Calls fn on every device in turn, then, with_alt, on every second lane (zoe_cuda_ctx::alt); stops at the first error.
+template <class Fn>
+int visit_devices(zoe_cuda_ctx *ctx, bool with_alt, Fn fn) {
+    for (Device &d : ctx->devs)
+        if (int rc = fn(d)) return rc;
+    if (with_alt)
+        for (Device &d : ctx->alt)
+            if (int rc = fn(d)) return rc;
+    return 0;
+}
+
+// Waits for every stream of the call on every device, errors ignored: no copy from the caller's buffers is in flight
+// afterwards, and no split upload is pending.
+void drain_devices(zoe_cuda_ctx *ctx) {
+    for (Device &d : ctx->devs) {
+        cudaSetDevice(d.id);
+        if (d.copy_stream) cudaStreamSynchronize(d.copy_stream);
+        cudaStreamSynchronize(d.stream);
+        d.copy_pending = false;
+    }
+}
 
 // Largest score each allowed integer type can report (striped.rs:608-633): signed T holds best - MIN < MAX - MIN, i.e.
 // score <= 2*MAX; unsigned T with a biased matrix needs best + bias + 1 not to overflow, i.e. score <= MAX - bias - 1.
@@ -592,11 +658,7 @@ void pick_scan2(zoe_cuda_ctx *ctx, const KernelEntry &k, void (**scan_fn)(const 
 }
 
 int upload_scoring_and_profiled(zoe_cuda_ctx *ctx) {
-    std::vector<Device *> all;
-    for (Device &d : ctx->devs) all.push_back(&d);
-    for (Device &d : ctx->alt) all.push_back(&d);
-    for (Device *dp : all) {
-        Device &d = *dp;
+    return visit_devices(ctx, true, [&](Device &d) {
         CU(ctx, cudaSetDevice(d.id));
         CU(ctx, d.ccodes.reserve(ctx->ccodes.size()));
         CU(ctx, d.coff.reserve(ctx->coff.size() * sizeof(uint32_t)));
@@ -627,8 +689,8 @@ int upload_scoring_and_profiled(zoe_cuda_ctx *ctx) {
         CU(ctx, cudaMemcpyAsync(d.weights.p, ctx->weights.data(), ctx->weights.size(), cudaMemcpyHostToDevice,
                                 d.stream));
         CU(ctx, cudaStreamSynchronize(d.stream));
-    }
-    return 0;
+        return 0;
+    });
 }
 
 // The host-side derivation of a profiled set (offsets validated by the caller; max_len its longest sequence): symbol
@@ -872,10 +934,7 @@ int stage_on_devices(zoe_cuda_ctx *ctx, const uint8_t *concat, const uint64_t *o
         }
     rc = prepare_batch(ctx, concat, offsets, n);
     if (rc) {
-        for (Device &d : ctx->devs) {
-            cudaSetDevice(d.id);
-            cudaStreamSynchronize(d.stream);
-        }
+        drain_devices(ctx);
         return rc;
     }
     if (!early)
@@ -1323,6 +1382,29 @@ __global__ void collect_mapped_kernel(const AlignEnd *ends, const uint8_t *statu
     const bool mapped = status[gid] == ZOE_CUDA_SOME;
     hazard[gid] = mapped ? 1 : 0;
     if (mapped) hazard_list[atomicAdd(&counters[5], 1ULL)] = gid;
+}
+
+// Queues the exclusive scan of the 32-bit counts cnt[first, first + n) into off[first, first + n], seeded with the
+// running base *base, and leaves the base after them in off[first + n] and *base: the CIGAR offset scan.  The caller
+// zeroes *base before the first scan of a chain.
+int scan_counts(zoe_cuda_ctx *ctx, Device &d, const uint32_t *cnt, uint64_t first, uint64_t n, uint64_t *off,
+                unsigned long long *base) {
+    if (n >= (1u << 16)) {  // three short launches instead of one block walking a million counts
+        const uint32_t nbk = (uint32_t)((n + 1023) / 1024);
+        CU(ctx, d.cig_bsum.reserve((size_t)nbk * sizeof(unsigned long long)));
+        cigar_block_sum_kernel<<<nbk, 1024, 0, d.stream>>>(cnt, first, n, d.cig_bsum.as<unsigned long long>());
+        CU(ctx, cudaGetLastError());
+        cigar_scan_sums_kernel<<<1, 1024, 0, d.stream>>>(d.cig_bsum.as<unsigned long long>(), nbk, base, off + first + n);
+        CU(ctx, cudaGetLastError());
+        cigar_block_scan_kernel<<<nbk, 1024, 0, d.stream>>>(cnt, first, n, d.cig_bsum.as<unsigned long long>(), off);
+        CU(ctx, cudaGetLastError());
+        ctx->last_launches += 3;
+    } else {
+        cigar_scan_kernel<<<1, 1024, 0, d.stream>>>(cnt, first, n, off, base);
+        CU(ctx, cudaGetLastError());
+        ctx->last_launches++;
+    }
+    return 0;
 }
 
 int run_ranges_long_on_device(zoe_cuda_ctx *ctx, Device &d);
@@ -1963,29 +2045,13 @@ int run_align_on_device(zoe_cuda_ctx *ctx, Device &d, uint64_t cigar_cap_words) 
             ctx->stats.hazard += n_exact - hc[4];
         }
         // ---- CIGAR compaction, chained through the device-side running base ctr[9] ----
-        if (cpairs >= (1u << 16)) {  // three short launches instead of one block walking a million counts
-            const uint32_t nbk = (cpairs + 1023) / 1024;
-            CU(ctx, d.cig_bsum.reserve((size_t)nbk * sizeof(unsigned long long)));
-            cigar_block_sum_kernel<<<nbk, 1024, 0, d.stream>>>(t.cig_count, (uint64_t)c0 * n_prof, cpairs,
-                                                               d.cig_bsum.as<unsigned long long>());
-            CU(ctx, cudaGetLastError());
-            cigar_scan_sums_kernel<<<1, 1024, 0, d.stream>>>(d.cig_bsum.as<unsigned long long>(), nbk, ctr + 9,
-                                                             d.cig_off.as<uint64_t>() + (uint64_t)c0 * n_prof + cpairs);
-            CU(ctx, cudaGetLastError());
-            cigar_block_scan_kernel<<<nbk, 1024, 0, d.stream>>>(t.cig_count, (uint64_t)c0 * n_prof, cpairs,
-                                                                d.cig_bsum.as<unsigned long long>(), d.cig_off.as<uint64_t>());
-            CU(ctx, cudaGetLastError());
-            ctx->last_launches += 2;
-        } else {
-            cigar_scan_kernel<<<1, 1024, 0, d.stream>>>(t.cig_count, (uint64_t)c0 * n_prof, cpairs, d.cig_off.as<uint64_t>(),
-                                                        ctr + 9);
-            CU(ctx, cudaGetLastError());
-        }
+        rc = scan_counts(ctx, d, t.cig_count, (uint64_t)c0 * n_prof, cpairs, d.cig_off.as<uint64_t>(), ctr + 9);
+        if (rc) return rc;
         cigar_gather_kernel<<<cpairs, 32, 0, d.stream>>>(t.cig_scratch, cig_cap, nullptr, cpairs, (uint32_t)(c0 * n_prof),
                                                          t.cig_count, d.cig_off.as<uint64_t>(), d.cig_out.as<uint32_t>(),
                                                          cigar_cap_words, t.hazard);
         CU(ctx, cudaGetLastError());
-        ctx->last_launches += 2;
+        ctx->last_launches++;
         if (n_exact > 0) {
             cigar_gather_kernel<<<n_exact, 32, 0, d.stream>>>(d.ex_cig.as<uint32_t>(), cig_cap, d.hazard_list.as<uint32_t>(),
                                                               n_exact, 0, t.cig_count, d.cig_off.as<uint64_t>(),
@@ -2629,23 +2695,8 @@ int run_3pass_on_device(zoe_cuda_ctx *ctx, Device &d, uint64_t cigar_cap_words) 
             }
         }
         // CIGAR compaction, chained through the device-side running base ctr[9]
-        if (cn >= (1u << 16)) {
-            const uint32_t nbk = (cn + 1023) / 1024;
-            CU(ctx, d.cig_bsum.reserve((size_t)nbk * sizeof(unsigned long long)));
-            cigar_block_sum_kernel<<<nbk, 1024, 0, d.stream>>>(t.cig_count, p0, cn, d.cig_bsum.as<unsigned long long>());
-            CU(ctx, cudaGetLastError());
-            cigar_scan_sums_kernel<<<1, 1024, 0, d.stream>>>(d.cig_bsum.as<unsigned long long>(), nbk, ctr + 9,
-                                                             d.cig_off.as<uint64_t>() + p0 + cn);
-            CU(ctx, cudaGetLastError());
-            cigar_block_scan_kernel<<<nbk, 1024, 0, d.stream>>>(t.cig_count, p0, cn, d.cig_bsum.as<unsigned long long>(),
-                                                                d.cig_off.as<uint64_t>());
-            CU(ctx, cudaGetLastError());
-            ctx->last_launches += 3;
-        } else {
-            cigar_scan_kernel<<<1, 1024, 0, d.stream>>>(t.cig_count, p0, cn, d.cig_off.as<uint64_t>(), ctr + 9);
-            CU(ctx, cudaGetLastError());
-            ctx->last_launches++;
-        }
+        rc = scan_counts(ctx, d, t.cig_count, p0, cn, d.cig_off.as<uint64_t>(), ctr + 9);
+        if (rc) return rc;
         tp_gather_kernel<<<(cn + 255) / 256, 256, 0, d.stream>>>(t, d.cig_off.as<uint64_t>(), d.cig_out.as<uint32_t>(),
                                                                  cigar_cap_words);
         CU(ctx, cudaGetLastError());
@@ -2685,12 +2736,7 @@ int for_each_device(zoe_cuda_ctx *ctx, Fn fn) {
 
 int sync_and_time(zoe_cuda_ctx *ctx) {
     float total = 0.f, dp = 0.f;
-    std::vector<Device *> all;
-    for (Device &d : ctx->devs) all.push_back(&d);
-    if (ctx->alt_used)
-        for (Device &d : ctx->alt) all.push_back(&d);
-    for (Device *dp_ : all) {
-        Device &d = *dp_;
+    int rc = visit_devices(ctx, ctx->alt_used, [&](Device &d) {
         CU(ctx, cudaSetDevice(d.id));
         CU(ctx, cudaEventRecord(d.ev_end, d.stream));
         CU(ctx, cudaStreamSynchronize(d.stream));
@@ -2701,20 +2747,17 @@ int sync_and_time(zoe_cuda_ctx *ctx) {
             CU(ctx, cudaEventElapsedTime(&t, d.ev_k0, d.ev_k1));
             dp = std::max(dp, t);
         }
-    }
+        return 0;
+    });
+    if (rc) return rc;
     ctx->last_total_ms = total;
     ctx->last_dp_ms = std::max(dp, ctx->last_dp_ms);
     return 0;
 }
 
 int gather_stats(zoe_cuda_ctx *ctx) {
-    std::vector<Device *> all;
-    for (Device &d : ctx->devs) all.push_back(&d);
-    if (ctx->alt_used)
-        for (Device &d : ctx->alt) all.push_back(&d);
-    for (Device *dp_ : all) {
-        Device &d = *dp_;
-        if (d.n_count == 0 || !d.counters.p) continue;
+    int rc = visit_devices(ctx, ctx->alt_used, [&](Device &d) {
+        if (d.n_count == 0 || !d.counters.p) return 0;
         CU(ctx, cudaSetDevice(d.id));
         unsigned long long c[16];
         CU(ctx, cudaMemcpy(c, d.counters.p, sizeof(c), cudaMemcpyDeviceToHost));
@@ -2723,7 +2766,9 @@ int gather_stats(zoe_cuda_ctx *ctx) {
         ctx->stats.tier32 += c[2];
         ctx->stats.unmapped += c[3];
         ctx->stats.overflowed += c[13];
-    }
+        return 0;
+    });
+    if (rc) return rc;
     ctx->stats.pairs = ctx->staged_n * ctx->n_prof;
     ctx->stats.cells = ctx->staged_cells;
     return 0;
@@ -2733,86 +2778,134 @@ void begin_call(zoe_cuda_ctx *ctx) {
     ctx->last_launches = 0;
     ctx->last_dp_ms = 0.f;
     ctx->stats = zoe_cuda_stats{};
-    for (Device &d : ctx->devs) d.timed_kernel = false;
-    for (Device &d : ctx->alt) d.timed_kernel = false;
+    visit_devices(ctx, true, [](Device &d) { d.timed_kernel = false; return 0; });
 }
 
-// Copies the per-pair alignment outputs and the compacted CIGAR stream of every device into the caller's arrays
-// (devices own contiguous index ranges; CIGAR offsets become global).  Shared by the align and 3-pass entry points.
-int fetch_alignments(zoe_cuda_ctx *ctx, uint32_t *score, uint8_t *status, uint8_t *tier, uint32_t *ref_start,
-                     uint32_t *ref_end, uint32_t *query_start, uint32_t *query_end, uint32_t *cigar, uint64_t *cigar_off,
-                     uint64_t cigar_cap, uint8_t *hazard) {
-    // CIGAR offsets: device-local running sums -> global offsets (devices own contiguous index ranges)
-    uint64_t total = 0;
-    for (Device &d : ctx->devs) total += d.cig_total;
-    if (total > cigar_cap) {
-        cigar_off[0] = total;
-        sync_and_time(ctx);
-        return fail(ctx, ZOE_CUDA_E_CIGAR_CAP, "CIGAR buffer too small: need %llu words, have %llu",
-                    (unsigned long long)total, (unsigned long long)cigar_cap);
-    }
+// The per-pair host outputs of a batch call (null: not wanted), as the C ABI functions receive them; hit / runner_up
+// are the best-hit search's per-read outputs.
+struct Outputs {
+    uint32_t *score = nullptr;
+    uint8_t *status = nullptr, *tier = nullptr;
+    uint32_t *ref_start = nullptr, *ref_end = nullptr, *query_start = nullptr, *query_end = nullptr;
+    uint32_t *cigar = nullptr;
+    uint64_t *cigar_off = nullptr;
+    uint64_t cigar_cap = 0;
+    uint8_t *hazard = nullptr, *strand = nullptr;
+    uint32_t *hit = nullptr, *runner_up = nullptr;
+};
+
+// One output of queue_rows_d2h: the caller's array, the device buffer its rows come from, the bytes of one row.
+struct RowOut {
+    void *dst;
+    const DevBuf &src;
+    size_t elem;
+};
+
+// Queues the D2H copies of the device's rows [first, first + count) of every output with a destination behind its
+// kernels (a device buffer holds the device's rows from its start).
+int queue_rows_d2h(zoe_cuda_ctx *ctx, Device &d, size_t first, size_t count, std::initializer_list<RowOut> outs) {
+    if (count == 0) return 0;
+    CU(ctx, cudaSetDevice(d.id));
+    for (const RowOut &o : outs)
+        if (o.dst)
+            CU(ctx, cudaMemcpyAsync((uint8_t *)o.dst + first * o.elem, o.src.p, count * o.elem, cudaMemcpyDeviceToHost,
+                                    d.stream));
+    return 0;
+}
+
+// The per-pair outputs of the score, ranges and align pipelines (the device's pairs are rows of n_prof entries).
+int queue_pair_outputs_d2h(zoe_cuda_ctx *ctx, Device &d, const Outputs &o) {
+    const size_t P = ctx->n_prof;
+    return queue_rows_d2h(ctx, d, d.n_first * P, d.n_count * P,
+                          {{o.score, d.score, 4}, {o.status, d.status, 1}, {o.tier, d.tier, 1}, {o.ref_start, d.ref_start, 4},
+                           {o.ref_end, d.ref_end, 4}, {o.query_start, d.query_start, 4}, {o.query_end, d.query_end, 4},
+                           {o.hazard, d.hazard, 1}});
+}
+
+int queue_pair_outputs_d2h(zoe_cuda_ctx *ctx, const Outputs &o) {
+    return visit_devices(ctx, false, [&](Device &d) { return queue_pair_outputs_d2h(ctx, d, o); });
+}
+
+// A CIGAR stream that does not fit the caller's buffer: the need goes to cigar_off[0].
+int cigar_cap_error(zoe_cuda_ctx *ctx, const Outputs &o, uint64_t need, const char *needs) {
+    o.cigar_off[0] = need;
+    return fail(ctx, ZOE_CUDA_E_CIGAR_CAP, "CIGAR buffer too small: %s %llu words, have %llu", needs,
+                (unsigned long long)need, (unsigned long long)o.cigar_cap);
+}
+
+// Copies every device's CIGAR stream into the caller's arrays: the offsets of its rows (rows_per_seq per sequence, one
+// more for the end) from d.*off and words[k] words from d.*cig, then rebases the offsets to global positions (devices
+// own contiguous row ranges).
+int fetch_cigar_stream(zoe_cuda_ctx *ctx, const Outputs &o, size_t rows_per_seq, DevBuf Device::*off, DevBuf Device::*cig,
+                       const std::vector<uint64_t> &words) {
     uint64_t base = 0;
-    for (Device &d : ctx->devs) {
+    for (size_t k = 0; k < ctx->devs.size(); ++k) {
+        Device &d = ctx->devs[k];
         if (d.n_count == 0) continue;
         CU(ctx, cudaSetDevice(d.id));
-        size_t first = (size_t)d.n_first * ctx->n_prof, pairs = (size_t)d.n_count * ctx->n_prof;
-        auto d2h = [&](void *dst, const DevBuf &src, size_t elem) -> cudaError_t {
-            if (!dst) return cudaSuccess;
-            return cudaMemcpyAsync((uint8_t *)dst + first * elem, src.p, pairs * elem, cudaMemcpyDeviceToHost, d.stream);
-        };
-        CU(ctx, d2h(score, d.score, 4));
-        CU(ctx, d2h(status, d.status, 1));
-        CU(ctx, d2h(tier, d.tier, 1));
-        CU(ctx, d2h(ref_start, d.ref_start, 4));
-        CU(ctx, d2h(ref_end, d.ref_end, 4));
-        CU(ctx, d2h(query_start, d.query_start, 4));
-        CU(ctx, d2h(query_end, d.query_end, 4));
-        if (hazard) CU(ctx, d2h(hazard, d.hazard, 1));
-        CU(ctx, cudaMemcpyAsync(cigar_off + first, d.cig_off.p, (pairs + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost,
+        const size_t first = d.n_first * rows_per_seq, rows = d.n_count * rows_per_seq;
+        CU(ctx, cudaMemcpyAsync(o.cigar_off + first, (d.*off).p, (rows + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost,
                                 d.stream));
-        if (d.cig_total)
-            CU(ctx, cudaMemcpyAsync(cigar + base, d.cig_out.p, d.cig_total * sizeof(uint32_t), cudaMemcpyDeviceToHost,
+        if (words[k])
+            CU(ctx, cudaMemcpyAsync(o.cigar + base, (d.*cig).p, words[k] * sizeof(uint32_t), cudaMemcpyDeviceToHost,
                                     d.stream));
         CU(ctx, cudaStreamSynchronize(d.stream));
         if (base)
-            for (size_t i = 0; i <= pairs; ++i) cigar_off[first + i] += base;
-        base += d.cig_total;
+            for (size_t i = 0; i <= rows; ++i) o.cigar_off[first + i] += base;
+        base += words[k];
     }
     return 0;
 }
 
-// Queues the D2H copies of a device's score outputs behind its kernels (score entry points).
-int queue_score_d2h(zoe_cuda_ctx *ctx, Device &d, uint32_t *score, uint8_t *status, uint8_t *tier) {
-    if (d.n_count == 0) return 0;
-    CU(ctx, cudaSetDevice(d.id));
-    size_t first = (size_t)d.n_first * ctx->n_prof, pairs = (size_t)d.n_count * ctx->n_prof;
-    if (score)
-        CU(ctx, cudaMemcpyAsync(score + first, d.score.p, pairs * sizeof(uint32_t), cudaMemcpyDeviceToHost, d.stream));
-    if (status) CU(ctx, cudaMemcpyAsync(status + first, d.status.p, pairs, cudaMemcpyDeviceToHost, d.stream));
-    if (tier) CU(ctx, cudaMemcpyAsync(tier + first, d.tier.p, pairs, cudaMemcpyDeviceToHost, d.stream));
-    return 0;
-}
-
-// Queues the D2H copies of every device's ranges outputs (ranges entry points).
-int queue_ranges_d2h(zoe_cuda_ctx *ctx, uint32_t *score, uint8_t *status, uint8_t *tier, uint32_t *ref_start,
-                     uint32_t *ref_end, uint32_t *query_start, uint32_t *query_end) {
+// Copies the per-pair alignment outputs and the compacted CIGAR stream of every device into the caller's arrays.
+// Shared by the align and 3-pass entry points.
+int fetch_alignments(zoe_cuda_ctx *ctx, const Outputs &o) {
+    std::vector<uint64_t> words;
+    uint64_t total = 0;
     for (Device &d : ctx->devs) {
-        if (d.n_count == 0) continue;
-        CU(ctx, cudaSetDevice(d.id));
-        size_t first = (size_t)d.n_first * ctx->n_prof, pairs = (size_t)d.n_count * ctx->n_prof;
-        auto d2h = [&](void *dst, const DevBuf &src, size_t elem) -> cudaError_t {
-            if (!dst) return cudaSuccess;
-            return cudaMemcpyAsync((uint8_t *)dst + first * elem, src.p, pairs * elem, cudaMemcpyDeviceToHost, d.stream);
-        };
-        CU(ctx, d2h(score, d.score, 4));
-        CU(ctx, d2h(status, d.status, 1));
-        CU(ctx, d2h(tier, d.tier, 1));
-        CU(ctx, d2h(ref_start, d.ref_start, 4));
-        CU(ctx, d2h(ref_end, d.ref_end, 4));
-        CU(ctx, d2h(query_start, d.query_start, 4));
-        CU(ctx, d2h(query_end, d.query_end, 4));
+        words.push_back(d.cig_total);
+        total += d.cig_total;
     }
-    return 0;
+    if (total > o.cigar_cap) {
+        sync_and_time(ctx);
+        return cigar_cap_error(ctx, o, total, "need");
+    }
+    int rc = queue_pair_outputs_d2h(ctx, o);
+    if (rc) return rc;
+    return fetch_cigar_stream(ctx, o, ctx->n_prof, &Device::cig_off, &Device::cig_out, words);
+}
+
+constexpr int kNotMixed = 1;
+int align_split_long_short(zoe_cuda_ctx *ctx, bool both_strands, const uint8_t *streamed_concat, const uint64_t *offsets,
+                           uint64_t n, const Outputs &o);
+
+// The single-strand align entry point.
+int align_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_concat, const uint64_t *offsets, uint64_t n, const Outputs &o) {
+    if (!o.cigar_off || (!o.cigar && o.cigar_cap)) return fail(ctx, ZOE_CUDA_E_BAD_ARG, "null CIGAR outputs");
+    begin_call(ctx);
+    DebugTimer dbg;
+    int rc = stage_on_devices(ctx, streamed_concat, offsets, n, /*split=*/true);
+    if (rc) return rc;
+    dbg.lap("align: stage");
+    // A batch that mixes long (> 1024 residues) and short sequences is split (align_split_long_short).
+    // Detected from the lengths the staging pass collects anyway (a separate pass that lists the indices of 1M reads
+    // cost 3-4 ms of host time in front of every call); the upload already queued for the whole batch is drained and dropped.
+    if (n > 0 && ctx->staged_max_len > (uint32_t)kMaxRowsSinglePass && ctx->staged_min_len <= (uint32_t)kMaxRowsSinglePass) {
+        drain_devices(ctx);
+        ctx->staged = false;
+        rc = align_split_long_short(ctx, false, streamed_concat, offsets, n, o);
+        if (rc != kNotMixed) return rc;
+    }
+    rc = for_each_device(ctx, [&](Device &d) { return run_align_on_device(ctx, d, o.cigar_cap); });
+    if (rc) return rc;
+    dbg.lap("align: run_align_on_device");
+    rc = fetch_alignments(ctx, o);
+    if (rc) return rc;
+    if (n == 0) o.cigar_off[0] = 0;
+    dbg.lap("align: d2h");
+    rc = sync_and_time(ctx);
+    if (rc) return rc;
+    return gather_stats(ctx);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -2856,13 +2949,7 @@ struct DoubledView {
     ~DoubledView() {
         leave();
         ctx->staged = false;
-        if (ok) return;
-        for (Device &d : ctx->devs) {
-            cudaSetDevice(d.id);
-            if (d.copy_stream) cudaStreamSynchronize(d.copy_stream);
-            cudaStreamSynchronize(d.stream);
-            d.copy_pending = false;
-        }
+        if (!ok) drain_devices(ctx);
     }
 };
 
@@ -2997,28 +3084,6 @@ int stage_pairs(zoe_cuda_ctx *ctx, DoubledView &view, const uint8_t *concat1, co
     return 0;
 }
 
-// Queues the exclusive scan of n 32-bit counts into off[0, n] (off[n] = the total, also left in *base, which is zeroed
-// first): the CIGAR offset scan of the align pipeline.
-int scan_counts(zoe_cuda_ctx *ctx, Device &d, const uint32_t *cnt, uint64_t n, uint64_t *off, unsigned long long *base) {
-    CU(ctx, cudaMemsetAsync(base, 0, sizeof(unsigned long long), d.stream));
-    if (n >= (1u << 16)) {
-        const uint32_t nbk = (uint32_t)((n + 1023) / 1024);
-        CU(ctx, d.cig_bsum.reserve((size_t)nbk * sizeof(unsigned long long)));
-        cigar_block_sum_kernel<<<nbk, 1024, 0, d.stream>>>(cnt, 0, n, d.cig_bsum.as<unsigned long long>());
-        CU(ctx, cudaGetLastError());
-        cigar_scan_sums_kernel<<<1, 1024, 0, d.stream>>>(d.cig_bsum.as<unsigned long long>(), nbk, base, off + n);
-        CU(ctx, cudaGetLastError());
-        cigar_block_scan_kernel<<<nbk, 1024, 0, d.stream>>>(cnt, 0, n, d.cig_bsum.as<unsigned long long>(), off);
-        CU(ctx, cudaGetLastError());
-        ctx->last_launches += 3;
-    } else {
-        cigar_scan_kernel<<<1, 1024, 0, d.stream>>>(cnt, 0, n, off, base);
-        CU(ctx, cudaGetLastError());
-        ctx->last_launches++;
-    }
-    return 0;
-}
-
 enum class StrandOutputs { Score, Ranges, Align, ThreePass };
 
 // Strand selection on one device (doubled view): gathers the selected strand's per-pair outputs into the buffers the
@@ -3063,7 +3128,8 @@ int select_strands(zoe_cuda_ctx *ctx, Device &d, StrandOutputs kind, uint64_t *c
     CU(ctx, d.sel_cig_off.reserve((n_out + 1) * sizeof(uint64_t)));
     CU(ctx, d.sel_ctr.reserve(sizeof(unsigned long long)));
     unsigned long long *base = d.sel_ctr.as<unsigned long long>();
-    int rc = scan_counts(ctx, d, d.sel_cig_count.as<uint32_t>(), n_out, d.sel_cig_off.as<uint64_t>(), base);
+    CU(ctx, cudaMemsetAsync(base, 0, sizeof(unsigned long long), d.stream));
+    int rc = scan_counts(ctx, d, d.sel_cig_count.as<uint32_t>(), 0, n_out, d.sel_cig_off.as<uint64_t>(), base);
     if (rc) return rc;
     unsigned long long need = 0;
     CU(ctx, cudaMemcpyAsync(&need, base, sizeof(need), cudaMemcpyDeviceToHost, d.stream));
@@ -3096,13 +3162,9 @@ int gather_strand_cigars(zoe_cuda_ctx *ctx, Device &d, uint64_t total) {
 // Copies every device's strand choices into the caller's array (real view).
 int queue_strand_d2h(zoe_cuda_ctx *ctx, uint8_t *strand) {
     if (!strand) return 0;
-    for (Device &d : ctx->devs) {
-        if (d.n_count == 0) continue;
-        CU(ctx, cudaSetDevice(d.id));
-        CU(ctx, cudaMemcpyAsync(strand + (size_t)d.n_first * ctx->n_prof, d.strand.p, (size_t)d.n_count * ctx->n_prof,
-                                cudaMemcpyDeviceToHost, d.stream));
-    }
-    return 0;
+    const size_t P = ctx->n_prof;
+    return visit_devices(ctx, false,
+                         [&](Device &d) { return queue_rows_d2h(ctx, d, d.n_first * P, d.n_count * P, {{strand, d.strand, 1}}); });
 }
 
 // The statistics of a both-strand call count the work done: gather_stats ran on the real view, its counters on the
@@ -3114,20 +3176,12 @@ int gather_both_strands_stats(zoe_cuda_ctx *ctx) {
     return rc;
 }
 
-constexpr int kNotMixed = 1;
-int align_split_long_short(zoe_cuda_ctx *ctx, bool both_strands, const uint8_t *streamed_concat, const uint64_t *offsets,
-                           uint64_t n, uint32_t *score, uint8_t *status, uint8_t *tier, uint32_t *ref_start,
-                           uint32_t *ref_end, uint32_t *query_start, uint32_t *query_end, uint32_t *cigar,
-                           uint64_t *cigar_off, uint64_t cigar_cap, uint8_t *hazard, uint8_t *strand);
-
 // The align and 3-pass both-strand entry points.  The doubled run gets its own device CIGAR capacity (the caller's
 // capacity bounds the selected strands only); a run whose non-selected strands overflowed it is repeated once with the
 // exact need.
 int align_both_strands(zoe_cuda_ctx *ctx, bool three_pass, const uint8_t *streamed_concat, const uint64_t *offsets,
-                       uint64_t n, uint32_t *score, uint8_t *status, uint8_t *tier, uint32_t *ref_start, uint32_t *ref_end,
-                       uint32_t *query_start, uint32_t *query_end, uint32_t *cigar, uint64_t *cigar_off, uint64_t cigar_cap,
-                       uint8_t *hazard, uint8_t *strand) {
-    if (!cigar_off || (!cigar && cigar_cap)) return fail(ctx, ZOE_CUDA_E_BAD_ARG, "null CIGAR outputs");
+                       uint64_t n, const Outputs &o) {
+    if (!o.cigar_off || (!o.cigar && o.cigar_cap)) return fail(ctx, ZOE_CUDA_E_BAD_ARG, "null CIGAR outputs");
     begin_call(ctx);
     DoubledView view(ctx);
     int rc = check_both_strands_limits(ctx, n, true);
@@ -3140,8 +3194,7 @@ int align_both_strands(zoe_cuda_ctx *ctx, bool three_pass, const uint8_t *stream
             CU(ctx, cudaSetDevice(d.id));
             CU(ctx, cudaStreamSynchronize(d.stream));
         }
-        rc = align_split_long_short(ctx, true, streamed_concat, offsets, n, score, status, tier, ref_start, ref_end,
-                                    query_start, query_end, cigar, cigar_off, cigar_cap, hazard, strand);
+        rc = align_split_long_short(ctx, true, streamed_concat, offsets, n, o);
         if (rc != kNotMixed) {
             view.ok = rc == 0;
             return rc;
@@ -3153,7 +3206,7 @@ int align_both_strands(zoe_cuda_ctx *ctx, bool three_pass, const uint8_t *stream
     }
     view.enter();
     const StrandOutputs kind = three_pass ? StrandOutputs::ThreePass : StrandOutputs::Align;
-    uint64_t dev_cap = 2 * cigar_cap + 1024;
+    uint64_t dev_cap = 2 * o.cigar_cap + 1024;
     std::vector<uint64_t> need(ctx->devs.size());
     for (int attempt = 0;; ++attempt) {
         rc = for_each_device(ctx, [&](Device &d) {
@@ -3167,11 +3220,7 @@ int align_both_strands(zoe_cuda_ctx *ctx, bool three_pass, const uint8_t *stream
             total += need[k];
             widest = std::max<uint64_t>(widest, ctx->devs[k].cig_total);
         }
-        if (total > cigar_cap) {
-            cigar_off[0] = total;
-            return fail(ctx, ZOE_CUDA_E_CIGAR_CAP, "CIGAR buffer too small: the selected strands need %llu words, have %llu",
-                        (unsigned long long)total, (unsigned long long)cigar_cap);
-        }
+        if (total > o.cigar_cap) return cigar_cap_error(ctx, o, total, "the selected strands need");
         if (widest <= dev_cap) break;
         if (attempt > 0) return fail(ctx, ZOE_CUDA_E_STATE, "internal error: both-strand CIGAR capacity not met on the re-run");
         dev_cap = widest;
@@ -3181,12 +3230,11 @@ int align_both_strands(zoe_cuda_ctx *ctx, bool three_pass, const uint8_t *stream
         if (rc) return rc;
     }
     view.leave();
-    rc = queue_strand_d2h(ctx, strand);
+    rc = queue_strand_d2h(ctx, o.strand);
     if (rc) return rc;
-    rc = fetch_alignments(ctx, score, status, tier, ref_start, ref_end, query_start, query_end, cigar, cigar_off, cigar_cap,
-                          three_pass ? nullptr : hazard);
+    rc = fetch_alignments(ctx, o);
     if (rc) return rc;
-    if (n == 0) cigar_off[0] = 0;
+    if (n == 0) o.cigar_off[0] = 0;
     rc = sync_and_time(ctx);
     if (rc) return rc;
     view.ok = true;
@@ -3195,12 +3243,10 @@ int align_both_strands(zoe_cuda_ctx *ctx, bool three_pass, const uint8_t *stream
 
 // A batch that mixes long (> 1024 residues) and short sequences is aligned in two parts: the short ones take the fast
 // pipelines, the long ones the long-row path (run_align_on_device, long_mode); results are merged in the caller's order.
-// Each part re-enters the entry point the caller used (single- or both-strand).  Returns kNotMixed, having done nothing,
+// Each part re-enters the align driver the caller used (single- or both-strand).  Returns kNotMixed, having done nothing,
 // when the batch has only one kind.
 int align_split_long_short(zoe_cuda_ctx *ctx, bool both_strands, const uint8_t *streamed_concat, const uint64_t *offsets,
-                           uint64_t n, uint32_t *score, uint8_t *status, uint8_t *tier, uint32_t *ref_start,
-                           uint32_t *ref_end, uint32_t *query_start, uint32_t *query_end, uint32_t *cigar,
-                           uint64_t *cigar_off, uint64_t cigar_cap, uint8_t *hazard, uint8_t *strand) {
+                           uint64_t n, const Outputs &o) {
     std::vector<uint64_t> idx[2];  // [0] short, [1] long
     for (uint64_t i = 0; i < n; ++i) idx[offsets[i + 1] - offsets[i] > (uint64_t)kMaxRowsSinglePass ? 1 : 0].push_back(i);
     if (idx[0].empty() || idx[1].empty()) return kNotMixed;
@@ -3229,15 +3275,11 @@ int align_split_long_short(zoe_cuda_ctx *ctx, bool both_strands, const uint8_t *
         for (auto *v : {&q.score, &q.rs, &q.re, &q.qs, &q.qe}) v->assign(pairs, 0);
         for (auto *v : {&q.status, &q.tier, &q.hz, &q.sd}) v->assign(pairs, 0);
         q.coff.assign(pairs + 1, 0);
-        q.cig.assign(std::max<uint64_t>(cigar_cap, 1), 0);
-        int rc = both_strands
-                     ? zoe_cuda_sw_align_both_strands_batch(ctx, q.buf.data(), q.off.data(), idx[w].size(), q.score.data(),
-                                                            q.status.data(), q.tier.data(), q.rs.data(), q.re.data(),
-                                                            q.qs.data(), q.qe.data(), q.cig.data(), q.coff.data(), cigar_cap,
-                                                            q.hz.data(), q.sd.data())
-                     : zoe_cuda_sw_align_batch(ctx, q.buf.data(), q.off.data(), idx[w].size(), q.score.data(), q.status.data(),
-                                               q.tier.data(), q.rs.data(), q.re.data(), q.qs.data(), q.qe.data(), q.cig.data(),
-                                               q.coff.data(), cigar_cap, q.hz.data());
+        q.cig.assign(std::max<uint64_t>(o.cigar_cap, 1), 0);
+        const Outputs qo{q.score.data(), q.status.data(), q.tier.data(), q.rs.data(), q.re.data(), q.qs.data(), q.qe.data(),
+                         q.cig.data(), q.coff.data(), o.cigar_cap, q.hz.data(), q.sd.data()};
+        int rc = both_strands ? align_both_strands(ctx, false, q.buf.data(), q.off.data(), idx[w].size(), qo)
+                              : align_batch(ctx, q.buf.data(), q.off.data(), idx[w].size(), qo);
         if (rc == ZOE_CUDA_E_CIGAR_CAP) {
             rc_cap = rc;
             need += q.coff[0];
@@ -3254,11 +3296,7 @@ int align_split_long_short(zoe_cuda_ctx *ctx, bool both_strands, const uint8_t *
         dp_ms += ctx->last_dp_ms;
         launches += ctx->last_launches.load();
     }
-    if (rc_cap || need > cigar_cap) {
-        cigar_off[0] = need;
-        return fail(ctx, ZOE_CUDA_E_CIGAR_CAP, "CIGAR buffer too small: need at least %llu words, have %llu",
-                    (unsigned long long)need, (unsigned long long)cigar_cap);
-    }
+    if (rc_cap || need > o.cigar_cap) return cigar_cap_error(ctx, o, need, "need at least");
     uint64_t pos = 0;
     size_t cursor[2] = {0, 0};
     for (uint64_t i = 0; i < n; ++i) {
@@ -3266,22 +3304,22 @@ int align_split_long_short(zoe_cuda_ctx *ctx, bool both_strands, const uint8_t *
         const Part &q = part[w];
         const size_t src = cursor[w]++ * np, dst = (size_t)i * np;
         for (uint32_t j = 0; j < np; ++j) {
-            if (score) score[dst + j] = q.score[src + j];
-            if (status) status[dst + j] = q.status[src + j];
-            if (tier) tier[dst + j] = q.tier[src + j];
-            if (ref_start) ref_start[dst + j] = q.rs[src + j];
-            if (ref_end) ref_end[dst + j] = q.re[src + j];
-            if (query_start) query_start[dst + j] = q.qs[src + j];
-            if (query_end) query_end[dst + j] = q.qe[src + j];
-            if (hazard) hazard[dst + j] = q.hz[src + j];
-            if (strand) strand[dst + j] = q.sd[src + j];
-            cigar_off[dst + j] = pos;
+            if (o.score) o.score[dst + j] = q.score[src + j];
+            if (o.status) o.status[dst + j] = q.status[src + j];
+            if (o.tier) o.tier[dst + j] = q.tier[src + j];
+            if (o.ref_start) o.ref_start[dst + j] = q.rs[src + j];
+            if (o.ref_end) o.ref_end[dst + j] = q.re[src + j];
+            if (o.query_start) o.query_start[dst + j] = q.qs[src + j];
+            if (o.query_end) o.query_end[dst + j] = q.qe[src + j];
+            if (o.hazard) o.hazard[dst + j] = q.hz[src + j];
+            if (o.strand) o.strand[dst + j] = q.sd[src + j];
+            o.cigar_off[dst + j] = pos;
             const uint64_t a = q.coff[src + j], b = q.coff[src + j + 1];
-            if (b > a) memcpy(cigar + pos, q.cig.data() + a, (b - a) * sizeof(uint32_t));
+            if (b > a) memcpy(o.cigar + pos, q.cig.data() + a, (b - a) * sizeof(uint32_t));
             pos += b - a;
         }
     }
-    cigar_off[(size_t)n * np] = pos;
+    o.cigar_off[(size_t)n * np] = pos;
     ctx->stats = total;
     ctx->last_total_ms = total_ms;
     ctx->last_dp_ms = dp_ms;
@@ -3491,7 +3529,9 @@ int bucket_best_hits(zoe_cuda_ctx *ctx, Device &d, uint32_t n_strands, bool spli
         CU(ctx, cudaGetLastError());
         ctx->last_launches++;
     }
-    return scan_counts(ctx, d, d.bh_llen.as<uint32_t>(), m, d.bh_loff.as<uint64_t>(), t + (size_t)kBhTabRows * n_keys);
+    unsigned long long *base = t + (size_t)kBhTabRows * n_keys;
+    CU(ctx, cudaMemsetAsync(base, 0, sizeof(unsigned long long), d.stream));
+    return scan_counts(ctx, d, d.bh_llen.as<uint32_t>(), 0, m, d.bh_loff.as<uint64_t>(), base);
 }
 
 // Grows b to `bytes`, keeping its first `used` bytes.
@@ -3501,8 +3541,7 @@ int reserve_keep(zoe_cuda_ctx *ctx, Device &d, DevBuf &b, size_t used, size_t by
     CU(ctx, nb.reserve(bytes));
     if (used) CU(ctx, cudaMemcpyAsync(nb.p, b.p, used, cudaMemcpyDeviceToDevice, d.stream));
     CU(ctx, cudaStreamSynchronize(d.stream));
-    b.release();
-    b = nb;
+    b = std::move(nb);
     return 0;
 }
 
@@ -3577,11 +3616,8 @@ struct PairedArgs {
 // The best-hit entry points.  align = false: score pass + selection only.  pair: the paired search, n pairs (concat /
 // offsets are mate 1); it runs on both strands, selects per pair and finishes with the pair outputs.
 int best_hit(zoe_cuda_ctx *ctx, bool align, bool both_strands, bool three_pass, const uint8_t *concat,
-             const uint64_t *offsets, uint64_t n, const PairedArgs *pair, uint32_t *hit, uint8_t *strand,
-             uint32_t *score, uint8_t *status, uint8_t *tier, uint32_t *runner_up, uint32_t *ref_start,
-             uint32_t *ref_end, uint32_t *query_start, uint32_t *query_end, uint32_t *cigar, uint64_t *cigar_off,
-             uint64_t cigar_cap, uint8_t *hazard) {
-    if (align && (!cigar_off || (!cigar && cigar_cap))) return fail(ctx, ZOE_CUDA_E_BAD_ARG, "null CIGAR outputs");
+             const uint64_t *offsets, uint64_t n, const PairedArgs *pair, const Outputs &o) {
+    if (align && (!o.cigar_off || (!o.cigar && o.cigar_cap))) return fail(ctx, ZOE_CUDA_E_BAD_ARG, "null CIGAR outputs");
     if (pair && pair->min_insert > pair->max_insert)
         return fail(ctx, ZOE_CUDA_E_BAD_ARG, "min_insert (%u) > max_insert (%u)", pair->min_insert, pair->max_insert);
     begin_call(ctx);
@@ -3672,7 +3708,7 @@ int best_hit(zoe_cuda_ctx *ctx, bool align, bool both_strands, bool three_pass, 
                 }
                 rc = for_each_device(ctx, [&](Device &d) {
                     const size_t k = (size_t)(&d - ctx->devs.data());
-                    return align_bucket(ctx, d, three_pass, S, at(k, kBhStart), at(k, kBhMax), cigar_cap, &acc_used[k]);
+                    return align_bucket(ctx, d, three_pass, S, at(k, kBhStart), at(k, kBhMax), o.cigar_cap, &acc_used[k]);
                 });
                 if (rc) return rc;
                 aligned += total;
@@ -3688,11 +3724,9 @@ int best_hit(zoe_cuda_ctx *ctx, bool align, bool both_strands, bool three_pass, 
         }
         uint64_t need = 0;
         for (uint64_t u : acc_used) need += u;
-        if (need > cigar_cap) {
-            cigar_off[0] = need;
+        if (need > o.cigar_cap) {
             sync_and_time(ctx);
-            return fail(ctx, ZOE_CUDA_E_CIGAR_CAP, "CIGAR buffer too small: the best hits need %llu words, have %llu",
-                        (unsigned long long)need, (unsigned long long)cigar_cap);
+            return cigar_cap_error(ctx, o, need, "the best hits need");
         }
         // the CIGAR stream in read order
         for (size_t k = 0; k < nd; ++k) {
@@ -3701,8 +3735,9 @@ int best_hit(zoe_cuda_ctx *ctx, bool align, bool both_strands, bool three_pass, 
             CU(ctx, cudaSetDevice(d.id));
             CU(ctx, d.bh_cig_off.reserve((d.n_count + 1) * sizeof(uint64_t)));
             CU(ctx, d.bh_cig.reserve(std::max<uint64_t>(acc_used[k], 1) * sizeof(uint32_t)));
-            rc = scan_counts(ctx, d, d.bh_cig_count.as<uint32_t>(), d.n_count, d.bh_cig_off.as<uint64_t>(),
-                             d.bh_tab.as<unsigned long long>() + (size_t)kBhTabRows * K);
+            unsigned long long *base = d.bh_tab.as<unsigned long long>() + (size_t)kBhTabRows * K;
+            CU(ctx, cudaMemsetAsync(base, 0, sizeof(unsigned long long), d.stream));
+            rc = scan_counts(ctx, d, d.bh_cig_count.as<uint32_t>(), 0, d.n_count, d.bh_cig_off.as<uint64_t>(), base);
             if (rc) return rc;
             if (acc_used[k]) {
                 const uint32_t blocks = (uint32_t)std::min<uint64_t>((d.n_count + 7) / 8, (uint64_t)d.sm_count * 16);
@@ -3721,53 +3756,23 @@ int best_hit(zoe_cuda_ctx *ctx, bool align, bool both_strands, bool three_pass, 
                 if (rc) return rc;
             }
     }
-    // per-read outputs (and the CIGAR stream) to the caller
-    uint64_t cig_base = 0;
-    for (size_t k = 0; k < nd; ++k) {
-        Device &d = ctx->devs[k];
-        if (d.n_count == 0) continue;
-        CU(ctx, cudaSetDevice(d.id));
-        const size_t first = d.n_first, cnt = d.n_count;
-        auto d2h = [&](void *dst, const DevBuf &src, size_t elem) -> cudaError_t {
-            if (!dst) return cudaSuccess;
-            return cudaMemcpyAsync((uint8_t *)dst + first * elem, src.p, cnt * elem, cudaMemcpyDeviceToHost, d.stream);
-        };
-        if (pair) {  // per-pair outputs: the device's pairs are its mates halved
-            auto pair_d2h = [&](void *dst, const DevBuf &src, size_t elem) -> cudaError_t {
-                if (!dst) return cudaSuccess;
-                return cudaMemcpyAsync((uint8_t *)dst + first / 2 * elem, src.p, cnt / 2 * elem, cudaMemcpyDeviceToHost,
-                                       d.stream);
-            };
-            CU(ctx, pair_d2h(hit, d.pr_hit, 4));
-            if (align) {
-                CU(ctx, pair_d2h(pair->proper, d.pr_proper, 1));
-                CU(ctx, pair_d2h(pair->tlen, d.pr_tlen, 4));
-            }
-        } else {
-            CU(ctx, d2h(hit, d.bh_hit, 4));
-        }
-        CU(ctx, d2h(strand, d.bh_strand, 1));
-        CU(ctx, d2h(score, d.bh_out32[0], 4));
-        CU(ctx, d2h(status, d.bh_out8[0], 1));
-        CU(ctx, d2h(tier, d.bh_out8[1], 1));
-        CU(ctx, d2h(runner_up, d.bh_runner, 4));
-        if (!align) continue;
-        CU(ctx, d2h(ref_start, d.bh_out32[1], 4));
-        CU(ctx, d2h(ref_end, d.bh_out32[2], 4));
-        CU(ctx, d2h(query_start, d.bh_out32[3], 4));
-        CU(ctx, d2h(query_end, d.bh_out32[4], 4));
-        CU(ctx, d2h(hazard, d.bh_out8[2], 1));
-        CU(ctx, cudaMemcpyAsync(cigar_off + first, d.bh_cig_off.p, (cnt + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost,
-                                d.stream));
-        if (acc_used[k])
-            CU(ctx, cudaMemcpyAsync(cigar + cig_base, d.bh_cig.p, acc_used[k] * sizeof(uint32_t), cudaMemcpyDeviceToHost,
-                                    d.stream));
-        CU(ctx, cudaStreamSynchronize(d.stream));
-        if (cig_base)
-            for (size_t i = 0; i <= cnt; ++i) cigar_off[first + i] += cig_base;
-        cig_base += acc_used[k];
+    // per-read outputs (and the CIGAR stream) to the caller; the per-pair outputs are the device's mates halved
+    rc = visit_devices(ctx, false, [&](Device &d) {
+        const int r = pair ? queue_rows_d2h(ctx, d, d.n_first / 2, d.n_count / 2,
+                                            {{o.hit, d.pr_hit, 4}, {pair->proper, d.pr_proper, 1}, {pair->tlen, d.pr_tlen, 4}})
+                           : queue_rows_d2h(ctx, d, d.n_first, d.n_count, {{o.hit, d.bh_hit, 4}});
+        return r ? r : queue_rows_d2h(ctx, d, d.n_first, d.n_count,
+                                  {{o.strand, d.bh_strand, 1}, {o.score, d.bh_out32[0], 4}, {o.status, d.bh_out8[0], 1},
+                                   {o.tier, d.bh_out8[1], 1}, {o.runner_up, d.bh_runner, 4}, {o.ref_start, d.bh_out32[1], 4},
+                                   {o.ref_end, d.bh_out32[2], 4}, {o.query_start, d.bh_out32[3], 4},
+                                   {o.query_end, d.bh_out32[4], 4}, {o.hazard, d.bh_out8[2], 1}});
+    });
+    if (rc) return rc;
+    if (align) {
+        rc = fetch_cigar_stream(ctx, o, 1, &Device::bh_cig_off, &Device::bh_cig, acc_used);
+        if (rc) return rc;
     }
-    if (align && n == 0) cigar_off[0] = 0;
+    if (align && n == 0) o.cigar_off[0] = 0;
     rc = sync_and_time(ctx);
     if (rc) return rc;
     view.ok = true;
@@ -3776,6 +3781,23 @@ int best_hit(zoe_cuda_ctx *ctx, bool align, bool both_strands, bool three_pass, 
     ctx->stats.pairs *= S;
     ctx->stats.cells *= S;
     return rc;
+}
+
+// The run_*_staged entry points: `run` drives one pipeline over the batch staged on every device.
+template <class Run>
+int run_staged(zoe_cuda_ctx *ctx, Run run) {
+    if (!ctx) return ZOE_CUDA_E_BAD_ARG;
+    if (!ctx->staged) return fail(ctx, ZOE_CUDA_E_STATE, "nothing staged");
+    begin_call(ctx);
+    for (Device &d : ctx->devs) {
+        CU(ctx, cudaSetDevice(d.id));
+        CU(ctx, cudaEventRecord(d.ev_begin, d.stream));
+    }
+    int rc = run();
+    if (rc) return rc;
+    rc = sync_and_time(ctx);
+    if (rc) return rc;
+    return gather_stats(ctx);
 }
 
 }  // namespace
@@ -3808,7 +3830,6 @@ int zoe_cuda_create(zoe_cuda_ctx **out, const int *device_ids, int n_devices) {
             delete ctx;
             return ZOE_CUDA_E_CUDA;
         }
-        ctx->devs.push_back(d);
         Device l;  // second stream + buffer set on the same GPU (score-batch pipelining)
         l.id = d.id;
         l.sm_count = d.sm_count;
@@ -3819,50 +3840,14 @@ int zoe_cuda_create(zoe_cuda_ctx **out, const int *device_ids, int n_devices) {
             delete ctx;
             return ZOE_CUDA_E_CUDA;
         }
-        ctx->alt.push_back(l);
+        ctx->devs.push_back(std::move(d));
+        ctx->alt.push_back(std::move(l));
     }
     *out = ctx;
     return 0;
 }
 
-void zoe_cuda_destroy(zoe_cuda_ctx *ctx) {
-    if (!ctx) return;
-    std::vector<Device *> all;
-    for (Device &d : ctx->devs) all.push_back(&d);
-    for (Device &d : ctx->alt) all.push_back(&d);
-    for (Device *dp : all) {
-        Device &d = *dp;
-        cudaSetDevice(d.id);
-        for (DevBuf *b : {&d.ccodes, &d.coff, &d.wk, &d.lut, &d.corder, &d.ccodes_g, &d.coff_g, &d.corder_g, &d.rseq, &d.roff, &d.best, &d.score, &d.status, &d.tier,
-                          &d.wide_ids, &d.counters, &d.pbytes, &d.ends, &d.flags, &d.flag_base, &d.ref_start, &d.ref_end,
-                          &d.query_start, &d.query_end, &d.hazard, &d.hazard_list, &d.cig_scratch, &d.cig_count,
-                          &d.cig_off, &d.cig_out, &d.ex_hbuf, &d.ex_fbuf, &d.ex_cig, &d.ex_lists, &d.ex_counts, &d.ex_fast_fbuf, &d.weights, &d.tp_pair, &d.tp_off, &d.tp_cap, &d.tp_slot,
-                          &d.tp_blob, &d.tp_ctr, &d.tp_cigoff, &d.tp_bw, &d.tp_list, &d.tp_cig, &d.sn_refs, &d.sn_roff, &d.sn_qry, &d.sn_qoff, &d.sn_out, &d.long_ids, &d.long_bnd,
-                          &d.long_queue, &d.ckpt, &d.ckpt_base, &d.win_hist, &d.win_bucket, &d.win_items, &d.win_nitems, &d.win_pitems, &d.win_pnitems, &d.win_amb, &d.starts, &d.cig_bsum})
-            b->release();
-        for (DevBuf *b : {&d.xs_seq, &d.xs_off, &d.strand, &d.sel_cig_count, &d.sel_cig_off, &d.sel_cig_out, &d.sel_ctr})
-            b->release();
-        for (DevBuf &b : d.sel32) b.release();
-        for (DevBuf &b : d.sel8) b.release();
-        for (DevBuf *b : {&d.bh_seq, &d.bh_off, &d.bh_key, &d.bh_tab, &d.bh_list, &d.bh_llen, &d.bh_loff, &d.bh_hit,
-                          &d.bh_strand, &d.bh_runner, &d.bh_cig_count, &d.bh_cig_src, &d.bh_acc, &d.bh_cig_off, &d.bh_cig})
-            b->release();
-        for (DevBuf &b : d.bh_out32) b.release();
-        for (DevBuf &b : d.bh_out8) b.release();
-        if (d.ev_begin) cudaEventDestroy(d.ev_begin);
-        if (d.ev_end) cudaEventDestroy(d.ev_end);
-        if (d.ev_k0) cudaEventDestroy(d.ev_k0);
-        if (d.ev_k1) cudaEventDestroy(d.ev_k1);
-        if (d.ev_fork) cudaEventDestroy(d.ev_fork);
-        if (d.ev_join) cudaEventDestroy(d.ev_join);
-        if (d.aux_stream) cudaStreamDestroy(d.aux_stream);
-        if (d.copy_stream) cudaStreamDestroy(d.copy_stream);
-        if (d.ev_first) cudaEventDestroy(d.ev_first);
-        if (d.ev_copied) cudaEventDestroy(d.ev_copied);
-        if (d.stream) cudaStreamDestroy(d.stream);
-    }
-    delete ctx;
-}
+void zoe_cuda_destroy(zoe_cuda_ctx *ctx) { delete ctx; }
 
 const char *zoe_cuda_last_error(const zoe_cuda_ctx *ctx) { return ctx ? ctx->err.c_str() : "null context"; }
 
@@ -3959,53 +3944,26 @@ int zoe_cuda_stage_streamed(zoe_cuda_ctx *ctx, const uint8_t *streamed_concat, c
 }
 
 int zoe_cuda_run_score_staged(zoe_cuda_ctx *ctx) {
-    if (!ctx) return ZOE_CUDA_E_BAD_ARG;
-    if (!ctx->staged) return fail(ctx, ZOE_CUDA_E_STATE, "nothing staged");
-    begin_call(ctx);
-    for (Device &d : ctx->devs) {
-        CU(ctx, cudaSetDevice(d.id));
-        CU(ctx, cudaEventRecord(d.ev_begin, d.stream));
-    }
-    for (Device &d : ctx->devs) {
-        int rc = run_score_on_device(ctx, d);
-        if (rc) return rc;
-    }
-    int rc = sync_and_time(ctx);
-    if (rc) return rc;
-    return gather_stats(ctx);
+    return run_staged(ctx, [&] {
+        return visit_devices(ctx, false, [&](Device &d) { return run_score_on_device(ctx, d); });
+    });
 }
 
 int zoe_cuda_run_align_staged(zoe_cuda_ctx *ctx) {
-    if (!ctx) return ZOE_CUDA_E_BAD_ARG;
-    if (!ctx->staged) return fail(ctx, ZOE_CUDA_E_STATE, "nothing staged");
-    begin_call(ctx);
-    for (Device &d : ctx->devs) {
-        CU(ctx, cudaSetDevice(d.id));
-        CU(ctx, cudaEventRecord(d.ev_begin, d.stream));
-    }
     // generous device-side CIGAR capacity: 64 words per pair, at most 1 GB (typical CIGARs have <= 5 entries; cheap gaps
     // fragment them).  Nothing is fetched by this entry point: words beyond the capacity are dropped, not an error.
-    int rc = for_each_device(ctx, [&](Device &d) {
-        return run_align_on_device(ctx, d, std::min<uint64_t>((uint64_t)d.n_count * ctx->n_prof * 64 + 1024, (uint64_t)1 << 28));
+    return run_staged(ctx, [&] {
+        return for_each_device(ctx, [&](Device &d) {
+            return run_align_on_device(ctx, d, std::min<uint64_t>((uint64_t)d.n_count * ctx->n_prof * 64 + 1024, (uint64_t)1 << 28));
+        });
     });
-    if (rc) return rc;
-    rc = sync_and_time(ctx);
-    if (rc) return rc;
-    return gather_stats(ctx);
 }
 
 int zoe_cuda_fetch_scores(zoe_cuda_ctx *ctx, uint32_t *score, uint8_t *status, uint8_t *tier) {
     if (!ctx) return ZOE_CUDA_E_BAD_ARG;
     if (!ctx->staged) return fail(ctx, ZOE_CUDA_E_STATE, "nothing staged");
-    for (Device &d : ctx->devs) {
-        if (d.n_count == 0) continue;
-        CU(ctx, cudaSetDevice(d.id));
-        size_t first = (size_t)d.n_first * ctx->n_prof, pairs = (size_t)d.n_count * ctx->n_prof;
-        if (score)
-            CU(ctx, cudaMemcpyAsync(score + first, d.score.p, pairs * sizeof(uint32_t), cudaMemcpyDeviceToHost, d.stream));
-        if (status) CU(ctx, cudaMemcpyAsync(status + first, d.status.p, pairs, cudaMemcpyDeviceToHost, d.stream));
-        if (tier) CU(ctx, cudaMemcpyAsync(tier + first, d.tier.p, pairs, cudaMemcpyDeviceToHost, d.stream));
-    }
+    int rc = queue_pair_outputs_d2h(ctx, Outputs{score, status, tier});
+    if (rc) return rc;
     for (Device &d : ctx->devs) {
         CU(ctx, cudaSetDevice(d.id));
         CU(ctx, cudaStreamSynchronize(d.stream));
@@ -4019,7 +3977,8 @@ int zoe_cuda_sw_score_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_concat, c
     begin_call(ctx);
     int rc = prepare_batch(ctx, streamed_concat, offsets, n);
     if (rc) return rc;
-    auto d2h = [&](Device &d) { return queue_score_d2h(ctx, d, score, status, tier); };
+    const Outputs out{score, status, tier};
+    auto d2h = [&](Device &d) { return queue_pair_outputs_d2h(ctx, d, out); };
     // Large batches are cut into sub-batches that alternate between the two streams of a GPU, so the H2D copy of the
     // next sub-batch and the D2H copy of the previous one overlap the kernels of the current one.  Not for the long-row
     // path (its copies are negligible next to its kernels) nor when packed lanes may overflow (the 32-bit re-run
@@ -4091,38 +4050,8 @@ int zoe_cuda_sw_align_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_concat, c
                             uint32_t *query_start, uint32_t *query_end, uint32_t *cigar, uint64_t *cigar_off,
                             uint64_t cigar_cap, uint8_t *hazard) {
     if (!ctx) return ZOE_CUDA_E_BAD_ARG;
-    if (!cigar_off || (!cigar && cigar_cap)) return fail(ctx, ZOE_CUDA_E_BAD_ARG, "null CIGAR outputs");
-    begin_call(ctx);
-    DebugTimer dbg;
-    int rc = stage_on_devices(ctx, streamed_concat, offsets, n, /*split=*/true);
-    if (rc) return rc;
-    dbg.lap("align: stage");
-    // A batch that mixes long (> 1024 residues) and short sequences is split (align_split_long_short).
-    // Detected from the lengths the staging pass collects anyway (a separate pass that lists the indices of 1M reads
-    // cost 3-4 ms of host time in front of every call); the upload already queued for the whole batch is drained and dropped.
-    if (n > 0 && ctx->staged_max_len > (uint32_t)kMaxRowsSinglePass && ctx->staged_min_len <= (uint32_t)kMaxRowsSinglePass) {
-        for (Device &d : ctx->devs) {
-            cudaSetDevice(d.id);
-            if (d.copy_stream) cudaStreamSynchronize(d.copy_stream);
-            cudaStreamSynchronize(d.stream);
-            d.copy_pending = false;
-        }
-        ctx->staged = false;
-        rc = align_split_long_short(ctx, false, streamed_concat, offsets, n, score, status, tier, ref_start, ref_end,
-                                    query_start, query_end, cigar, cigar_off, cigar_cap, hazard, nullptr);
-        if (rc != kNotMixed) return rc;
-    }
-    rc = for_each_device(ctx, [&](Device &d) { return run_align_on_device(ctx, d, cigar_cap); });
-    if (rc) return rc;
-    dbg.lap("align: run_align_on_device");
-    rc = fetch_alignments(ctx, score, status, tier, ref_start, ref_end, query_start, query_end, cigar, cigar_off, cigar_cap,
-                          hazard);
-    if (rc) return rc;
-    if (n == 0) cigar_off[0] = 0;
-    dbg.lap("align: d2h");
-    rc = sync_and_time(ctx);
-    if (rc) return rc;
-    return gather_stats(ctx);
+    return align_batch(ctx, streamed_concat, offsets, n,
+                       {score, status, tier, ref_start, ref_end, query_start, query_end, cigar, cigar_off, cigar_cap, hazard});
 }
 
 int zoe_cuda_sw_score_ranges_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_concat, const uint64_t *offsets, uint64_t n,
@@ -4134,7 +4063,7 @@ int zoe_cuda_sw_score_ranges_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_co
     if (rc) return rc;
     rc = for_each_device(ctx, [&](Device &d) { return run_ranges_on_device(ctx, d); });
     if (rc) return rc;
-    rc = queue_ranges_d2h(ctx, score, status, tier, ref_start, ref_end, query_start, query_end);
+    rc = queue_pair_outputs_d2h(ctx, Outputs{score, status, tier, ref_start, ref_end, query_start, query_end});
     if (rc) return rc;
     rc = sync_and_time(ctx);
     if (rc) return rc;
@@ -4142,18 +4071,7 @@ int zoe_cuda_sw_score_ranges_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_co
 }
 
 int zoe_cuda_run_ranges_staged(zoe_cuda_ctx *ctx) {
-    if (!ctx) return ZOE_CUDA_E_BAD_ARG;
-    if (!ctx->staged) return fail(ctx, ZOE_CUDA_E_STATE, "nothing staged");
-    begin_call(ctx);
-    for (Device &d : ctx->devs) {
-        CU(ctx, cudaSetDevice(d.id));
-        CU(ctx, cudaEventRecord(d.ev_begin, d.stream));
-    }
-    int rc = for_each_device(ctx, [&](Device &d) { return run_ranges_on_device(ctx, d); });
-    if (rc) return rc;
-    rc = sync_and_time(ctx);
-    if (rc) return rc;
-    return gather_stats(ctx);
+    return run_staged(ctx, [&] { return for_each_device(ctx, [&](Device &d) { return run_ranges_on_device(ctx, d); }); });
 }
 
 int zoe_cuda_sw_align_3pass_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_concat, const uint64_t *offsets, uint64_t n,
@@ -4167,8 +4085,7 @@ int zoe_cuda_sw_align_3pass_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_con
     if (rc) return rc;
     rc = for_each_device(ctx, [&](Device &d) { return run_3pass_on_device(ctx, d, cigar_cap); });
     if (rc) return rc;
-    rc = fetch_alignments(ctx, score, status, tier, ref_start, ref_end, query_start, query_end, cigar, cigar_off, cigar_cap,
-                          nullptr);
+    rc = fetch_alignments(ctx, {score, status, tier, ref_start, ref_end, query_start, query_end, cigar, cigar_off, cigar_cap});
     if (rc) return rc;
     if (n == 0) cigar_off[0] = 0;
     rc = sync_and_time(ctx);
@@ -4177,18 +4094,9 @@ int zoe_cuda_sw_align_3pass_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_con
 }
 
 int zoe_cuda_run_3pass_staged(zoe_cuda_ctx *ctx) {
-    if (!ctx) return ZOE_CUDA_E_BAD_ARG;
-    if (!ctx->staged) return fail(ctx, ZOE_CUDA_E_STATE, "nothing staged");
-    begin_call(ctx);
-    for (Device &d : ctx->devs) {
-        CU(ctx, cudaSetDevice(d.id));
-        CU(ctx, cudaEventRecord(d.ev_begin, d.stream));
-    }
-    int rc = for_each_device(ctx, [&](Device &d) { return run_3pass_on_device(ctx, d, (uint64_t)d.n_count * ctx->n_prof * 8 + 1024); });
-    if (rc) return rc;
-    rc = sync_and_time(ctx);
-    if (rc) return rc;
-    return gather_stats(ctx);
+    return run_staged(ctx, [&] {
+        return for_each_device(ctx, [&](Device &d) { return run_3pass_on_device(ctx, d, (uint64_t)d.n_count * ctx->n_prof * 8 + 1024); });
+    });
 }
 
 int zoe_cuda_sw_score_both_strands_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_concat, const uint64_t *offsets,
@@ -4206,10 +4114,8 @@ int zoe_cuda_sw_score_both_strands_batch(zoe_cuda_ctx *ctx, const uint8_t *strea
         if (rc) return rc;
     }
     view.leave();
-    for (Device &d : ctx->devs) {
-        rc = queue_score_d2h(ctx, d, score, status, tier);
-        if (rc) return rc;
-    }
+    rc = queue_pair_outputs_d2h(ctx, Outputs{score, status, tier});
+    if (rc) return rc;
     rc = queue_strand_d2h(ctx, strand);
     if (rc) return rc;
     rc = sync_and_time(ctx);
@@ -4235,7 +4141,7 @@ int zoe_cuda_sw_score_ranges_both_strands_batch(zoe_cuda_ctx *ctx, const uint8_t
         if (rc) return rc;
     }
     view.leave();
-    rc = queue_ranges_d2h(ctx, score, status, tier, ref_start, ref_end, query_start, query_end);
+    rc = queue_pair_outputs_d2h(ctx, Outputs{score, status, tier, ref_start, ref_end, query_start, query_end});
     if (rc) return rc;
     rc = queue_strand_d2h(ctx, strand);
     if (rc) return rc;
@@ -4250,8 +4156,9 @@ int zoe_cuda_sw_align_both_strands_batch(zoe_cuda_ctx *ctx, const uint8_t *strea
                                          uint32_t *ref_end, uint32_t *query_start, uint32_t *query_end, uint32_t *cigar,
                                          uint64_t *cigar_off, uint64_t cigar_cap, uint8_t *hazard, uint8_t *strand) {
     if (!ctx) return ZOE_CUDA_E_BAD_ARG;
-    return align_both_strands(ctx, false, streamed_concat, offsets, n, score, status, tier, ref_start, ref_end, query_start,
-                              query_end, cigar, cigar_off, cigar_cap, hazard, strand);
+    return align_both_strands(ctx, false, streamed_concat, offsets, n,
+                              {score, status, tier, ref_start, ref_end, query_start, query_end, cigar, cigar_off, cigar_cap,
+                               hazard, strand});
 }
 
 int zoe_cuda_sw_align_3pass_both_strands_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_concat, const uint64_t *offsets,
@@ -4260,16 +4167,20 @@ int zoe_cuda_sw_align_3pass_both_strands_batch(zoe_cuda_ctx *ctx, const uint8_t 
                                                uint32_t *query_end, uint32_t *cigar, uint64_t *cigar_off, uint64_t cigar_cap,
                                                uint8_t *strand) {
     if (!ctx) return ZOE_CUDA_E_BAD_ARG;
-    return align_both_strands(ctx, true, streamed_concat, offsets, n, score, status, tier, ref_start, ref_end, query_start,
-                              query_end, cigar, cigar_off, cigar_cap, nullptr, strand);
+    return align_both_strands(ctx, true, streamed_concat, offsets, n,
+                              {score, status, tier, ref_start, ref_end, query_start, query_end, cigar, cigar_off, cigar_cap,
+                               nullptr, strand});
 }
 
 int zoe_cuda_sw_score_best_hit_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_concat, const uint64_t *offsets,
                                      uint64_t n, int both_strands, uint32_t *hit, uint8_t *strand, uint32_t *score,
                                      uint8_t *status, uint8_t *tier, uint32_t *runner_up) {
     if (!ctx) return ZOE_CUDA_E_BAD_ARG;
-    return best_hit(ctx, false, both_strands != 0, false, streamed_concat, offsets, n, nullptr, hit, strand, score, status, tier,
-                    runner_up, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 0, nullptr);
+    Outputs o{score, status, tier};
+    o.strand = strand;
+    o.hit = hit;
+    o.runner_up = runner_up;
+    return best_hit(ctx, false, both_strands != 0, false, streamed_concat, offsets, n, nullptr, o);
 }
 
 int zoe_cuda_sw_align_best_hit_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_concat, const uint64_t *offsets,
@@ -4278,8 +4189,9 @@ int zoe_cuda_sw_align_best_hit_batch(zoe_cuda_ctx *ctx, const uint8_t *streamed_
                                      uint32_t *ref_start, uint32_t *ref_end, uint32_t *query_start, uint32_t *query_end,
                                      uint32_t *cigar, uint64_t *cigar_off, uint64_t cigar_cap, uint8_t *hazard) {
     if (!ctx) return ZOE_CUDA_E_BAD_ARG;
-    return best_hit(ctx, true, both_strands != 0, three_pass != 0, streamed_concat, offsets, n, nullptr, hit, strand, score, status,
-                    tier, runner_up, ref_start, ref_end, query_start, query_end, cigar, cigar_off, cigar_cap, hazard);
+    return best_hit(ctx, true, both_strands != 0, three_pass != 0, streamed_concat, offsets, n, nullptr,
+                    {score, status, tier, ref_start, ref_end, query_start, query_end, cigar, cigar_off, cigar_cap, hazard, strand,
+                     hit, runner_up});
 }
 
 int zoe_cuda_sw_score_paired_best_hit_batch(zoe_cuda_ctx *ctx, const uint8_t *mate1_concat, const uint64_t *mate1_offsets,
@@ -4288,8 +4200,11 @@ int zoe_cuda_sw_score_paired_best_hit_batch(zoe_cuda_ctx *ctx, const uint8_t *ma
                                             uint32_t *runner_up) {
     if (!ctx) return ZOE_CUDA_E_BAD_ARG;
     const PairedArgs pair{mate2_concat, mate2_offsets, 0, ~0u, nullptr, nullptr};
-    return best_hit(ctx, false, true, false, mate1_concat, mate1_offsets, n_pairs, &pair, hit, strand, score, status, tier,
-                    runner_up, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 0, nullptr);
+    Outputs o{score, status, tier};
+    o.strand = strand;
+    o.hit = hit;
+    o.runner_up = runner_up;
+    return best_hit(ctx, false, true, false, mate1_concat, mate1_offsets, n_pairs, &pair, o);
 }
 
 int zoe_cuda_sw_align_paired_best_hit_batch(zoe_cuda_ctx *ctx, const uint8_t *mate1_concat, const uint64_t *mate1_offsets,
@@ -4301,8 +4216,9 @@ int zoe_cuda_sw_align_paired_best_hit_batch(zoe_cuda_ctx *ctx, const uint8_t *ma
                                             uint64_t cigar_cap, uint8_t *hazard) {
     if (!ctx) return ZOE_CUDA_E_BAD_ARG;
     const PairedArgs pair{mate2_concat, mate2_offsets, min_insert, max_insert, proper, tlen};
-    return best_hit(ctx, true, true, three_pass != 0, mate1_concat, mate1_offsets, n_pairs, &pair, hit, strand, score,
-                    status, tier, runner_up, ref_start, ref_end, query_start, query_end, cigar, cigar_off, cigar_cap, hazard);
+    return best_hit(ctx, true, true, three_pass != 0, mate1_concat, mate1_offsets, n_pairs, &pair,
+                    {score, status, tier, ref_start, ref_end, query_start, query_end, cigar, cigar_off, cigar_cap, hazard, strand,
+                     hit, runner_up});
 }
 
 int zoe_cuda_sneaky_snake_batch(zoe_cuda_ctx *ctx, const uint8_t *refs, const uint64_t *ref_offsets, const uint8_t *queries,
@@ -4405,7 +4321,6 @@ int zoe_cuda_dpx_peak(zoe_cuda_ctx *ctx, int kind, double *giga_lane_instr_per_s
         CU(ctx, cudaEventElapsedTime(&ms, d.ev_k0, d.ev_k1));
         if (rep > 0) best_ms = std::min(best_ms, ms);
     }
-    out.release();
     // kind 0: 16 DPX instructions per inner iteration; kind 1: 8 cell pairs x 5.5 instructions
     // kind 2: 8 x (2 hmax2 + 2 integer ops); kind 3: 8 cell pairs x 6 instructions
     double instr_per_thread = (kind == 0) ? 16.0 * iters : (kind == 2 ? 32.0 * iters : (kind == 3 ? 48.0 * iters : 8.0 * 5.5 * iters));
