@@ -318,7 +318,8 @@ typedef struct {
 int zoe_cuda_last_stats(const zoe_cuda_ctx *ctx, zoe_cuda_stats *out);
 
 /* Integer max-plus issue-rate microbenchmark (the roofline denominator, SURVEY.md 8(d)):
- * kind 0 = VIADDMNMX.S16x2 only, 1 = the score kernel's instruction mix without memory.
+ * kind 0 = VIADDMNMX.S16x2 only; 4 = the score kernel's instruction mix without memory (2 per-half adds + 3.5 DPX
+ * per cell pair), 1 = the mix it replaced (1 add + 4.5 DPX).  Kinds 1 and 4 both count 5.5 instructions per pair.
  * Returns giga warp-lane-instructions per second on device 0 of the context. */
 int zoe_cuda_dpx_peak(zoe_cuda_ctx *ctx, int kind, double *giga_lane_instr_per_s, float *ms);
 

@@ -19,13 +19,20 @@
 //
 // Arithmetic (true, un-offset values; zoe's MIN-offset saturating arithmetic computes the same
 // H, SURVEY.md 8(a) "Equivalent closed form"):
-//     x  = max(E^, F^, go) - go            (E^ = E + go, F^ = F + go: the shifted gap states)
-//     H  = max(Hdiag + W, x)               VIADDMNMX.S16x2
-//     E^ = max(E^ - ge, H)                 VIADDMNMX.S16x2
-//     F^ = max(F^ - ge, H)                 VIADDMNMX.S16x2
-//     best = max(best, H, H')              VIMNMX3.S16x2 (two rows per instruction)
-// i.e. 4.5 DPX/ALU instructions + 1 plain add per packed cell pair.  The subtraction is exact as a
-// plain 32-bit add because max(..., go) - go >= 0 in both halves (no borrow crosses the halves).
+//     dW = Hdiag + W                       VIADD.16x2 (per-half add, not on the ALU pipe)
+//     H  = max(dW, E, F, 0)                VIMNMX3.S16x2.RELU
+//     Hg = H - go                          VIADD.16x2
+//     E  = max(E - ge, Hg)                 VIADDMNMX.S16x2
+//     F  = max(F - ge, Hg)                 VIADDMNMX.S16x2
+//     best = max(best, dW, dW')            VIMNMX3.S16x2 (two rows per instruction)
+// i.e. 3.5 ALU-pipe instructions + 2 per-half adds per packed cell pair (DESIGN.md section 4 gives the proofs):
+//   * E, F <= 0 give the same H as -inf (the 0 floor), so zero initial states and zeros entering lane 0 are exact;
+//   * E, F >= -go always and dW >= kPadWeight, so no half wraps below the overflow threshold;
+//   * max over cells of H = max(0, max over cells of dW): a cell whose H comes from E or F never beats the cell that
+//     opened the gap (go, ge >= 0), and the running maximum must read dW -- with H, ptxas fuses the add and the
+//     max3 back into VIADDMNMX.RELU + VIMNMX.RELU (4.5 ALU instructions again);
+//   * the first cell whose H reaches the packed threshold takes H = dW <= 32766, so best >= threshold still detects
+//     the overflow, and a wrap after it stays inside its own 16-bit half.
 //
 // Overflow / escalation: the packed kernel is exact while every H < OVF_THRESH (= 32767 - max
 // weight); a task whose best reaches the threshold is reported as "needs wide" and re-run by the
@@ -115,6 +122,10 @@ struct Ops<true> {
     static __device__ __forceinline__ uint32_t max3(uint32_t a, uint32_t b, uint32_t c) {
         return __vimax3_s16x2(a, b, c);
     }
+    static __device__ __forceinline__ uint32_t max3z(uint32_t a, uint32_t b, uint32_t c) {  // max(a, b, c, 0)
+        return __vimax3_s16x2_relu(a, b, c);
+    }
+    static __device__ __forceinline__ uint32_t add(uint32_t a, uint32_t b) { return __vadd2(a, b); }  // per half, no carry
     static __device__ __forceinline__ uint32_t max2(uint32_t a, uint32_t b) { return __vmaxs2(a, b); }
     static __device__ __forceinline__ uint32_t min2(uint32_t a, uint32_t b) { return __vmins2(a, b); }
     static __device__ __forceinline__ uint32_t splat(int v) {
@@ -130,18 +141,20 @@ struct Ops<false> {
     static __device__ __forceinline__ uint32_t max3(uint32_t a, uint32_t b, uint32_t c) {
         return (uint32_t)__vimax3_s32((int)a, (int)b, (int)c);
     }
+    static __device__ __forceinline__ uint32_t max3z(uint32_t a, uint32_t b, uint32_t c) {
+        return (uint32_t)__vimax3_s32_relu((int)a, (int)b, (int)c);
+    }
+    static __device__ __forceinline__ uint32_t add(uint32_t a, uint32_t b) { return a + b; }
     static __device__ __forceinline__ uint32_t max2(uint32_t a, uint32_t b) { return (uint32_t)max((int)a, (int)b); }
     static __device__ __forceinline__ uint32_t min2(uint32_t a, uint32_t b) { return (uint32_t)min((int)a, (int)b); }
     static __device__ __forceinline__ uint32_t splat(int v) { return (uint32_t)v; }
 };
 
 // Where the packed score kernel takes the gap penalties from.  A DPX instruction accepts a 32-bit immediate but no
-// constant-bank or uniform-register operand, so a penalty known only at run time occupies a vector register in three of
-// the four DPX instructions of every row (max3 with go, the two addmax with -ge).
+// constant-bank or uniform-register operand, so a penalty known only at run time occupies a vector register in three
+// instructions of every row (the "- go" add, the two addmax with -ge).
 //   GapRt         the penalties of ScoreParams, kept opaque in registers (any scoring)
-//   GapImm<O, E>  go = O, ge = E compiled in: the DPX instructions take them as immediates
-// With immediates ptxas emits the "- go" of a row as VIADD rather than IMAD.IADD.  Pinning it to IMAD (a mad.lo.u32
-// with a multiplier of 1 ptxas cannot see) measured slower on B200, config 2: 281.1 against 279.9 ms per step.
+//   GapImm<O, E>  go = O, ge = E compiled in: the instructions take them as immediates
 struct GapRt {
     static constexpr bool kImm = false;
     static constexpr int GO = 0, GE = 0;
@@ -293,20 +306,22 @@ __device__ __forceinline__ void build_task_table(const TaskSmem &m, const ScoreP
 // column symbol's table row; (diag, E) enter from the lane above.
 // H is kept in two register sets (P = step parity): column j-1 is read from set P, column j is written to
 // set 1-P, so the loop-carried "diag = H[i]" needs no register moves.
+// E and F are the true gap states (see the header); the running maximum reads dW, not H (see there why).
 #define ZOE_SCORE_ROW(ST, W)                                     \
     {                                                            \
-        uint32_t x = O::max3(ST##E, ST##F[i], go_s) - go_s;      \
-        uint32_t H = O::addmax(ST##diag, W, x);                  \
+        const uint32_t dW = O::add(ST##diag, W);                 \
+        const uint32_t H = O::max3z(dW, ST##E, ST##F[i]);        \
+        const uint32_t Hg = O::add(H, neg_go);                   \
         ST##diag = ST##H[PO][i];                                 \
-        ST##E = O::addmax(ST##E, neg_ge, H);                     \
-        ST##F[i] = O::addmax(ST##F[i], neg_ge, H);               \
+        ST##E = O::addmax(ST##E, neg_ge, Hg);                    \
+        ST##F[i] = O::addmax(ST##F[i], neg_ge, Hg);              \
         ST##H[PN][i] = H;                                        \
         if (PACKED && kHalfMax) {                                \
             ST##best = half2_max_bits(ST##best, H);              \
         } else if (i & 1) {                                      \
-            ST##best = O::max3(ST##best, H, ST##hp);             \
+            ST##best = O::max3(ST##best, dW, ST##hp);            \
         } else {                                                 \
-            ST##hp = H;                                          \
+            ST##hp = dW;                                         \
         }                                                        \
     }
 
@@ -340,7 +355,7 @@ __global__ void __launch_bounds__((NS == 2 && (PP || K > 20)) ? ZOE_SCORE2_THREA
     const uint8_t *cc = p.cols_in_smem ? s_cc : p.ccodes;
 
     static_assert(!Gap::kImm || PACKED, "compiled-in gap penalties exist for the packed kernels only");
-    uint32_t go_s = O::splat(Gap::kImm ? Gap::GO : p.go), neg_ge = O::splat(Gap::kImm ? -Gap::GE : -p.ge);
+    uint32_t neg_go = O::splat(Gap::kImm ? -Gap::GO : -p.go), neg_ge = O::splat(Gap::kImm ? -Gap::GE : -p.ge);
     const uint4 *tab_lane = tab + lig;
     // Loop invariants kept opaque so the compiler does not rematerialise them inside the hot loops (S2R + address
     // arithmetic); the table offset stays a 32-bit offset into the shared array so the loads remain LDS.128.
@@ -351,7 +366,7 @@ __global__ void __launch_bounds__((NS == 2 && (PP || K > 20)) ? ZOE_SCORE2_THREA
     if constexpr (Gap::kImm)
         asm volatile("" : "+r"(tab_lane_off), "+r"(nz));
     else
-        asm volatile("" : "+r"(go_s), "+r"(neg_ge), "+r"(tab_lane_off), "+r"(nz));
+        asm volatile("" : "+r"(neg_go), "+r"(neg_ge), "+r"(tab_lane_off), "+r"(nz));
 
     // Static round-robin task assignment: every group of a warp makes the same number of trips,
     // so the warp never diverges on the task loop (invalid trips run on empty sequences).

@@ -6,7 +6,8 @@
 // 32 lanes x K rows that the warp sweeps one after the other over all columns; the H / E values leaving
 // a chunk's last row are parked in a per-warp boundary row in global memory (8 bytes per column,
 // L2-resident) and picked up as the top boundary of the next chunk:
-//     * bottom boundary: lane 31 stores (H, E^) of its last row, one 8-byte store per column;
+//     * bottom boundary: lane 31 stores (H, E) of its last row, one 8-byte store per column (E = the true gap state
+//       of sw_score.cuh; the next chunk's lane 0 takes it as its incoming E);
 //     * top boundary: all lanes prefetch the next 32 columns with one coalesced 256-byte load, and
 //       lane 0 receives its column's entry by __shfl_sync -- the load latency never sits on the systolic
 //       critical path.
@@ -59,11 +60,11 @@ __global__ void __launch_bounds__(512) sw_score_long_kernel(const LongParams lp)
     __syncthreads();
     const uint8_t *cc = p.cols_in_smem ? s_cc : p.ccodes;
 
-    uint32_t go_s = O::splat(p.go), neg_ge = O::splat(-p.ge);
+    uint32_t neg_go = O::splat(-p.go), neg_ge = O::splat(-p.ge);
     // loop invariants kept opaque (no rematerialisation in the hot loop); table offset as a 32-bit shared offset
     uint32_t tab_lane_off = (uint32_t)warp * (uint32_t)tab_bytes + (uint32_t)lane * 16u;
     uint32_t nz = lane != 0 ? 1u : 0u;  // lane 0 takes its inputs from the previous chunk's boundary row instead
-    asm volatile("" : "+r"(go_s), "+r"(neg_ge), "+r"(tab_lane_off), "+r"(nz));
+    asm volatile("" : "+r"(neg_go), "+r"(neg_ge), "+r"(tab_lane_off), "+r"(nz));
     uint2 *bnd = lp.boundary + (size_t)(blockIdx.x * warps_per_block + warp) * lp.max_L;
 
     for (;;) {
@@ -156,16 +157,18 @@ __global__ void __launch_bounds__(512) sw_score_long_kernel(const LongParams lp)
 #pragma unroll
                             for (int q = 0; q < 4; ++q) {
                                 const int i = i4 * 4 + q;
-                                const uint32_t x = O::max3(E, F[i], go_s) - go_s;
-                                const uint32_t Hn = O::addmax(diag, w[q], x);
+                                // the recurrence of ZOE_SCORE_ROW (sw_score.cuh)
+                                const uint32_t dW = O::add(diag, w[q]);
+                                const uint32_t Hn = O::max3z(dW, E, F[i]);
+                                const uint32_t Hg = O::add(Hn, neg_go);
                                 diag = H[PO][i];
-                                E = O::addmax(E, neg_ge, Hn);
-                                F[i] = O::addmax(F[i], neg_ge, Hn);
+                                E = O::addmax(E, neg_ge, Hg);
+                                F[i] = O::addmax(F[i], neg_ge, Hg);
                                 H[PN][i] = Hn;
                                 if (q & 1)
-                                    best = O::max3(best, Hn, hp);
+                                    best = O::max3(best, dW, hp);
                                 else
-                                    hp = Hn;
+                                    hp = dW;
                             }
                             h_last = H[PN][i4 * 4 + 3];
                         }

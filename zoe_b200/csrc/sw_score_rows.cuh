@@ -15,7 +15,7 @@
 //   * a group (warp) sweeps TWO tasks at once as independent dependency chains (the table is shared, so the second
 //                chain costs registers only).
 //
-// Per packed cell pair: 4.5 DPX/ALU + 2 FMA-pipe (x - go, weight assembly) + 0.5 LDS.128.  The sweep is as short as a
+// Per packed cell pair: 3.5 DPX/ALU + 2 per-half adds (dW, H - go) + 1 FMA-pipe IMAD (weight assembly) + 0.5 LDS.128.  The sweep is as short as a
 // streamed sequence (300 columns in config 5), so the lane skew (G-1 steps of ramp and tail) is a real cost here:
 // skew 1 is used (the shuffle latency is covered by the second chain).
 //
@@ -76,11 +76,11 @@ __global__ void __launch_bounds__(K > 20 ? 256 : 384) sw_score_rows_kernel(const
     }
     __syncthreads();
 
-    uint32_t go_s = O::splat(p.go), neg_ge = O::splat(-p.ge);
+    uint32_t neg_go = O::splat(-p.go), neg_ge = O::splat(-p.ge);
     uint32_t lane_off = (uint32_t)lane * 16u;
     uint32_t nz = lane != 0 ? 1u : 0u;
     uint32_t sym_stride_r = sym_stride;  // opaque: symbol index -> table offset by an IMAD (FMA pipe), not a shift (ALU)
-    asm volatile("" : "+r"(go_s), "+r"(neg_ge), "+r"(lane_off), "+r"(nz), "+r"(sym_stride_r));
+    asm volatile("" : "+r"(neg_go), "+r"(neg_ge), "+r"(lane_off), "+r"(nz), "+r"(sym_stride_r));
     const uint32_t pad_sym = (uint32_t)p.S;
 
     // a "task" = two streamed sequences (2t, 2t+1); a warp sweeps two tasks (chains a and b) per trip
@@ -227,8 +227,9 @@ __global__ void __launch_bounds__(K > 20 ? 256 : 384) sw_score_rows_kernel(const
 // very first ramp and the very last tail of a warp's whole stream are idle.
 //   * a trip's length is max over its four sequences (pad symbols beyond a sequence's own end, as before);
 //   * boundary steps (the first 32 steps of a trip): lane l is still in trip t-1 while step < l, crosses at step == l
-//     (parks its per-trip maxima in shared memory, zeroes its H / F registers and the pending diagonal), and reads the
-//     column symbols of whichever trip it is in (two staging buffers per warp);
+//     (parks its per-trip maxima in shared memory, zeroes its H / F registers and the pending diagonal -- a zero gap
+//     state is exact, see sw_score.cuh), and reads the column symbols of whichever trip it is in (two staging buffers
+//     per warp);
 //   * steady steps: every lane is in the current trip, no per-lane tests -- the same loop as above.
 // Requires every streamed sequence to have at least 64 residues (the host falls back to sw_score_rows_kernel otherwise).
 // ---------------------------------------------------------------------------------------------
@@ -270,11 +271,11 @@ __global__ void __launch_bounds__(K > 20 ? 256 : 384) sw_score_rows_stream_kerne
     }
     __syncthreads();
 
-    uint32_t go_s = O::splat(p.go), neg_ge = O::splat(-p.ge);
+    uint32_t neg_go = O::splat(-p.go), neg_ge = O::splat(-p.ge);
     uint32_t lane_off = (uint32_t)lane * 16u;
     uint32_t nz = lane != 0 ? 1u : 0u;
     uint32_t sym_stride_r = sym_stride;
-    asm volatile("" : "+r"(go_s), "+r"(neg_ge), "+r"(lane_off), "+r"(nz), "+r"(sym_stride_r));
+    asm volatile("" : "+r"(neg_go), "+r"(neg_ge), "+r"(lane_off), "+r"(nz), "+r"(sym_stride_r));
     const uint32_t pad_sym = (uint32_t)p.S;
 
     const uint32_t n_tasks = (p.n_rseq + 1) / 2;

@@ -478,7 +478,8 @@ __global__ void __launch_bounds__(256) dpx_peak_kernel(uint32_t *out, int iters,
         a[i] = seed * (threadIdx.x + 1) + i;
         b[i] = seed + i * 7u;
     }
-    const uint32_t c = seed ^ 0x00030003u, g = 0x000a000au;
+    const uint32_t c = seed ^ 0x00030003u, g = 0x000a000au, ng = 0xfff6fff6u;
+    uint32_t dp = 0;
     for (int it = 0; it < iters; ++it) {
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
@@ -500,8 +501,20 @@ __global__ void __launch_bounds__(256) dpx_peak_kernel(uint32_t *out, int iters,
                 b[i] = __viaddmax_s16x2(b[i], c, h);
                 __half2 hm = __hmax2(*reinterpret_cast<__half2 *>(&a[(i + 3) & 7]), *reinterpret_cast<__half2 *>(&h));
                 a[(i + 3) & 7] = *reinterpret_cast<uint32_t *>(&hm);
+            } else if (KIND == 4) {
+                // the score kernel's per-cell-pair mix: 2 per-half adds + 1 relu max3 + 2 addmax + 0.5 max3 (the
+                // running maximum reads dW of both rows, as the kernel does, so ptxas cannot fuse the add into the max)
+                uint32_t d = __vadd2(a[(i + 1) & 7], c);
+                uint32_t h = __vimax3_s16x2_relu(d, a[i], b[i]);
+                uint32_t hg = __vadd2(h, ng);
+                a[i] = __viaddmax_s16x2(a[i], c, hg);
+                b[i] = __viaddmax_s16x2(b[i], c, hg);
+                if (i & 1)
+                    a[(i + 3) & 7] = __vimax3_s16x2(a[(i + 3) & 7], d, dp);
+                else
+                    dp = d;
             } else {
-                // the score kernel's per-cell-pair mix: 1 max3 + 1 add + 3 addmax + 0.5 max3
+                // the score kernel's per-cell-pair mix before the relu form: 1 max3 + 1 add + 3 addmax + 0.5 max3
                 uint32_t x = __vimax3_s16x2(a[i], b[i], g) - g;
                 uint32_t h = __viaddmax_s16x2(a[(i + 1) & 7], c, x);
                 a[i] = __viaddmax_s16x2(a[i], c, h);
@@ -4312,6 +4325,8 @@ int zoe_cuda_dpx_peak(zoe_cuda_ctx *ctx, int kind, double *giga_lane_instr_per_s
             dpx_peak_kernel<2><<<blocks, threads, 0, d.stream>>>(out.as<uint32_t>(), iters, 12345u + rep);
         else if (kind == 3)
             dpx_peak_kernel<3><<<blocks, threads, 0, d.stream>>>(out.as<uint32_t>(), iters, 12345u + rep);
+        else if (kind == 4)
+            dpx_peak_kernel<4><<<blocks, threads, 0, d.stream>>>(out.as<uint32_t>(), iters, 12345u + rep);
         else
             dpx_peak_kernel<1><<<blocks, threads, 0, d.stream>>>(out.as<uint32_t>(), iters, 12345u + rep);
         CU(ctx, cudaGetLastError());
@@ -4321,7 +4336,7 @@ int zoe_cuda_dpx_peak(zoe_cuda_ctx *ctx, int kind, double *giga_lane_instr_per_s
         CU(ctx, cudaEventElapsedTime(&ms, d.ev_k0, d.ev_k1));
         if (rep > 0) best_ms = std::min(best_ms, ms);
     }
-    // kind 0: 16 DPX instructions per inner iteration; kind 1: 8 cell pairs x 5.5 instructions
+    // kind 0: 16 DPX instructions per inner iteration; kinds 1 and 4: 8 cell pairs x 5.5 instructions
     // kind 2: 8 x (2 hmax2 + 2 integer ops); kind 3: 8 cell pairs x 6 instructions
     double instr_per_thread = (kind == 0) ? 16.0 * iters : (kind == 2 ? 32.0 * iters : (kind == 3 ? 48.0 * iters : 8.0 * 5.5 * iters));
     double lanes = (double)blocks * threads;
